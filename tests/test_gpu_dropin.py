@@ -30,15 +30,15 @@ PYREF = osp.join(ROOT, 'oracle', '_ref', 'pyref.zip')
 
 @pytest.fixture(scope='module')
 def ref_model_module(tmp_path_factory):
-    if osp.isdir('/root/reference/models'):
-        ref_root = '/root/reference'
+    from oracle import build_ref
+    if build_ref.REF_ROOT and osp.isdir(osp.join(build_ref.REF_ROOT, 'models')):
+        ref_root = build_ref.REF_ROOT
     elif osp.isfile(PYREF):
         ref_root = str(tmp_path_factory.mktemp('pyref'))
         with zipfile.ZipFile(PYREF) as z:
             z.extractall(ref_root)
     else:
-        pytest.skip('reference Python not staged (run python oracle/build_ref.py where /root/reference exists)')
-    from oracle import build_ref
+        pytest.skip('reference Python not staged (set FASTPCC_REFERENCE_ROOT to a checkout of the reference, or run oracle/build_ref.py there)')
     from tests import ref_import
     from fastpcc_b200 import space_filling_curves_ext
     from fastpcc_b200.int_sparse_conv import ext

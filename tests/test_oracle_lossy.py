@@ -1,5 +1,5 @@
 """The float oracle of the lossy codec is deterministic and matches its committed fixture: the reference's unmodified
-lossy_coord_v2 model (imported from /root/reference, or from the staged oracle/_ref/pyref.zip) on the CPU
+lossy_coord_v2 model (imported from $FASTPCC_REFERENCE_ROOT, or from the staged oracle/_ref/pyref.zip) on the CPU
 MinkowskiEngine stand-in (oracle/me_cpu.py) reproduces tests/golden/lossy_v2_golden.json -- bytes, decoded point count,
 D1 PSNR and the losslessly coded stride-2 geometry."""
 import json
@@ -14,14 +14,15 @@ PYREF = osp.join(ROOT, 'oracle', '_ref', 'pyref.zip')
 
 
 def reference_root(tmp_path_factory):
-    if osp.isdir('/root/reference/models'):
-        return '/root/reference'
+    from oracle import build_ref
+    if build_ref.REF_ROOT and osp.isdir(osp.join(build_ref.REF_ROOT, 'models')):
+        return build_ref.REF_ROOT
     if osp.isfile(PYREF):
         root = str(tmp_path_factory.mktemp('pyref'))
         with zipfile.ZipFile(PYREF) as z:
             z.extractall(root)
         return root
-    pytest.skip('reference Python not staged (run python oracle/build_ref.py where /root/reference exists)')
+    pytest.skip('reference Python not staged (set FASTPCC_REFERENCE_ROOT to a checkout of the reference, or run oracle/build_ref.py there)')
 
 
 def golden():

@@ -1,12 +1,19 @@
 """Pins the C restatement of the range coders (oracle/rans_oracle.c):
 (1) against the committed golden vectors minted from the compiled reference, and
-(2) byte-for-byte against the compiled reference itself (oracle/_ref) on random inputs, when present."""
+(2) byte-for-byte against the reference's outputs on seeded random inputs: the committed vectors of
+tests/golden/rans_random_golden.json, and the compiled reference itself (oracle/_ref) when it is built."""
+import json
+import os.path as osp
+
 import numpy as np
 import pytest
 
 from oracle import rans as orans
 from oracle import build_ref
-from tests.golden import rans_cases
+from tests.golden import rans_cases, rans_random_cases as R
+
+with open(osp.join(osp.dirname(__file__), 'golden', 'rans_random_golden.json')) as _f:
+    RANDOM_GOLDEN = json.load(_f)
 
 
 def test_oracle_matches_golden(rans_kat):
@@ -19,73 +26,49 @@ def test_oracle_matches_golden(rans_kat):
 
 
 def _ref():
+    """-> (simple_rans_ext_cpp, rans_ext_cpp), the reference's compiled coders, or None when they are not built"""
     s = build_ref.load_ref('simple_rans_ext_cpp')
     b = build_ref.load_ref('rans_ext_cpp')
-    if s is None or b is None:
-        pytest.skip('oracle/_ref not built (reference sources absent)')
-    return s, b
+    return (s, b) if s is not None and b is not None else None
 
 
-@pytest.mark.parametrize('seed', [0, 1, 2])
+@pytest.mark.parametrize('seed', R.SIMPLE_SEEDS)
 def test_simple_coder_vs_reference(seed):
-    s, _ = _ref()
-    rng = np.random.default_rng(seed)
-    enc_r, enc_o = s.RansEncoder(1 << 22), orans.RansEncoder(1 << 22)
-    calls = []
-    for _i in range(4):
-        n = int(rng.integers(1, 3000))
-        S = int(rng.integers(2, 300))
-        pm = rng.integers(1, 50, (n, S)) ** 2
-        pm = pm * (65536 - S) // pm.sum(1, keepdims=True) + 1
-        cdf = np.cumsum(pm, 1); cdf[:, -1] = 65535
-        cdf = cdf.astype(np.uint16)
-        if _i == 2:
-            cdf = cdf[:1]
-        sym = rng.integers(0, S, n).astype(np.uint16)
-        calls.append((cdf, sym))
-        assert enc_r.encode(cdf, sym) == enc_o.encode(cdf, sym)
-    br, bo = enc_r.flush(), enc_o.flush()
-    assert br == bo
-    dec_r, dec_o = s.RansDecoder(), orans.RansDecoder()
-    dec_r.flush(br); dec_o.flush(bo)
+    got, stream, calls = R.simple_coder(orans.RansEncoder, seed)
+    assert got == RANDOM_GOLDEN[f'simple_{seed}']
+    ref = _ref()
+    if ref is not None:
+        assert R.simple_coder(ref[0].RansEncoder, seed)[0] == got
+    decoders = [orans.RansDecoder()] + ([ref[0].RansDecoder()] if ref is not None else [])
+    for dec in decoders:
+        dec.flush(stream)
     for cdf, sym in reversed(calls):
-        a = np.zeros_like(sym); b = np.zeros_like(sym)
-        dec_r.decode(cdf, a); dec_o.decode(cdf, b)
-        assert (a == sym).all() and (b == sym).all()
+        for dec in decoders:
+            out = np.zeros_like(sym)
+            dec.decode(cdf, out)
+            assert (out == sym).all()
 
 
 @pytest.mark.parametrize('overflow', [True, False])
 def test_indexed_coder_vs_reference(overflow):
-    _, b = _ref()
-    rng = np.random.default_rng(11)
-    T, S, B, n = 7, 20, 3, 2500
-    pm = rng.random((T, S)) ** 3 + 1e-4
-    pm[1, 10:] = 0
-    off_r = np.full(T, -9, dtype=np.int32); off_o = off_r.copy()
-    cr, co = b.IndexedRansCoder(overflow, B), orans.IndexedRansCoder(overflow, B)
-    cr.init_with_pmfs(pm.copy(), off_r); co.init_with_pmfs(pm.copy(), off_o)
-    assert (off_r == off_o).all()
-    assert [list(c) for c in cr.get_cdfs()] == co.get_cdfs()
-    idx = rng.integers(0, T, (B, n)).astype(np.int32)
-    if overflow:
-        sym = np.round(rng.normal(0, 8, (B, n))).astype(np.int32)
-    else:
-        lens = np.array([len(c) - 1 for c in co.get_cdfs()])
-        sym = (rng.integers(0, 1 << 30, (B, n)) % lens[idx] + off_o[idx]).astype(np.int32)
-    er, eo = cr.encode_with_indexes(sym, idx), co.encode_with_indexes(sym, idx)
-    assert [bytes(x) for x in er] == eo
-    d = np.empty_like(sym); co.decode_with_indexes(eo, idx, d)
+    got, streams, (idx, sym) = R.indexed_coder(orans.IndexedRansCoder, overflow)
+    assert got == RANDOM_GOLDEN[f'indexed_overflow_{int(overflow)}']
+    ref = _ref()
+    if ref is not None:
+        assert R.indexed_coder(ref[1].IndexedRansCoder, overflow)[0] == got
+    co = orans.IndexedRansCoder(overflow, idx.shape[0])
+    co.init_with_quantized_cdfs(got['cdfs'], np.array(got['offsets'], dtype=np.int32))
+    d = np.empty_like(sym)
+    co.decode_with_indexes(streams, idx, d)
     assert (d == sym).all()
 
 
 def test_binary_coder_vs_reference():
-    _, b = _ref()
-    rng = np.random.default_rng(3)
-    B, n = 2, 30000
-    prob = np.clip(np.round(rng.random((B, n)) ** 2 * 65536), 1, 65535).astype(np.uint32)
-    sym = rng.random((B, n)) * 65536 < prob
-    er = b.BinaryRansCoder(B, 100).encode(sym, prob)
-    eo = orans.BinaryRansCoder(B, 100).encode(sym, prob)
-    assert [bytes(x) for x in er] == eo
-    d = np.empty_like(sym); orans.BinaryRansCoder(B).decode(eo, prob, d)
+    got, streams, (prob, sym) = R.binary_coder(orans.BinaryRansCoder)
+    assert got == RANDOM_GOLDEN['binary']
+    ref = _ref()
+    if ref is not None:
+        assert R.binary_coder(ref[1].BinaryRansCoder)[0] == got
+    d = np.empty_like(sym)
+    orans.BinaryRansCoder(sym.shape[0]).decode(streams, prob, d)
     assert (d == sym).all()

@@ -6,8 +6,8 @@ from tests import ref_import
 from fastpcc_b200 import me, space_filling_curves_ext, synth
 from tests.golden.lossy_cases import CASES, case_cloud
 from tests.golden.make_lossy_golden import run_case
-ref_root = '/root/reference'
-if not osp.isdir(ref_root + '/models'):
+ref_root = build_ref.REF_ROOT
+if not ref_root or not osp.isdir(ref_root + '/models'):
     ref_root = tempfile.mkdtemp(); zipfile.ZipFile(osp.join(ROOT, 'oracle/_ref/pyref.zip')).extractall(ref_root)
 ref = ref_import.import_reference_lossy_v2(ref_root, me, rans=build_ref.load_ref('rans_ext_cpp'), morton_ext=space_filling_curves_ext)
 case = CASES[0]

@@ -1,5 +1,5 @@
-import sys, time
-sys.path.insert(0, '/root/repo')
+import os, sys, time
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from fastpcc_b200 import synth
 from fastpcc_b200.lossl_coord_int import Config, Model
