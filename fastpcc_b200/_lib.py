@@ -53,6 +53,8 @@ SIGNATURES = {
     'fpcc_bytes_list_concat': (_i64, [_vp, _vp, _i, _vp, _i64]),
     'fpcc_bytes_list_split': (_i64, [_vp, _i64, _i, _vp, _vp]),
     'fpcc_nn_search': (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
+    'fpcc_knn_workspace': (_sz, [_i64, _i]),
+    'fpcc_knn_search': (_i, [_i, _i, _i, _vp, _i64, _i, _i, _i, _vp, _i64, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     'fpcc_gemm_i8': (_i, [_vp, _vp, _vp, _i, _vp, _i, _i, _i, _vp]),
     'fpcc_gather_gemm_scatter_i8': (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     'fpcc_requant': (_i, [_vp, _i64, _i, _EP, _vp, _vp]),

@@ -18,6 +18,7 @@
  *   models/convolutional/lossy_coord_v3/rans_coder/simple_rans_wrapper.cpp:272-286   RansEncoder / RansDecoder
  *   lib/entropy_models/rans_coder/rans_wrapper.cpp:430-451  IndexedRansCoder / BinaryRansCoder / batched_pmf_to_quantized_cdf
  *   models/convolutional/lossl_coord_int/model.py:261-295, 344-353, 81-91   get_bin / batch_quantize_pmf_torch / child generation
+ *   lib/knn3d/src/knn3d.cu:25,75                        KNearestNeighborKernelV0/V2 (fpcc_knn_search)
  */
 #ifndef FASTPCC_B200_H_
 #define FASTPCC_B200_H_
@@ -181,6 +182,26 @@ int64_t fpcc_bytes_list_split(const uint8_t *data, int64_t len, int n, int64_t *
  * idx_out[nq] (optional) = its row, the lowest row among equidistant ones. */
 int fpcc_nn_search(const int32_t *query, int nq, int q_ld, int q_col, const int32_t *ref, int nr, int r_ld, int r_col,
                    int coord_bits, int64_t *d2_out, int32_t *idx_out, void *stream);
+
+/* Exact K nearest neighbours, batched, on a uniform cell grid built on the reference rows inside the call (device
+ * reductions, cub radix sort, open-addressing cell table; no host round trip).  Replaces lib/knn3d/src/knn3d.cu
+ * (KNearestNeighborKernelV0/V2, brute force, float32, D = 3) and the search under pc_error
+ * (lib/metrics/pc_error_wrapper.py:40-106); metrics.pc_error runs on it with k = 1.
+ * coord_type 0: int32 coordinates, |c| < 2^30, dist_out int64 exact squared distances.  coord_type 1: finite float32
+ * coordinates, dist_out float32 = ((dx*dx + dy*dy) + dz*dz) with one rounding per operation (no FMA), so NumPy float32
+ * evaluating that expression gives the same bits.  Rows of q_ld / r_ld elements, xyz at column q_col / r_col.
+ * Batches: q_batch_col = r_batch_col = -1 is one cloud (n_batch must be 1); otherwise both columns hold the batch id
+ * (an int32, or for coord_type 1 a float32 holding an integer), queries match references of their own batch only,
+ * 1 <= n_batch <= 1023, and rows whose id lies outside [0, n_batch) are ignored (as queries they get padding).
+ * Output [nq, k] row-major, ascending by (distance, reference row): the lowest row wins among equal distances.
+ * idx_out holds reference rows of the call (not per-batch indices); slots beyond the batch's point count get idx -1,
+ * distance 0.  1 <= k <= 32; nq, nr < 2^31 (either may be 0).
+ * workspace: fpcc_knn_workspace(nr, n_batch) bytes (16-byte aligned or better). */
+size_t fpcc_knn_workspace(int64_t n_ref, int n_batch);
+int fpcc_knn_search(int coord_type, int k, int n_batch,
+                    const void *query, int64_t nq, int q_ld, int q_col, int q_batch_col,
+                    const void *ref, int64_t nr, int r_ld, int r_col, int r_batch_col,
+                    void *dist_out, int32_t *idx_out, void *workspace, size_t workspace_bytes, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
  * int8 GEMMs.  A [M,K] int8 row-major, B [N,K] int8 row-major (= one kernel offset's weight
