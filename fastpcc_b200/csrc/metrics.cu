@@ -9,6 +9,9 @@
 // lib/knn3d/src/knn3d.cu (KNearestNeighborKernelV0/V2) and, at K = 1, under metrics.pc_error.  O(N*K) for voxel
 // clouds instead of the O(N^2) of the brute force above, which stays as the workspace-free entry point and as the
 // on-device reference of the tests.
+//
+// All-ties nearest neighbour with attribute sums (fpcc_nn_tie_attr, DESIGN 3.7): the same grid and ring walk with a
+// collector that keeps every reference row at the least distance, for recolouring and pc_error's colour figures.
 #include <cub/cub.cuh>
 
 #include "common.cuh"
@@ -354,15 +357,23 @@ __global__ void __launch_bounds__(256) knn_cell_kernel(const T *ref, int nr, int
     if (last) hhi[slot] = i + 1;
 }
 
+// Collectors of the ring walk: begin (bind the outputs, empty), reset (empty), offer(distance, row), settled(bound, k)
+// (every unvisited point is at distance >= bound: may the walk stop?), store(query, k).
 template <typename T, int KB>
-struct KnnList {
+struct KnnList {  // the K best (distance, row) pairs, sorted in registers
     typedef typename KnnT<T>::D D;
+    struct Out {
+        D *dist;
+        int32_t *idx;
+    };
+    static constexpr int min_blocks = KB >= 16 ? 2 : 4;
     D d[KB];
     int r[KB];
     __device__ __forceinline__ void reset() {
 #pragma unroll
         for (int j = 0; j < KB; ++j) { d[j] = KnnT<T>::far(); r[j] = INT_MAX; }
     }
+    __device__ __forceinline__ void begin(const Out &) { reset(); }
     static __device__ __forceinline__ bool better(D da, int ra, D db, int rb) { return da < db || (da == db && ra < rb); }
     __device__ __forceinline__ void offer(D nd, int nr) {
         if (!better(nd, nr, d[KB - 1], r[KB - 1])) return;
@@ -375,22 +386,74 @@ struct KnnList {
         }
         if (better(nd, nr, d[0], r[0])) { d[0] = nd; r[0] = nr; }
     }
+    // K held and the bound strictly beyond the K-th distance: an equal distance at a lower row would still win
+    __device__ __forceinline__ bool settled(D bnd, int k) const {
+        D kd = d[0];  // the k-th best so far (the list is sorted: the last of the first k)
+        int kr = r[0];
+#pragma unroll
+        for (int j = 1; j < KB; ++j) {
+            kd = j < k ? d[j] : kd;
+            kr = j < k ? r[j] : kr;
+        }
+        return kr != INT_MAX && bnd > kd;
+    }
+    __device__ __forceinline__ void store(const Out &o, int q, int k) const {
+#pragma unroll
+        for (int j = 0; j < KB; ++j) {
+            if (j < k) {
+                const bool hit = r[j] != INT_MAX;
+                o.dist[(int64_t)q * k + j] = hit ? d[j] : (D)0;
+                o.idx[(int64_t)q * k + j] = hit ? r[j] : -1;
+            }
+        }
+    }
 };
 
-template <typename T, int KB>
-__global__ void __launch_bounds__(KNN_THREADS, KB >= 16 ? 2 : 4) knn_grid_search_kernel(
+// every reference row at the least distance (int32 rows): that distance, their number and the sums of their uint8
+// RGB rows.  Integer sums: the result does not depend on the order of the visit.
+struct KnnTie {
+    typedef unsigned long long D;
+    struct Out {
+        const uint8_t *rgb;
+        int64_t *d2;
+        int32_t *count;
+        int64_t *sum;
+    };
+    static constexpr int min_blocks = 4;
+    const uint8_t *__restrict__ rgb;
+    D best;
+    int n;
+    long long s0, s1, s2;
+    __device__ __forceinline__ void reset() { best = ~0ull; n = 0; s0 = s1 = s2 = 0; }
+    __device__ __forceinline__ void begin(const Out &o) { rgb = o.rgb; reset(); }
+    __device__ __forceinline__ void offer(D d, int row) {
+        if (d > best) return;
+        if (d < best) { best = d; n = 0; s0 = s1 = s2 = 0; }
+        const uint8_t *c = rgb + 3 * (int64_t)row;
+        ++n; s0 += __ldg(c); s1 += __ldg(c + 1); s2 += __ldg(c + 2);
+    }
+    // strictly beyond: a point at exactly `best` may still be unvisited
+    __device__ __forceinline__ bool settled(D bnd, int) const { return n > 0 && bnd > best; }
+    __device__ __forceinline__ void store(const Out &o, int q, int) const {
+        o.d2[q] = n ? (int64_t)best : 0;
+        o.count[q] = n;
+        o.sum[3 * (int64_t)q] = s0; o.sum[3 * (int64_t)q + 1] = s1; o.sum[3 * (int64_t)q + 2] = s2;
+    }
+};
+
+template <typename T, typename Coll>
+__global__ void __launch_bounds__(KNN_THREADS, Coll::min_blocks) knn_grid_search_kernel(
     const T *__restrict__ query, int nq, int ld, int col, int bcol, int nb, int k, const KnnBatch *__restrict__ bt,
     const typename KnnT<T>::P *__restrict__ pts, const unsigned long long *__restrict__ hkeys, const int32_t *__restrict__ hlo,
-    const int32_t *__restrict__ hhi, uint32_t cap, typename KnnT<T>::D *__restrict__ dist_out, int32_t *__restrict__ idx_out) {
+    const int32_t *__restrict__ hhi, uint32_t cap, const typename Coll::Out out) {
     typedef KnnT<T> C;
-    typedef typename C::D D;
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= nq) return;
     const T *qp = query + (int64_t)q * ld;
     const int b = knn_row_batch(qp, bcol, nb);
     const T qx = qp[col], qy = qp[col + 1], qz = qp[col + 2];
-    KnnList<T, KB> L;
-    L.reset();
+    Coll L;
+    L.begin(out);
     const int count = b < 0 ? 0 : bt[b].count;
     if (count > 0) {
         const int start = bt[b].start;
@@ -441,14 +504,7 @@ __global__ void __launch_bounds__(KNN_THREADS, KB >= 16 ? 2 : 4) knn_grid_search
                     if (qc[a] + r < nc[a] - 1) g = fmin(g, __dsub_rd((lo0[a] + (double)((qc[a] + r + 1) * step)) * e0p, qd[a]));
                 }
                 if (g == INFINITY) { done = true; break; }  // every cell of the batch visited
-                D kd = L.d[0];  // the k-th best so far (the list is sorted: the last of the first k)
-                int kr = L.r[0];
-#pragma unroll
-                for (int j = 1; j < KB; ++j) {
-                    kd = j < k ? L.d[j] : kd;
-                    kr = j < k ? L.r[j] : kr;
-                }
-                if (kr != INT_MAX && C::bound(g) > kd) { done = true; break; }
+                if (L.settled(C::bound(g), k)) { done = true; break; }
             }
         }
         if (!done) {  // small batch, or a query the rings did not settle: every point of the batch
@@ -459,31 +515,24 @@ __global__ void __launch_bounds__(KNN_THREADS, KB >= 16 ? 2 : 4) knn_grid_search
             }
         }
     }
-#pragma unroll
-    for (int j = 0; j < KB; ++j) {
-        if (j < k) {
-            const bool hit = L.r[j] != INT_MAX;
-            dist_out[(int64_t)q * k + j] = hit ? L.d[j] : (D)0;
-            idx_out[(int64_t)q * k + j] = hit ? L.r[j] : -1;
-        }
-    }
+    L.store(out, q, k);
 }
 
 static inline size_t knn_a256(size_t b) { return (b + 255) & ~(size_t)255; }
 static inline uint32_t knn_capacity(int64_t n_ref) { return (uint32_t)(2 * n_ref + 64); }
 
-template <typename T, int KB>
-static void knn_launch(const T *query, int nq, int ld, int col, int bcol, int nb, int k, const KnnBatch *bt, const void *pts,
-                       const unsigned long long *hkeys, const int32_t *hlo, const int32_t *hhi, uint32_t cap, void *dist,
-                       int32_t *idx, cudaStream_t s) {
-    knn_grid_search_kernel<T, KB><<<ceil_div(nq, KNN_THREADS), KNN_THREADS, 0, s>>>(
-        query, nq, ld, col, bcol, nb, k, bt, (const typename KnnT<T>::P *)pts, hkeys, hlo, hhi, cap,
-        (typename KnnT<T>::D *)dist, idx);
-}
+struct KnnGrid {  // the cell grid of the reference rows, in the workspace
+    KnnBatch *bt;
+    void *pts;
+    unsigned long long *hkeys;
+    int32_t *hlo, *hhi;
+    uint32_t cap;
+};
 
+// target: points per occupied cell (knn_level_kernel)
 template <typename T>
-static int knn_run(int k, int nb, const T *query, int nq, int q_ld, int q_col, int q_bcol, const T *ref, int nr, int r_ld,
-                   int r_col, int r_bcol, void *dist, int32_t *idx, void *workspace, size_t workspace_bytes, cudaStream_t s) {
+static int knn_build(int target, int nb, const T *ref, int nr, int r_ld, int r_col, int r_bcol, void *workspace,
+                     size_t workspace_bytes, cudaStream_t s, KnnGrid &g) {
     char *w = (char *)workspace;
     const uint32_t cap = knn_capacity(nr);
     KnnBatch *bt = (KnnBatch *)w; w += knn_a256((size_t)nb * sizeof(KnnBatch));
@@ -496,6 +545,7 @@ static int knn_run(int k, int nb, const T *query, int nq, int q_ld, int q_col, i
     int32_t *hlo = (int32_t *)w; w += knn_a256((size_t)cap * 4);
     int32_t *hhi = (int32_t *)w; w += knn_a256((size_t)cap * 4);
     size_t tmp_bytes = workspace_bytes - (size_t)(w - (char *)workspace);
+    g = KnnGrid{bt, pts, hkeys, hlo, hhi, cap};
     knn_init_kernel<<<ceil_div(nb, 256), 256, 0, s>>>(bt, nb);
     FPCC_LAUNCH_CHECK();
     if (nr > 0) {
@@ -506,16 +556,35 @@ static int knn_run(int k, int nb, const T *query, int nq, int q_ld, int q_col, i
         FPCC_LAUNCH_CHECK();
         FPCC_CUDA(cub::DeviceRadixSort::SortPairs(w, tmp_bytes, keys, keys_s, rows, rows_s, nr, 0, 64, s));
         knn_hist_kernel<<<ceil_div(nr, 256), 256, 0, s>>>(keys_s, nr, bt);
-        // points per occupied cell: a few for small K, about K/2 for large K (the 27 cells around a query then
-        // hold several times K points)
-        knn_level_kernel<<<1, 1024, 0, s>>>(bt, nb, k / 2 > 4 ? k / 2 : 4);
+        knn_level_kernel<<<1, 1024, 0, s>>>(bt, nb, target);
         knn_cell_kernel<T><<<ceil_div(nr, 256), 256, 0, s>>>(ref, nr, r_ld, r_col, keys_s, rows_s, bt,
                                                              (typename KnnT<T>::P *)pts, hkeys, hlo, hhi, cap);
         FPCC_LAUNCH_CHECK();
     }
+    return FPCC_OK;
+}
+
+template <typename T, typename Coll>
+static int knn_launch(const T *query, int nq, int ld, int col, int bcol, int nb, int k, const KnnGrid &g,
+                      const typename Coll::Out &out, cudaStream_t s) {
     if (nq == 0) return FPCC_OK;
+    knn_grid_search_kernel<T, Coll><<<ceil_div(nq, KNN_THREADS), KNN_THREADS, 0, s>>>(
+        query, nq, ld, col, bcol, nb, k, g.bt, (const typename KnnT<T>::P *)g.pts, g.hkeys, g.hlo, g.hhi, g.cap, out);
+    FPCC_LAUNCH_CHECK();
+    return FPCC_OK;
+}
+
+template <typename T>
+static int knn_run(int k, int nb, const T *query, int nq, int q_ld, int q_col, int q_bcol, const T *ref, int nr, int r_ld,
+                   int r_col, int r_bcol, void *dist, int32_t *idx, void *workspace, size_t workspace_bytes, cudaStream_t s) {
+    KnnGrid g;
+    // points per occupied cell: a few for small K, about K/2 for large K (the 27 cells around a query then hold several
+    // times K points)
+    const int rc = knn_build<T>(k / 2 > 4 ? k / 2 : 4, nb, ref, nr, r_ld, r_col, r_bcol, workspace, workspace_bytes, s, g);
+    if (rc != FPCC_OK) return rc;
+    typedef typename KnnT<T>::D D;
 #define FPCC_KNN_CASE(KB)                                                                                                   \
-    knn_launch<T, KB>(query, nq, q_ld, q_col, q_bcol, nb, k, bt, pts, hkeys, hlo, hhi, cap, dist, idx, s)
+    return knn_launch<T, KnnList<T, KB>>(query, nq, q_ld, q_col, q_bcol, nb, k, g, {(D *)dist, idx}, s)
     if (k <= 1) FPCC_KNN_CASE(1);
     else if (k <= 2) FPCC_KNN_CASE(2);
     else if (k <= 4) FPCC_KNN_CASE(4);
@@ -523,8 +592,6 @@ static int knn_run(int k, int nb, const T *query, int nq, int q_ld, int q_col, i
     else if (k <= 16) FPCC_KNN_CASE(16);
     else FPCC_KNN_CASE(32);
 #undef FPCC_KNN_CASE
-    FPCC_LAUNCH_CHECK();
-    return FPCC_OK;
 }
 
 static bool knn_layout_ok(int ld, int col, int bcol) {
@@ -565,28 +632,60 @@ extern "C" size_t fpcc_knn_workspace(int64_t n_ref, int n_batch) {
            knn_a256((size_t)n_ref * 16) + knn_a256(cap * 8) + 2 * knn_a256(cap * 4) + knn_a256(sort_tmp);
 }
 
+// the row checks of fpcc_knn_search and fpcc_nn_tie_attr, messages prefixed with the entry point's name
+static int knn_check_rows(const char *who, int n_batch, int64_t nq, int q_ld, int q_col, int q_batch_col, int64_t nr,
+                          int r_ld, int r_col, int r_batch_col) {
+    FPCC_REQUIRE(n_batch >= 1 && n_batch <= 1023, "%s: n_batch must be in 1..1023 (10-bit batch field of the cell keys), got %d",
+                 who, n_batch);
+    FPCC_REQUIRE(nq >= 0 && nr >= 0 && nq < ((int64_t)1 << 31) && nr < ((int64_t)1 << 31),
+                 "%s: row counts must be in 0..2^31-1 (nq=%lld nr=%lld)", who, (long long)nq, (long long)nr);
+    FPCC_REQUIRE((q_batch_col < 0) == (r_batch_col < 0), "%s: a batch column is needed on both sides or on neither", who);
+    FPCC_REQUIRE(q_batch_col >= 0 || n_batch == 1, "%s: one cloud (no batch column) needs n_batch = 1", who);
+    FPCC_REQUIRE(knn_layout_ok(q_ld, q_col, q_batch_col) && knn_layout_ok(r_ld, r_col, r_batch_col),
+                 "%s: bad row layout (q: ld %d col %d batch col %d, ref: ld %d col %d batch col %d)", who, q_ld, q_col,
+                 q_batch_col, r_ld, r_col, r_batch_col);
+    return FPCC_OK;
+}
+
+static int knn_check_workspace(const char *who, const void *workspace, size_t workspace_bytes, int64_t nr, int n_batch) {
+    FPCC_REQUIRE(((uintptr_t)workspace & 15) == 0, "%s: workspace must be 16-byte aligned", who);
+    const size_t need = fpcc_knn_workspace(nr, n_batch);
+    FPCC_REQUIRE(workspace_bytes >= need, "%s: workspace too small (%zu < %zu bytes)", who, workspace_bytes, need);
+    return FPCC_OK;
+}
+
 extern "C" int fpcc_knn_search(int coord_type, int k, int n_batch, const void *query, int64_t nq, int q_ld, int q_col,
                                int q_batch_col, const void *ref, int64_t nr, int r_ld, int r_col, int r_batch_col,
                                void *dist_out, int32_t *idx_out, void *workspace, size_t workspace_bytes, void *stream) {
     FPCC_REQUIRE(coord_type == 0 || coord_type == 1, "knn_search: coord_type must be 0 (int32) or 1 (float32), got %d", coord_type);
     FPCC_REQUIRE(k >= 1 && k <= 32, "knn_search: k must be in 1..32, got %d", k);
-    FPCC_REQUIRE(n_batch >= 1 && n_batch <= 1023, "knn_search: n_batch must be in 1..1023 (10-bit batch field of the cell keys), got %d",
-                 n_batch);
-    FPCC_REQUIRE(nq >= 0 && nr >= 0 && nq < ((int64_t)1 << 31) && nr < ((int64_t)1 << 31),
-                 "knn_search: row counts must be in 0..2^31-1 (nq=%lld nr=%lld)", (long long)nq, (long long)nr);
-    FPCC_REQUIRE((q_batch_col < 0) == (r_batch_col < 0), "knn_search: a batch column is needed on both sides or on neither");
-    FPCC_REQUIRE(q_batch_col >= 0 || n_batch == 1, "knn_search: one cloud (no batch column) needs n_batch = 1");
-    FPCC_REQUIRE(knn_layout_ok(q_ld, q_col, q_batch_col) && knn_layout_ok(r_ld, r_col, r_batch_col),
-                 "knn_search: bad row layout (q: ld %d col %d batch col %d, ref: ld %d col %d batch col %d)", q_ld, q_col,
-                 q_batch_col, r_ld, r_col, r_batch_col);
+    int rc = knn_check_rows("knn_search", n_batch, nq, q_ld, q_col, q_batch_col, nr, r_ld, r_col, r_batch_col);
+    if (rc != FPCC_OK) return rc;
     FPCC_REQUIRE(workspace && (nq == 0 || (query && dist_out && idx_out)) && (nr == 0 || ref), "knn_search: NULL pointer");
-    FPCC_REQUIRE(((uintptr_t)workspace & 15) == 0, "knn_search: workspace must be 16-byte aligned");
-    const size_t need = fpcc_knn_workspace(nr, n_batch);
-    FPCC_REQUIRE(workspace_bytes >= need, "knn_search: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+    rc = knn_check_workspace("knn_search", workspace, workspace_bytes, nr, n_batch);
+    if (rc != FPCC_OK) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     if (coord_type == 0)
         return knn_run<int32_t>(k, n_batch, (const int32_t *)query, (int)nq, q_ld, q_col, q_batch_col, (const int32_t *)ref,
                                 (int)nr, r_ld, r_col, r_batch_col, dist_out, idx_out, workspace, workspace_bytes, s);
     return knn_run<float>(k, n_batch, (const float *)query, (int)nq, q_ld, q_col, q_batch_col, (const float *)ref, (int)nr,
                           r_ld, r_col, r_batch_col, dist_out, idx_out, workspace, workspace_bytes, s);
+}
+
+extern "C" int fpcc_nn_tie_attr(int n_batch, const int32_t *query, int64_t nq, int q_ld, int q_col, int q_batch_col,
+                                const int32_t *ref, int64_t nr, int r_ld, int r_col, int r_batch_col, const uint8_t *ref_rgb,
+                                int64_t *d2_out, int32_t *count_out, int64_t *sum_out, void *workspace,
+                                size_t workspace_bytes, void *stream) {
+    int rc = knn_check_rows("nn_tie_attr", n_batch, nq, q_ld, q_col, q_batch_col, nr, r_ld, r_col, r_batch_col);
+    if (rc != FPCC_OK) return rc;
+    FPCC_REQUIRE(workspace && (nq == 0 || (query && d2_out && count_out && sum_out)) && (nr == 0 || (ref && ref_rgb)),
+                 "nn_tie_attr: NULL pointer");
+    rc = knn_check_workspace("nn_tie_attr", workspace, workspace_bytes, nr, n_batch);
+    if (rc != FPCC_OK) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    KnnGrid g;
+    rc = knn_build<int32_t>(4, n_batch, ref, (int)nr, r_ld, r_col, r_batch_col, workspace, workspace_bytes, s, g);  // the K = 1 cells
+    if (rc != FPCC_OK) return rc;
+    return knn_launch<int32_t, KnnTie>(query, (int)nq, q_ld, q_col, q_batch_col, n_batch, 1, g,
+                                       {ref_rgb, d2_out, count_out, sum_out}, s);
 }

@@ -3,13 +3,14 @@
 lib/metrics/pc_error_wrapper.py:40-106 as used by lib/evaluators.py:49-124; result keys are pc_error's own
 (the ones the reference's evaluator reads).  Nearest neighbours come from the cell-grid search fpcc_knn_search at
 K = 1 (exact, O(N)); the brute-force fpcc_nn_search stays available as `nn_search_bruteforce`, the on-device
-reference of the tests and the workspace-free C entry point."""
+reference of the tests and the workspace-free C entry point.  The colour figures (pc_error's `-c 1`) run on the
+all-ties search fpcc_nn_tie_attr (attributes.nearest_tie_attr)."""
 import math
 from typing import Callable, Dict, Optional
 
 import torch
 
-from . import _lib, knn3d
+from . import _lib, attributes, knn3d
 from .ops import _p, _s
 
 
@@ -55,14 +56,47 @@ def _psnr(mse: float, peak: float) -> float:
     return float('inf') if mse == 0 else 10.0 * math.log10(3.0 * peak * peak / mse)
 
 
+def _yuv(rgb: torch.Tensor) -> torch.Tensor:
+    """[n, 3] RGB in 0..255 (double) -> BT.709 YUV normalised to [0, 1]"""
+    r, g, b = rgb.double().unbind(1)
+    return torch.stack([(0.2126 * r + 0.7152 * g + 0.0722 * b) / 255,
+                        (-0.1146 * r - 0.3854 * g + 0.5 * b) / 255 + 0.5,
+                        (0.5 * r - 0.4542 * g - 0.0458 * b) / 255 + 0.5], 1)
+
+
+def _color_mse(a: torch.Tensor, a_rgb: torch.Tensor, b: torch.Tensor, b_rgb: torch.Tensor):
+    """per-channel YUV MSE over the points of a against the colour of b at each of them: the mean colour of every
+    point of b at the least distance"""
+    _, n, s = attributes.nearest_tie_attr(a[:, -3:], b[:, -3:], b_rgb)
+    return (_yuv(a_rgb) - _yuv(s.double() / n.double()[:, None])).square().mean(0).tolist()
+
+
+def _check_colors(rgb: torch.Tensor, xyz: torch.Tensor, what: str):
+    if rgb.dtype != torch.uint8 or tuple(rgb.shape) != (xyz.shape[0], 3) or rgb.device != xyz.device:
+        raise RuntimeError(f'pc_error: {what} must be uint8 [n,3] rows of the cloud, on its device')
+
+
 def pc_error(org: torch.Tensor, rec: torch.Tensor, resolution: float, org_normals: Optional[torch.Tensor] = None,
-             hausdorff: bool = False, search: Optional[Callable] = None) -> Dict[str, float]:
+             hausdorff: bool = False, search: Optional[Callable] = None, org_colors: Optional[torch.Tensor] = None,
+             rec_colors: Optional[torch.Tensor] = None) -> Dict[str, float]:
     """`mpeg_pc_error(infile1=org, infile2=rec, resolution)` for geometry: peak = resolution - 1
     (pc_error_wrapper.py:50).  1 = loop over org (A->B), 2 = loop over rec (B->A), F = symmetric = max of both.
     With `org_normals` (float [n_org,3]) the point-to-plane figures are added: the error vector of a pair is
     projected on the normal of its ORIGINAL point (for B->A: the normal of the nearest original point).
     `search`: the nearest-neighbour function, nn_search (cell grid) by default; nn_search_bruteforce gives the same
-    results by brute force."""
+    results by brute force.
+    With `org_colors` and `rec_colors` (uint8 [n,3] RGB rows of org / rec) pc_error's colour figures (`-c 1`) are
+    added: 1 = for every original point a, its colour against the colour of rec at a (the mean colour of all rec
+    points at the least distance from a), 2 = the mirror image, both in BT.709 YUV normalised to [0, 1]; per channel
+    'c[i],    1' = MSE and 'c[i],PSNR1' = 10 log10(1 / MSE), F = the larger MSE of 1 and 2.  Parity unpinned: the
+    pc_error source is not in the reference repository; pc_error keeps YUV in float32 where this keeps double, and by
+    default merges duplicate coordinates before averaging where this counts every row at the least distance once
+    (the same on duplicate-free clouds, such as everything frontend.voxelize and the decoders produce)."""
+    if (org_colors is None) != (rec_colors is None):
+        raise RuntimeError('pc_error: colours need both org_colors and rec_colors')
+    if org_colors is not None:
+        _check_colors(org_colors, org, 'org_colors')
+        _check_colors(rec_colors, rec, 'rec_colors')
     search = search or nn_search
     peak = float(resolution) - 1.0
     d_ab, i_ab = search(org, rec)
@@ -88,6 +122,13 @@ def pc_error(org: torch.Tensor, rec: torch.Tensor, resolution: float, org_normal
         out['mseF      (p2plane)'], out['mseF,PSNR (p2plane)'] = ef, _psnr(ef, peak)
     out['mse1+mse2 (p2point)'] = m1 + m2              # pc_error_wrapper.py:97-98
     out['mse1+mse2/2(p2point)'] = (m1 + m2) / 2
+    if org_colors is not None:
+        c1 = _color_mse(org, org_colors, rec, rec_colors)
+        c2 = _color_mse(rec, rec_colors, org, org_colors)
+        for tag, mse in (('1', c1), ('2', c2), ('F', [max(x, y) for x, y in zip(c1, c2)])):
+            for i, m in enumerate(mse):
+                psnr = float('inf') if m == 0 else 10.0 * math.log10(1.0 / m)
+                out[f'c[{i}],    {tag}'], out[f'c[{i}],PSNR{tag}'] = m, psnr
     return out
 
 

@@ -4,6 +4,7 @@ No datasets or trained checkpoints exist offline, so measurement and parity both
   * `lidar_frame`  -- S2 "lidar-120k": a 64-beam spinning-LiDAR model voxelised with exactly the
     dataset transform of the reference (lib/datasets/KITTIOdometry/dataset.py:90-102).
   * `surface_cloud` -- S1/S3 style voxelised shell surfaces on a 2^bits grid.
+  * `colored_surface` -- S4 style: a surface cloud with a smooth, noisy uint8 RGB field.
   * `make_lossl_int_state_dict` -- random int8 parameters for models/convolutional/lossl_coord_int,
     produced with the reference's own PTQ formulas (lib/int_sparse_conv/cuda_ops.py:223-301,
     487-503, 541-607) from seeded float weights and fixed activation scales, under the reference's
@@ -78,6 +79,19 @@ def surface_cloud(seed: int, bits: int = 10, n_target: int = 200000):
     if xyz.shape[0] > n_target:
         xyz = xyz[np.sort(rng.choice(xyz.shape[0], n_target, replace=False))]
     return xyz
+
+
+def colored_surface(seed: int, bits: int = 10, n_target: int = 200000):
+    """S4 "8iVFB-color" style: `surface_cloud` plus uint8 RGB = a low-frequency sinusoid field of position + N(0, 8)
+    noise, clipped to 0..255.  -> (xyz int32 [N,3], rgb uint8 [N,3])."""
+    xyz = surface_cloud(seed, bits, n_target)
+    rng = np.random.default_rng([seed, 404])
+    u = xyz.astype(np.float64) / float(1 << bits)                       # position in [0, 1)
+    freq = rng.uniform(1.0, 3.0, (3, 3))                                # cycles over the grid, per channel and axis
+    phase = rng.uniform(0.0, 2 * np.pi, (3, 3))
+    field = 128.0 + 40.0 * np.sin(2 * np.pi * u[:, None, :] * freq[None] + phase[None]).sum(2)
+    rgb = np.clip(np.rint(field + rng.normal(0.0, 8.0, field.shape)), 0, 255).astype(np.uint8)
+    return xyz, rgb
 
 
 def with_batch(xyz: np.ndarray, b: int = 0) -> np.ndarray:

@@ -203,6 +203,19 @@ int fpcc_knn_search(int coord_type, int k, int n_batch,
                     const void *ref, int64_t nr, int r_ld, int r_col, int r_batch_col,
                     void *dist_out, int32_t *idx_out, void *workspace, size_t workspace_bytes, void *stream);
 
+/* All-ties nearest neighbour with attribute sums, on the cell grid of fpcc_knn_search (same build at its k = 1 cell
+ * size, same workspace: fpcc_knn_workspace(nr, n_batch)).  int32 rows as coord_type 0 of fpcc_knn_search, |c| < 2^30,
+ * the same batch rules.  For every query row: d2_out[nq] int64 = d*, the least squared distance to a reference row of
+ * its batch; count_out[nq] int32 = the reference rows at exactly d*; sum_out[nq,3] int64 = the per-channel sums of
+ * their ref_rgb[nr,3] uint8 rows.  Integer sums: exact, independent of the visiting order.  A query whose batch has no
+ * reference row gets d2 0, count 0, sums 0.  Replaces the colour neighbour search of pc_error
+ * (lib/metrics/pc_error_wrapper.py:40-106) and the KNN recolour of
+ * models/convolutional/lossy_coord_lossy_color/layers.py:269-333 (metrics.pc_error colours, attributes.recolor). */
+int fpcc_nn_tie_attr(int n_batch, const int32_t *query, int64_t nq, int q_ld, int q_col, int q_batch_col,
+                     const int32_t *ref, int64_t nr, int r_ld, int r_col, int r_batch_col, const uint8_t *ref_rgb,
+                     int64_t *d2_out, int32_t *count_out, int64_t *sum_out, void *workspace, size_t workspace_bytes,
+                     void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * int8 GEMMs.  A [M,K] int8 row-major, B [N,K] int8 row-major (= one kernel offset's weight
  * C_out x C_in), int32 accumulation (exact; wraps, never saturates at the sizes in use).
