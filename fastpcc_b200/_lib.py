@@ -56,6 +56,7 @@ SIGNATURES = {
     'fpcc_knn_workspace': (_sz, [_i64, _i]),
     'fpcc_knn_search': (_i, [_i, _i, _i, _vp, _i64, _i, _i, _i, _vp, _i64, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     'fpcc_nn_tie_attr': (_i, [_i, _vp, _i64, _i, _i, _i, _vp, _i64, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'fpcc_knn_normals': (_i, [_i, _i, _vp, _i64, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     'fpcc_gemm_i8': (_i, [_vp, _vp, _vp, _i, _vp, _i, _i, _i, _vp]),
     'fpcc_gather_gemm_scatter_i8': (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     'fpcc_requant': (_i, [_vp, _i64, _i, _EP, _vp, _vp]),

@@ -357,7 +357,8 @@ __global__ void __launch_bounds__(256) knn_cell_kernel(const T *ref, int nr, int
     if (last) hhi[slot] = i + 1;
 }
 
-// Collectors of the ring walk: begin (bind the outputs, empty), reset (empty), offer(distance, row), settled(bound, k)
+// Collectors of the ring walk: begin (bind the outputs, empty), reset (empty), offer(distance, packed point),
+// settled(bound, k)
 // (every unvisited point is at distance >= bound: may the walk stop?), store(query, k).
 template <typename T, int KB>
 struct KnnList {  // the K best (distance, row) pairs, sorted in registers
@@ -375,7 +376,8 @@ struct KnnList {  // the K best (distance, row) pairs, sorted in registers
     }
     __device__ __forceinline__ void begin(const Out &) { reset(); }
     static __device__ __forceinline__ bool better(D da, int ra, D db, int rb) { return da < db || (da == db && ra < rb); }
-    __device__ __forceinline__ void offer(D nd, int nr) {
+    __device__ __forceinline__ void offer(D nd, const typename KnnT<T>::P &p) {
+        const int nr = KnnT<T>::row(p);
         if (!better(nd, nr, d[KB - 1], r[KB - 1])) return;
 #pragma unroll
         for (int j = KB - 1; j > 0; --j) {  // j > slot: shift down, j == slot: insert, j < slot: keep
@@ -426,8 +428,9 @@ struct KnnTie {
     long long s0, s1, s2;
     __device__ __forceinline__ void reset() { best = ~0ull; n = 0; s0 = s1 = s2 = 0; }
     __device__ __forceinline__ void begin(const Out &o) { rgb = o.rgb; reset(); }
-    __device__ __forceinline__ void offer(D d, int row) {
+    __device__ __forceinline__ void offer(D d, const int4 &p) {
         if (d > best) return;
+        const int row = p.w;
         if (d < best) { best = d; n = 0; s0 = s1 = s2 = 0; }
         const uint8_t *c = rgb + 3 * (int64_t)row;
         ++n; s0 += __ldg(c); s1 += __ldg(c + 1); s2 += __ldg(c + 2);
@@ -441,81 +444,269 @@ struct KnnTie {
     }
 };
 
+// The ring walk of one query (x, y, z) of batch b (b >= 0) over the grid, feeding every visited row to L.  rings false:
+// go straight to the scan of the whole batch.  Returns false when the walk ended in that scan, true when the rings
+// settled (or the rings visited every cell of the batch).
+template <typename T, typename Coll>
+__device__ __forceinline__ bool knn_walk(Coll &L, T qx, T qy, T qz, int b, int k, bool rings, const KnnBatch *__restrict__ bt,
+                                         const typename KnnT<T>::P *__restrict__ pts, const unsigned long long *__restrict__ hkeys,
+                                         const int32_t *__restrict__ hlo, const int32_t *__restrict__ hhi, uint32_t cap) {
+    typedef KnnT<T> C;
+    const int count = bt[b].count, start = bt[b].start;
+    if (rings && count > KNN_SCAN_MAX) {
+        const int lv = bt[b].level, e0 = bt[b].e0;
+        int64_t qc[3];
+        int nc[3];
+        double qd[3] = {(double)qx, (double)qy, (double)qz}, lo0[3];
+        const double s = knn_pow2(-e0);
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            const long long m = bt[b].minc[a];
+            // clamped far outside the grid: the gaps below stay valid bounds for such a query
+            const double rel = fmin(fmax(floor(qd[a] * s) - (double)m, -1099511627776.0), 1099511627776.0);
+            qc[a] = (int64_t)rel >> lv;
+            nc[a] = bt[b].ncell[a];
+            lo0[a] = (double)m;
+        }
+        const int64_t step = (int64_t)1 << lv;  // base cells per search cell
+        const double e0p = knn_pow2(e0);        // base cell edge
+        for (int r = 0; r <= KNN_RING_CAP; ++r) {
+            const int64_t x0 = max(qc[0] - r, (int64_t)0), x1 = min(qc[0] + r, (int64_t)nc[0] - 1);
+            const int64_t y0 = max(qc[1] - r, (int64_t)0), y1 = min(qc[1] + r, (int64_t)nc[1] - 1);
+            const int64_t z0 = max(qc[2] - r, (int64_t)0), z1 = min(qc[2] + r, (int64_t)nc[2] - 1);
+            for (int64_t x = x0; x <= x1; ++x) {
+                for (int64_t y = y0; y <= y1; ++y) {
+                    // shell columns on an x or y face: every z; inner columns (r >= 1): the two z faces
+                    const bool face = x == qc[0] - r || x == qc[0] + r || y == qc[1] - r || y == qc[1] + r;
+                    const int64_t zs = face ? 1 : 2 * r;
+                    for (int64_t z = face ? z0 : qc[2] - r; z <= (face ? z1 : qc[2] + r); z += zs) {
+                        if (z < z0 || z > z1) continue;
+                        const uint32_t slot = knn_hash_find(hkeys, cap, pack_key(b, (int)x, (int)y, (int)z));
+                        if (slot == 0xffffffffu) continue;
+                        const int e = __ldg(&hhi[slot]);
+                        for (int j = __ldg(&hlo[slot]); j < e; ++j) {
+                            const typename C::P p = pts[j];
+                            L.offer(C::dist(qx, qy, qz, p), p);
+                        }
+                    }
+                }
+            }
+            // least gap to a face of the visited box that still has cells behind it
+            double g = INFINITY;
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                if (qc[a] - r > 0) g = fmin(g, __dsub_rd(qd[a], (lo0[a] + (double)((qc[a] - r) * step)) * e0p));
+                if (qc[a] + r < nc[a] - 1) g = fmin(g, __dsub_rd((lo0[a] + (double)((qc[a] + r + 1) * step)) * e0p, qd[a]));
+            }
+            if (g == INFINITY) return true;  // every cell of the batch visited
+            if (L.settled(C::bound(g), k)) return true;
+        }
+    }
+    // small batch, or a query the rings did not settle: every point of the batch
+    L.reset();
+    for (int j = start; j < start + count; ++j) {
+        const typename C::P p = pts[j];
+        L.offer(C::dist(qx, qy, qz, p), p);
+    }
+    return false;
+}
+
 template <typename T, typename Coll>
 __global__ void __launch_bounds__(KNN_THREADS, Coll::min_blocks) knn_grid_search_kernel(
     const T *__restrict__ query, int nq, int ld, int col, int bcol, int nb, int k, const KnnBatch *__restrict__ bt,
     const typename KnnT<T>::P *__restrict__ pts, const unsigned long long *__restrict__ hkeys, const int32_t *__restrict__ hlo,
     const int32_t *__restrict__ hhi, uint32_t cap, const typename Coll::Out out) {
-    typedef KnnT<T> C;
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= nq) return;
     const T *qp = query + (int64_t)q * ld;
     const int b = knn_row_batch(qp, bcol, nb);
-    const T qx = qp[col], qy = qp[col + 1], qz = qp[col + 2];
     Coll L;
     L.begin(out);
-    const int count = b < 0 ? 0 : bt[b].count;
-    if (count > 0) {
-        const int start = bt[b].start;
-        bool done = false;
-        if (count > KNN_SCAN_MAX) {
-            const int lv = bt[b].level, e0 = bt[b].e0;
-            int64_t qc[3];
-            int nc[3];
-            double qd[3] = {(double)qx, (double)qy, (double)qz}, lo0[3];
-            const double s = knn_pow2(-e0);
+    if (b >= 0 && bt[b].count > 0) knn_walk<T, Coll>(L, qp[col], qp[col + 1], qp[col + 2], b, k, true, bt, pts, hkeys, hlo, hhi, cap);
+    L.store(out, q, k);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Point normals from all-ties K-neighbourhoods (fpcc_knn_normals, DESIGN 3.8), int32 rows, the query set = the
+// reference set.  Per query p: d_K = the K-th least squared distance to the rows of its own batch (KnnList walk);
+// N(p) = every row at distance <= d_K (KnnMoments walk); M = n sum d d^T - (sum d)(sum d)^T over the offsets d of N(p),
+// exact in 128-bit integers and rounded once to double; the normal = the unit eigenvector of M's least eigenvalue
+// (cyclic Jacobi in double), zero when n < 3 or rank M <= 1.
+// Bound: |c| < 2^30 (the search's own).  Then |d| < 2^31, every product d_i d_j < 2^62 fits int64, and with n < 2^31
+// rows sum d < 2^62, sum d_i d_j < 2^93, n sum d_i d_j and (sum d_i)(sum d_j) < 2^124: M fits signed 128 bits.
+typedef __int128 i128;
+typedef unsigned __int128 u128;
+
+// every row at distance <= lim: their number, the sums of their offsets and of the offsets' products
+struct KnnMoments {
+    typedef unsigned long long D;
+    static constexpr int min_blocks = 2;
+    int qx, qy, qz;
+    D lim;
+    int n;
+    long long s[3];
+    i128 m[6];  // xx, yy, zz, xy, xz, yz
+    __device__ __forceinline__ void reset() {
+        n = 0;
+        s[0] = s[1] = s[2] = 0;
 #pragma unroll
-            for (int a = 0; a < 3; ++a) {
-                const long long m = bt[b].minc[a];
-                // clamped far outside the grid: the gaps below stay valid bounds for such a query
-                const double rel = fmin(fmax(floor(qd[a] * s) - (double)m, -1099511627776.0), 1099511627776.0);
-                qc[a] = (int64_t)rel >> lv;
-                nc[a] = bt[b].ncell[a];
-                lo0[a] = (double)m;
-            }
-            const int64_t step = (int64_t)1 << lv;  // base cells per search cell
-            const double e0p = knn_pow2(e0);        // base cell edge
-            for (int r = 0; r <= KNN_RING_CAP; ++r) {
-                const int64_t x0 = max(qc[0] - r, (int64_t)0), x1 = min(qc[0] + r, (int64_t)nc[0] - 1);
-                const int64_t y0 = max(qc[1] - r, (int64_t)0), y1 = min(qc[1] + r, (int64_t)nc[1] - 1);
-                const int64_t z0 = max(qc[2] - r, (int64_t)0), z1 = min(qc[2] + r, (int64_t)nc[2] - 1);
-                for (int64_t x = x0; x <= x1; ++x) {
-                    for (int64_t y = y0; y <= y1; ++y) {
-                        // shell columns on an x or y face: every z; inner columns (r >= 1): the two z faces
-                        const bool face = x == qc[0] - r || x == qc[0] + r || y == qc[1] - r || y == qc[1] + r;
-                        const int64_t zs = face ? 1 : 2 * r;
-                        for (int64_t z = face ? z0 : qc[2] - r; z <= (face ? z1 : qc[2] + r); z += zs) {
-                            if (z < z0 || z > z1) continue;
-                            const uint32_t slot = knn_hash_find(hkeys, cap, pack_key(b, (int)x, (int)y, (int)z));
-                            if (slot == 0xffffffffu) continue;
-                            const int e = __ldg(&hhi[slot]);
-                            for (int j = __ldg(&hlo[slot]); j < e; ++j) {
-                                const typename C::P p = pts[j];
-                                L.offer(C::dist(qx, qy, qz, p), C::row(p));
-                            }
-                        }
-                    }
-                }
-                // least gap to a face of the visited box that still has cells behind it
-                double g = INFINITY;
-    #pragma unroll
-            for (int a = 0; a < 3; ++a) {
-                    if (qc[a] - r > 0) g = fmin(g, __dsub_rd(qd[a], (lo0[a] + (double)((qc[a] - r) * step)) * e0p));
-                    if (qc[a] + r < nc[a] - 1) g = fmin(g, __dsub_rd((lo0[a] + (double)((qc[a] + r + 1) * step)) * e0p, qd[a]));
-                }
-                if (g == INFINITY) { done = true; break; }  // every cell of the batch visited
-                if (L.settled(C::bound(g), k)) { done = true; break; }
+        for (int j = 0; j < 6; ++j) m[j] = 0;
+    }
+    __device__ __forceinline__ void offer(D d, const int4 &p) {
+        if (d > lim) return;
+        const long long dx = (long long)p.x - qx, dy = (long long)p.y - qy, dz = (long long)p.z - qz;
+        ++n; s[0] += dx; s[1] += dy; s[2] += dz;
+        m[0] += dx * dx; m[1] += dy * dy; m[2] += dz * dz; m[3] += dx * dy; m[4] += dx * dz; m[5] += dy * dz;
+    }
+    // strictly beyond: a row at exactly lim may still be unvisited
+    __device__ __forceinline__ bool settled(D bnd, int) const { return bnd > lim; }
+};
+
+// round-to-nearest-even conversion of a 128-bit integer (one rounding: the bits below the top 64 fold into a sticky
+// bit, which sits below the rounding position of a 64-bit value of more than 53 significant bits)
+__device__ __forceinline__ double knn_i128_to_double(i128 v) {
+    const bool neg = v < 0;
+    u128 u = neg ? (u128)0 - (u128)v : (u128)v;
+    const unsigned long long hi = (unsigned long long)(u >> 64);
+    double r;
+    if (hi == 0) {
+        r = __ull2double_rn((unsigned long long)u);
+    } else {
+        const int sh = 64 - __clzll((long long)hi);  // 1..64: u >> sh fits 64 bits
+        const u128 low = u & (((u128)1 << sh) - 1);
+        r = __ull2double_rn((unsigned long long)(u >> sh) | (low != 0)) * knn_pow2(sh);
+    }
+    return neg ? -r : r;
+}
+
+// a * b == c * c for 0 <= a, b, |c| < 2^127, in 256 bits
+__device__ __forceinline__ void knn_mul256(u128 a, u128 b, u128 &hi, u128 &lo) {
+    const unsigned long long a0 = (unsigned long long)a, a1 = (unsigned long long)(a >> 64);
+    const unsigned long long b0 = (unsigned long long)b, b1 = (unsigned long long)(b >> 64);
+    const u128 p00 = (u128)a0 * b0, p01 = (u128)a0 * b1, p10 = (u128)a1 * b0, p11 = (u128)a1 * b1;
+    const u128 mid = (p00 >> 64) + (unsigned long long)p01 + (unsigned long long)p10;  // < 3 * 2^64
+    lo = (u128)(unsigned long long)p00 | (mid << 64);
+    hi = p11 + (p01 >> 64) + (p10 >> 64) + (mid >> 64);
+}
+__device__ __forceinline__ bool knn_minor_zero(i128 a, i128 b, i128 c) {
+    const u128 uc = c < 0 ? (u128)0 - (u128)c : (u128)c;
+    u128 h1, l1, h2, l2;
+    knn_mul256((u128)a, (u128)b, h1, l1);
+    knn_mul256(uc, uc, h2, l2);
+    return h1 == h2 && l1 == l2;
+}
+
+constexpr int KNN_JACOBI_SWEEPS = 16;  // a cap: convergence is quadratic, a 3 x 3 matrix is expected to stop well before
+
+// eigenvector of the least eigenvalue of the symmetric a (xx, yy, zz, xy, xz, yz), cyclic Jacobi; unit length
+__device__ __forceinline__ void knn_least_eigvec(const double a[6], double &vx, double &vy, double &vz) {
+    double A[3][3] = {{a[0], a[3], a[4]}, {a[3], a[1], a[5]}, {a[4], a[5], a[2]}};
+    double V[3][3] = {{1, 0, 0}, {0, 1, 0}, {0, 0, 1}};
+    for (int sweep = 0; sweep < KNN_JACOBI_SWEEPS; ++sweep) {
+        bool rotated = false;
+#pragma unroll
+        for (int pq = 0; pq < 3; ++pq) {
+            const int P = pq == 2 ? 1 : 0, Q = pq == 0 ? 1 : 2;
+            const double apq = A[P][Q];
+            // negligible against both diagonal entries (relative to the eigenvalues they converge to)
+            if (fabs(apq) <= 1e-18 * sqrt(fabs(A[P][P]) * fabs(A[Q][Q])) || apq == 0.0) continue;
+            rotated = true;
+            const double theta = (A[Q][Q] - A[P][P]) / (2.0 * apq);
+            const double t = copysign(1.0, theta) / (fabs(theta) + sqrt(theta * theta + 1.0));
+            const double c = 1.0 / sqrt(t * t + 1.0), sn = t * c;
+            const int R = 3 - P - Q;
+            const double arp = A[R][P], arq = A[R][Q];
+            A[P][P] -= t * apq;
+            A[Q][Q] += t * apq;
+            A[P][Q] = A[Q][P] = 0.0;
+            A[R][P] = A[P][R] = c * arp - sn * arq;
+            A[R][Q] = A[Q][R] = sn * arp + c * arq;
+#pragma unroll
+            for (int i = 0; i < 3; ++i) {
+                const double vp = V[i][P], vq = V[i][Q];
+                V[i][P] = c * vp - sn * vq;
+                V[i][Q] = sn * vp + c * vq;
             }
         }
-        if (!done) {  // small batch, or a query the rings did not settle: every point of the batch
-            L.reset();
-            for (int j = start; j < start + count; ++j) {
-                const typename C::P p = pts[j];
-                L.offer(C::dist(qx, qy, qz, p), C::row(p));
+        if (!rotated) break;
+    }
+    // the least diagonal entry, the lowest index on a tie (selects, not a run-time index: the arrays stay in registers)
+    const bool m1 = A[1][1] < A[0][0];
+    const double l01 = m1 ? A[1][1] : A[0][0];
+    const bool m2 = A[2][2] < l01;
+    const double x = m2 ? V[0][2] : (m1 ? V[0][1] : V[0][0]);
+    const double y = m2 ? V[1][2] : (m1 ? V[1][1] : V[1][0]);
+    const double z = m2 ? V[2][2] : (m1 ? V[2][1] : V[2][0]);
+    const double inv = 1.0 / sqrt(x * x + y * y + z * z);
+    vx = x * inv; vy = y * inv; vz = z * inv;
+}
+
+struct KnnView {  // the orientation reference: use = 0 -> the largest component positive
+    double x, y, z;
+    int use;
+};
+
+template <int KB>
+__global__ void __launch_bounds__(KNN_THREADS, 2) knn_normals_kernel(
+    const int32_t *__restrict__ rows, int n, int ld, int col, int bcol, int nb, int k, const KnnBatch *__restrict__ bt,
+    const int4 *__restrict__ pts, const unsigned long long *__restrict__ hkeys, const int32_t *__restrict__ hlo,
+    const int32_t *__restrict__ hhi, uint32_t cap, KnnView view, float *__restrict__ normal_out) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n) return;
+    const int32_t *qp = rows + (int64_t)q * ld;
+    const int b = knn_row_batch(qp, bcol, nb);
+    const int qx = qp[col], qy = qp[col + 1], qz = qp[col + 2];
+    float *o = normal_out + 3 * (int64_t)q;
+    double nx = 0.0, ny = 0.0, nz = 0.0;
+    if (b >= 0) {  // the query is a row of its own batch: count >= 1
+        // phase 1: d_K (far when the batch has fewer than k rows: N(p) is then the whole batch)
+        KnnList<int32_t, KB> L;
+        L.reset();
+        const bool rings = knn_walk<int32_t>(L, qx, qy, qz, b, k, true, bt, pts, hkeys, hlo, hhi, cap);
+        unsigned long long dk = L.d[0];
+        int rk = L.r[0];
+#pragma unroll
+        for (int j = 1; j < KB; ++j) {
+            dk = j < k ? L.d[j] : dk;
+            rk = j < k ? L.r[j] : rk;
+        }
+        // phase 2: every row at <= d_K; a query whose phase 1 ended in the batch scan scans again
+        KnnMoments S;
+        S.qx = qx; S.qy = qy; S.qz = qz;
+        S.lim = rk == INT_MAX ? ~0ull : dk;
+        S.reset();
+        knn_walk<int32_t>(S, qx, qy, qz, b, k, rings, bt, pts, hkeys, hlo, hhi, cap);
+        if (S.n >= 3) {
+            const i128 nn = S.n;
+            i128 M[6];
+            M[0] = nn * S.m[0] - (i128)S.s[0] * S.s[0];
+            M[1] = nn * S.m[1] - (i128)S.s[1] * S.s[1];
+            M[2] = nn * S.m[2] - (i128)S.s[2] * S.s[2];
+            M[3] = nn * S.m[3] - (i128)S.s[0] * S.s[1];
+            M[4] = nn * S.m[4] - (i128)S.s[0] * S.s[2];
+            M[5] = nn * S.m[5] - (i128)S.s[1] * S.s[2];
+            // M is positive semidefinite: rank <= 1 exactly when every 2 x 2 principal minor vanishes
+            const bool flat = knn_minor_zero(M[0], M[1], M[3]) && knn_minor_zero(M[0], M[2], M[4]) &&
+                              knn_minor_zero(M[1], M[2], M[5]);
+            if (!flat) {
+                double a[6];
+#pragma unroll
+                for (int j = 0; j < 6; ++j) a[j] = knn_i128_to_double(M[j]);
+                knn_least_eigvec(a, nx, ny, nz);
+                bool flip;
+                if (view.use) {
+                    const double dot = nx * (view.x - (double)qx) + ny * (view.y - (double)qy) + nz * (view.z - (double)qz);
+                    flip = dot < 0.0;
+                } else {  // the component of largest magnitude positive, the lowest axis on a tie
+                    const bool y1 = fabs(ny) > fabs(nx);
+                    const double top = y1 ? ny : nx;
+                    flip = (fabs(nz) > fabs(top) ? nz : top) < 0.0;
+                }
+                if (flip) { nx = -nx; ny = -ny; nz = -nz; }
             }
         }
     }
-    L.store(out, q, k);
+    o[0] = (float)nx; o[1] = (float)ny; o[2] = (float)nz;
 }
 
 static inline size_t knn_a256(size_t b) { return (b + 255) & ~(size_t)255; }
@@ -574,13 +765,15 @@ static int knn_launch(const T *query, int nq, int ld, int col, int bcol, int nb,
     return FPCC_OK;
 }
 
+// cell size of the K-NN search: a few points per occupied cell for small K, about K/2 for large K (the 27 cells around
+// a query then hold several times K points)
+static inline int knn_target(int k) { return k / 2 > 4 ? k / 2 : 4; }
+
 template <typename T>
 static int knn_run(int k, int nb, const T *query, int nq, int q_ld, int q_col, int q_bcol, const T *ref, int nr, int r_ld,
                    int r_col, int r_bcol, void *dist, int32_t *idx, void *workspace, size_t workspace_bytes, cudaStream_t s) {
     KnnGrid g;
-    // points per occupied cell: a few for small K, about K/2 for large K (the 27 cells around a query then hold several
-    // times K points)
-    const int rc = knn_build<T>(k / 2 > 4 ? k / 2 : 4, nb, ref, nr, r_ld, r_col, r_bcol, workspace, workspace_bytes, s, g);
+    const int rc = knn_build<T>(knn_target(k), nb, ref, nr, r_ld, r_col, r_bcol, workspace, workspace_bytes, s, g);
     if (rc != FPCC_OK) return rc;
     typedef typename KnnT<T>::D D;
 #define FPCC_KNN_CASE(KB)                                                                                                   \
@@ -592,6 +785,25 @@ static int knn_run(int k, int nb, const T *query, int nq, int q_ld, int q_col, i
     else if (k <= 16) FPCC_KNN_CASE(16);
     else FPCC_KNN_CASE(32);
 #undef FPCC_KNN_CASE
+}
+
+static int knn_normals_run(int k, int nb, const int32_t *rows, int n, int ld, int col, int bcol, const KnnView &view,
+                           float *normal_out, void *workspace, size_t workspace_bytes, cudaStream_t s) {
+    KnnGrid g;
+    const int rc = knn_build<int32_t>(knn_target(k), nb, rows, n, ld, col, bcol, workspace, workspace_bytes, s, g);
+    if (rc != FPCC_OK) return rc;
+    if (n == 0) return FPCC_OK;
+#define FPCC_NORMALS_CASE(KB)                                                                                               \
+    knn_normals_kernel<KB><<<ceil_div(n, KNN_THREADS), KNN_THREADS, 0, s>>>(rows, n, ld, col, bcol, nb, k, g.bt,           \
+                                                                           (const int4 *)g.pts, g.hkeys, g.hlo, g.hhi,     \
+                                                                           g.cap, view, normal_out)
+    if (k <= 4) FPCC_NORMALS_CASE(4);
+    else if (k <= 8) FPCC_NORMALS_CASE(8);
+    else if (k <= 16) FPCC_NORMALS_CASE(16);
+    else FPCC_NORMALS_CASE(32);
+#undef FPCC_NORMALS_CASE
+    FPCC_LAUNCH_CHECK();
+    return FPCC_OK;
 }
 
 static bool knn_layout_ok(int ld, int col, int bcol) {
@@ -688,4 +900,23 @@ extern "C" int fpcc_nn_tie_attr(int n_batch, const int32_t *query, int64_t nq, i
     if (rc != FPCC_OK) return rc;
     return knn_launch<int32_t, KnnTie>(query, (int)nq, q_ld, q_col, q_batch_col, n_batch, 1, g,
                                        {ref_rgb, d2_out, count_out, sum_out}, s);
+}
+
+extern "C" int fpcc_knn_normals(int k, int n_batch, const int32_t *pts, int64_t n, int ld, int col, int batch_col,
+                                const double *viewpoint, float *normal_out, void *workspace, size_t workspace_bytes,
+                                void *stream) {
+    FPCC_REQUIRE(k >= 3 && k <= 32, "knn_normals: k must be in 3..32, got %d", k);
+    int rc = knn_check_rows("knn_normals", n_batch, n, ld, col, batch_col, n, ld, col, batch_col);
+    if (rc != FPCC_OK) return rc;
+    FPCC_REQUIRE(workspace && (n == 0 || (pts && normal_out)), "knn_normals: NULL pointer");
+    rc = knn_check_workspace("knn_normals", workspace, workspace_bytes, n, n_batch);
+    if (rc != FPCC_OK) return rc;
+    KnnView view = {0.0, 0.0, 0.0, 0};
+    if (viewpoint) {
+        FPCC_REQUIRE(isfinite(viewpoint[0]) && isfinite(viewpoint[1]) && isfinite(viewpoint[2]),
+                     "knn_normals: viewpoint must be three finite numbers");
+        view = KnnView{viewpoint[0], viewpoint[1], viewpoint[2], 1};
+    }
+    return knn_normals_run(k, n_batch, pts, (int)n, ld, col, batch_col, view, normal_out, workspace, workspace_bytes,
+                           (cudaStream_t)stream);
 }

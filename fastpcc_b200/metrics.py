@@ -78,11 +78,15 @@ def _check_colors(rgb: torch.Tensor, xyz: torch.Tensor, what: str):
 
 def pc_error(org: torch.Tensor, rec: torch.Tensor, resolution: float, org_normals: Optional[torch.Tensor] = None,
              hausdorff: bool = False, search: Optional[Callable] = None, org_colors: Optional[torch.Tensor] = None,
-             rec_colors: Optional[torch.Tensor] = None) -> Dict[str, float]:
+             rec_colors: Optional[torch.Tensor] = None, normals_k: Optional[int] = None) -> Dict[str, float]:
     """`mpeg_pc_error(infile1=org, infile2=rec, resolution)` for geometry: peak = resolution - 1
     (pc_error_wrapper.py:50).  1 = loop over org (A->B), 2 = loop over rec (B->A), F = symmetric = max of both.
     With `org_normals` (float [n_org,3]) the point-to-plane figures are added: the error vector of a pair is
     projected on the normal of its ORIGINAL point (for B->A: the normal of the nearest original point).
+    With `normals_k` (3..32) instead, those normals are estimated on the device from org itself:
+    attributes.estimate_normals(org[:, -3:], normals_k) (one cloud, as everywhere here; all-ties K-neighbourhood PCA,
+    the project's own definition, DESIGN 3.8; parity with the normals file MPEG pc_error reads is unpinned).  Passing
+    both raises.
     `search`: the nearest-neighbour function, nn_search (cell grid) by default; nn_search_bruteforce gives the same
     results by brute force.
     With `org_colors` and `rec_colors` (uint8 [n,3] RGB rows of org / rec) pc_error's colour figures (`-c 1`) are
@@ -97,6 +101,10 @@ def pc_error(org: torch.Tensor, rec: torch.Tensor, resolution: float, org_normal
     if org_colors is not None:
         _check_colors(org_colors, org, 'org_colors')
         _check_colors(rec_colors, rec, 'rec_colors')
+    if normals_k is not None:
+        if org_normals is not None:
+            raise RuntimeError('pc_error: pass org_normals or normals_k, not both')
+        org_normals = attributes.estimate_normals(org[:, -3:], normals_k)  # one cloud, as the searches
     search = search or nn_search
     peak = float(resolution) - 1.0
     d_ab, i_ab = search(org, rec)

@@ -216,6 +216,20 @@ int fpcc_nn_tie_attr(int n_batch, const int32_t *query, int64_t nq, int q_ld, in
                      int64_t *d2_out, int32_t *count_out, int64_t *sum_out, void *workspace, size_t workspace_bytes,
                      void *stream);
 
+/* Point normals from all-ties K-neighbourhoods (DESIGN 3.8), on the cell grid of fpcc_knn_search (same build at its
+ * k cell size, same workspace: fpcc_knn_workspace(n, n_batch)).  One set of int32 rows is both the query and the
+ * reference set: n rows of ld elements, xyz at column col, |c| < 2^30, batch id at batch_col (-1: one cloud, n_batch
+ * must be 1), the batch rules of fpcc_knn_search.  For every row p: d_K = the k-th least squared distance to the rows
+ * of its batch (p itself counts, at 0); N(p) = every row of the batch at distance <= d_K (the whole batch when it has
+ * fewer than k rows); M = n sum d d^T - (sum d)(sum d)^T over the offsets d of N(p), n = |N(p)|, exact in integers
+ * and rounded once to double; normal_out[n,3] float32 = the unit eigenvector of M's least eigenvalue, solved in
+ * double.  Zero vector when n < 3, when M has rank <= 1 (decided exactly), or when the batch id lies outside
+ * [0, n_batch).  Orientation: viewpoint NULL: the component of largest magnitude positive, the lowest axis on a tie;
+ * otherwise (three finite doubles in host memory, read during the call) normal . (viewpoint - p) >= 0.  The result
+ * is a function of the point set alone, not of the row order.  3 <= k <= 32; n < 2^31. */
+int fpcc_knn_normals(int k, int n_batch, const int32_t *pts, int64_t n, int ld, int col, int batch_col,
+                     const double *viewpoint, float *normal_out, void *workspace, size_t workspace_bytes, void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * int8 GEMMs.  A [M,K] int8 row-major, B [N,K] int8 row-major (= one kernel offset's weight
  * C_out x C_in), int32 accumulation (exact; wraps, never saturates at the sizes in use).
