@@ -22,40 +22,9 @@ def _newest_src():
     return t
 
 
-def build(force=False, verbose=False):
-    if not force and osp.isfile(SO) and osp.getmtime(SO) >= _newest_src():
-        return SO
+def _compile_and_link(out_dir, extra_flags=(), verbose=False):
+    """Compiles every source in parallel into out_dir/obj, writes out_dir/ptxas.log and links out_dir/libfastpcc_b200.so."""
     nvcc = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
-    os.makedirs(osp.join(OUT_DIR, 'obj'), exist_ok=True)
-    procs = []
-    objs = []
-    for src in SOURCES:
-        obj = osp.join(OUT_DIR, 'obj', src.replace('.cu', '.o'))
-        objs.append(obj)
-        # FPCC_NVCC_EXTRA: build-time experiment knobs, e.g. "-DFPCC_PAIRS_PRODUCER_WARPS=2" (use with force=True / -f)
-        cmd = [nvcc] + NVCC_FLAGS + os.environ.get('FPCC_NVCC_EXTRA', '').split() + ['-Xptxas', '-v', '-c', osp.join(CSRC, src), '-o', obj]
-        procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
-    log = []
-    for src, p in procs:
-        out, _ = p.communicate()
-        log.append(f'==== {src}\n{out}')
-        if p.returncode != 0:
-            sys.stderr.write(out)
-            raise RuntimeError(f'nvcc failed on {src}')
-    with open(osp.join(OUT_DIR, 'ptxas.log'), 'w') as f:
-        f.write('\n'.join(log))
-    if verbose:
-        print('\n'.join(log))
-    subprocess.run([nvcc, '-shared', '-o', SO] + objs, check=True)
-    return SO
-
-
-def build_variant(name, extra_flags):
-    """Experiment builds for A/B runs in ONE GPU call: the same sources with extra nvcc flags (e.g.
-    ['-DFPCC_PAIRS_PRODUCER_WARPS=2', '-DFPCC_EPI_TILE_DISPATCH=1']) into _C/variants/<name>/libfastpcc_b200.so,
-    selected at run time with FPCC_LIB_PATH (fastpcc_b200/_lib.py).  The default library is untouched."""
-    nvcc = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
-    out_dir = osp.join(OUT_DIR, 'variants', name)
     os.makedirs(osp.join(out_dir, 'obj'), exist_ok=True)
     procs, objs = [], []
     for src in SOURCES:
@@ -72,9 +41,24 @@ def build_variant(name, extra_flags):
             raise RuntimeError(f'nvcc failed on {src}')
     with open(osp.join(out_dir, 'ptxas.log'), 'w') as f:
         f.write('\n'.join(log))
+    if verbose:
+        print('\n'.join(log))
     so = osp.join(out_dir, 'libfastpcc_b200.so')
     subprocess.run([nvcc, '-shared', '-o', so] + objs, check=True)
     return so
+
+
+def build(force=False, verbose=False):
+    if not force and osp.isfile(SO) and osp.getmtime(SO) >= _newest_src():
+        return SO
+    return _compile_and_link(OUT_DIR, verbose=verbose)
+
+
+def build_variant(name, extra_flags):
+    """Diagnostic builds for A/B runs in ONE GPU call: the same sources with extra nvcc flags (e.g. ['-DFPCC_TC_TRACE'])
+    into _C/variants/<name>/libfastpcc_b200.so, selected at run time with FPCC_LIB_PATH (fastpcc_b200/_lib.py).  The
+    default library is untouched."""
+    return _compile_and_link(osp.join(OUT_DIR, 'variants', name), extra_flags)
 
 
 if __name__ == '__main__':

@@ -65,59 +65,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
         "WAIT_DONE:\n\t"
         "}" ::"r"(smem_u32(bar)), "r"(parity), "r"(0x989680u) : "memory");
 }
-// Wait of the 12-16 epilogue warps for the accumulator: test + nanosleep back-off instead of the blocking try_wait loop, so
-// that their polls do not take issue slots from the gather-producer warps (FPCC_EPI_SLEEP ns, 0 = plain mbar_wait).
-#ifndef FPCC_EPI_SLEEP
-#define FPCC_EPI_SLEEP 0
-#endif
-__device__ __forceinline__ void mbar_wait_epi(uint64_t *bar, uint32_t parity) {
-#if FPCC_EPI_SLEEP > 0
-    uint32_t done;
-    for (;;) {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-        if (done) break;
-        __nanosleep(FPCC_EPI_SLEEP);
-    }
-#else
-    mbar_wait(bar, parity);
-#endif
-}
-// ---- 2-CTA cluster helpers (weight tiles shared by TMA multicast, see CL2 below) ----
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t local_smem_addr, uint32_t rank) {  // same offset in CTA `rank` of the cluster
-    uint32_t a;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(local_smem_addr), "r"(rank));
-    return a;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t *bar, uint32_t parity) {  // acquire at cluster scope: sees the peer's DSMEM store
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "WAITC_LOOP:\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1, %2;\n\t"
-        "@p bra.uni WAITC_DONE;\n\t"
-        "bra.uni WAITC_LOOP;\n\t"
-        "WAITC_DONE:\n\t"
-        "}" ::"r"(smem_u32(bar)), "r"(parity), "r"(0x989680u) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-        ::"r"(dst), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(cta_mask) : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint64_t *bar, uint16_t cta_mask) {  // arrives on `bar` of every CTA in the mask
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
-}
 __device__ __forceinline__ void cp_async16(uint32_t dst, const void *src, uint32_t src_bytes) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
 }
@@ -351,9 +298,6 @@ __device__ __forceinline__ void ldg256(const void *p, int4 &lo, int4 &hi) {
     asm volatile("ld.global.nc.v8.s32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
                  : "=r"(lo.x), "=r"(lo.y), "=r"(lo.z), "=r"(lo.w), "=r"(hi.x), "=r"(hi.y), "=r"(hi.z), "=r"(hi.w) : "l"(p));
 }
-#ifndef FPCC_ST256
-#define FPCC_ST256 1
-#endif
 __device__ __forceinline__ int64_t pack64(uint32_t lo, uint32_t hi) {
     int64_t d;
     asm("mov.b64 %0, {%1, %2};" : "=l"(d) : "r"(lo), "r"(hi));
@@ -465,7 +409,6 @@ struct LeanU {
     uint32_t post2_addr;         // shared-space address of the staged second-stage constants (POST2 instantiations only):
                                  // words {mul2, thr2, slope2, shift2 - 32, c02 lo, c02 hi, nt2},  c02 = zp2 + 2^(shift2 - 1),
                                  // nt2 = 1 when the second stage cannot tie for any int32 input (no sign handling)
-    uint32_t nt_addr;            // shared-space address of the per-chunk tie-free flags (stage_nt_chunks)
     int64_t k24;                 // 2^24 - 1, read back from shared memory: ptxas splits an immediate or uniform 64-bit addend of
                                  // IMAD.WIDE into IADD3 + IMAD.X; a vector register pair stays the instruction's C operand
 };
@@ -513,44 +456,10 @@ __device__ __forceinline__ bool stage_channel(int32_t bias, uint32_t mul, int64_
     return ok;
 }
 
-// Measured on B200 (profiles/r02_epilogue_variants.txt): the per-chunk dispatch between the tie-free and the sign-exact body
-// costs more than the two instructions per element it saves (int8 linear 0.083 -> 0.096 ms: code size, spills at the
-// 80-register cap).  The first stage therefore keeps ONE sign-exact body; the flag remains a build-time experiment.  The
-// second stage of the fused [PReLU +] requant uses the tie analysis unconditionally (one CTA-uniform test, no extra body
-// per chunk).
-#ifndef FPCC_NT_SMEM
-#define FPCC_NT_SMEM 0
-#endif
-// Tie-free ("NT") chunks (epi_nt.cuh): when NO channel of a 16-channel chunk can produce a rounding tie inside the static
-// accumulator bound, rha(v*mul + zp, s) == (v*mul + zp + 2^(s-1)) >> s and the chunk needs no sign handling.  Called by a
-// whole warp for 32 consecutive channels (lane = channel; `valid` lanes hold a real channel, `ok` = the lean preconditions
-// of stage_channel hold); sets the per-chunk flags, the staged (bias, mul, thr) stay as they are.
-__device__ __forceinline__ void stage_nt_chunks(bool nt_on, bool valid, bool ok, int c, int32_t bias, uint32_t mul, int64_t zp, int shift,
-                                                int64_t abound, uint32_t *nt_flags) {
-    if (!nt_on) return;  // kernel-uniform
-    const int64_t ab = bias < 0 ? -(int64_t)bias : (int64_t)bias;
-    const bool nt = !valid || (ok && !tie_possible(mul, zp, shift, abound + ab));
-    const uint32_t b = __ballot_sync(0xffffffffu, nt);
-    const bool chunk_nt = ((b >> (threadIdx.x & 16)) & 0xffffu) == 0xffffu;
-    if (valid && (c & 15) == 0) nt_flags[c >> 4] = chunk_nt ? 1u : 0u;
-}
-
-// One tie-free chunk: (v * mul + c0) >> shift with the CTA-uniform c0 = zp + 2^(shift-1), no sign handling.  HI: shift >= 32
-// (arithmetic shift of the high word: one IMAD.HI + one SHF per element), else clamped funnel shift (shift <= 32).
-template <bool SLOPE, bool HI>
-__device__ __forceinline__ void lean_chunk_nt(const uint32_t (&acc)[EC], uint32_t chan_addr, const LeanU &u, int32_t (&o)[EC]) {
-    const int64_t c0 = pack64(u.c0_lo, u.c0_hi);
-#pragma unroll
-    for (int q = 0; q < EC; ++q) {
-        int32_t bias, mul;
-        asm volatile("ld.shared.v2.s32 {%0, %1}, [%2];" : "=r"(bias), "=r"(mul) : "r"(chan_addr + q * 16));
-        int32_t v = (int32_t)acc[q] + bias;
-        if (SLOPE) v = prelu_unit(v, u.slope, u.k24);
-        const int64_t t = HI ? mad_wide_c(v, mul, c0) : mad_wide(v, mul, c0);
-        o[q] = HI ? ((int32_t)(t >> 32) >> (u.shift - 32)) : (int32_t)__funnelshift_rc((uint32_t)t, (uint32_t)((uint64_t)t >> 32), u.shift);
-    }
-}
-
+// The first stage has ONE sign-exact body.  A second, tie-free body per 16-channel chunk (no sign handling where no channel
+// of the chunk can tie, epi_nt.cuh) was measured slower on B200: int8 linear 0.083 -> 0.096 ms from code size and spills at
+// the 80-register cap (profiles/r02_epilogue_variants.txt).  The fused second stage uses the tie analysis (one CTA-uniform
+// test, no extra body per chunk).
 template <int OUT, bool SLOPE, int SGN>
 __device__ __forceinline__ bool lean_chunk(const uint32_t (&acc)[EC], uint32_t chan_addr, const LeanU &u, int32_t (&o)[EC]) {
     bool bad = false;
@@ -689,16 +598,7 @@ __device__ __forceinline__ void lean_tile(const LeanTile &lt, const LeanU &u, in
             }
         }
         int32_t o[EC];
-        bool good = true;
-        constexpr bool NT_ON = FPCC_NT_SMEM && OUT == FPCC_OUT_I8 && !POST2;  // tie-free chunks (stage_nt_chunks), warp-uniform per chunk
-        bool nt = false;
-        if (NT_ON) {
-            uint32_t f;
-            asm volatile("ld.shared.u32 %0, [%1];" : "=r"(f) : "r"(u.nt_addr + (uint32_t)(c0 >> 4) * 4));
-            nt = f != 0u;
-        }
-        if (NT_ON && nt) lean_chunk_nt<SLOPE, SGN == SGN_HI0 || SGN == SGN_THR_HI>(acc, lt.chan_addr + (uint32_t)c0 * 16, u, o);
-        else good = lean_chunk<OUT, SLOPE, SGN>(acc, lt.chan_addr + (uint32_t)c0 * 16, u, o);
+        const bool good = lean_chunk<OUT, SLOPE, SGN>(acc, lt.chan_addr + (uint32_t)c0 * 16, u, o);
         if (OUT == FPCC_OUT_I32 && (SGN == SGN_LO0 || SGN == SGN_THR_LO)) {
             if (__any_sync(0xffffffffu, !good)) {  // warp-uniform, rare
                 if (held_valid) {  // the redo stores this chunk itself: flush the waiting even chunk of the pair first
@@ -729,10 +629,7 @@ __device__ __forceinline__ void lean_tile(const LeanTile &lt, const LeanU &u, in
                 const int4 k2 = lds128(u.post2_addr);          // mul2, thr2, slope2, shift2 - 32
                 const int4 k3 = lds128(u.post2_addr + 16);     // c02 lo, c02 hi, nt2
                 const int64_t c02 = pack64((uint32_t)k3.x, (uint32_t)k3.y), c02m1 = c02 - 1;
-#ifndef FPCC_NT2
-#define FPCC_NT2 1
-#endif
-                if (FPCC_NT2 && k3.z) {  // CTA-uniform: no int32 input can tie in the second stage, no sign handling
+                if (k3.z) {  // CTA-uniform: no int32 input can tie in the second stage, no sign handling
 #pragma unroll
                     for (int q = 0; q < EC; ++q) {
                         int32_t y = o[q];
@@ -745,16 +642,12 @@ __device__ __forceinline__ void lean_tile(const LeanTile &lt, const LeanU &u, in
                     for (int q = 0; q < EC; ++q) {
                         int32_t y = o[q];
                         if (SLOPE2) y = prelu_unit(y, k2.z, u.k24);
-#ifdef FPCC_POST2_ASM
-                        const int64_t t2 = mad_wide(y, k2.x, y < k2.y ? c02m1 : c02);
-#else
                         const int64_t t2 = mad_wide_c(y, k2.x, y < k2.y ? c02m1 : c02);
-#endif
                         o[q] = (int32_t)((uint64_t)t2 >> 32) >> k2.w;
                     }
                 }
             } else {
-                if (FPCC_ST256 && wide32) {  // 64 bytes of the int32 row: two whole sectors
+                if (wide32) {  // 64 bytes of the int32 row: two whole sectors
                     char *op = lt.orow + (size_t)c0 * esz;
                     stg256(op, o[0], o[1], o[2], o[3], o[4], o[5], o[6], o[7]);
                     stg256(op + 32, o[8], o[9], o[10], o[11], o[12], o[13], o[14], o[15]);
@@ -776,7 +669,7 @@ __device__ __forceinline__ void lean_tile(const LeanTile &lt, const LeanU &u, in
                 asm("cvt.pack.sat.s8.s32.b32 %0, %1, %2, %3;" : "=r"(up) : "r"(o[q + 3]), "r"(o[q + 2]), "r"(0));
                 asm("cvt.pack.sat.s8.s32.b32 %0, %1, %2, %3;" : "=r"(w[t]) : "r"(o[q + 1]), "r"(o[q]), "r"(up));
             }
-            if (FPCC_ST256 && wide8) {
+            if (wide8) {
                 // even chunk of a pair: hold its 16 bytes; odd chunk: one 32-byte store of both (a whole sector per lane)
                 if ((((c0 - lt.c_begin) >> 4) & 1) == 0 && c0 + EC < c_last) {
                     held[0] = w[0]; held[1] = w[1]; held[2] = w[2]; held[3] = w[3];
@@ -1021,16 +914,8 @@ __device__ __forceinline__ void epi_chunk_f(const uint32_t (&acc)[EC], const int
 // Fewer epilogue warps leave more issue slots (and registers: 128 / 96 / 80 per thread) to everyone else; the
 // gather-heavy conv prefers 12, the epilogue-bound linears 16.
 constexpr int EPI_WARPS_CONV = 12, EPI_WARPS_PAIRS = 16;
-// Gather-producer warps.  The conv needs a thread per output row (4 warps: per-row neighbour prefetch in registers).
-// The linears can run on 2 (each lane then issues 16 instead of 8 copies per stage): 16 + 2 + 2 = 20 warps put 5 warps
-// on every SM sub-partition, which lifts the register budget from 80 to 96 per thread (22 warps: 6 on one sub-partition,
-// 16384 / 192 = 85 -> 80).  Build-time experiment knob (-DFPCC_PAIRS_PRODUCER_WARPS=2); the default keeps 4.
-#ifndef FPCC_PAIRS_PRODUCER_WARPS
-#define FPCC_PAIRS_PRODUCER_WARPS 4
-#endif
-template <int MODE>
-constexpr int prod_warps() { return MODE == 1 ? FPCC_PAIRS_PRODUCER_WARPS : 4; }
-static_assert(FPCC_PAIRS_PRODUCER_WARPS == 4 || FPCC_PAIRS_PRODUCER_WARPS == 2, "producer warps: 2 or 4");
+// Gather-producer warps: a thread per output row of the tile (the conv keeps each row's neighbour indices in registers).
+constexpr int PROD_WARPS = TC_M / 32;
 
 struct PMeta {  // per-tile metadata, double buffered
     uint32_t kmask;
@@ -1070,16 +955,11 @@ __device__ __forceinline__ void pairs_tile_lookup(const TcArgs &a, int tile_m, P
 // one body the int8 linears lost 30 % to the pressure of the int32 quad code.
 enum { OK_I8 = 0, OK_I16 = 1, OK_I32 = 2, OK_POST2 = 3 };
 
-// CL2 (sparse conv only): the kernel runs as clusters of two CTAs.  CTA r of cluster c works on tile 2p + r of the tile
-// pairs p = c, c + n_clusters, ...; both follow the UNION of their two tiles' offset masks (row grouping makes adjacent
-// tiles nearly equal), each loads HALF of every weight tile and TMA-multicasts it into both CTAs' shared memory, so the
-// L2->SM weight bytes -- 69 % of the operand traffic of the L2-bound conv -- halve.  A stage is free when BOTH CTAs'
-// MMAs have consumed it: every tcgen05.commit arrives on the `empty` barrier of both CTAs.
-template <int MODE, int STAGES, int KIND, int EW, int OUTK, bool CL2>
-__global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_tc_persistent(TcArgs a, const __grid_constant__ CUtensorMap tmap_w,
+template <int MODE, int STAGES, int KIND, int EW, int OUTK>
+__global__ void __launch_bounds__((EW + PROD_WARPS + 2) * 32, 1) igemm_tc_persistent(TcArgs a, const __grid_constant__ CUtensorMap tmap_w,
                                                                     EpiParams ep, FEpi fe, void *__restrict__ out, int tiles_m,
                                                                     int tiles_n) {
-    constexpr int PW = prod_warps<MODE>(), PT = PW * 32;  // producer warps / threads
+    constexpr int PW = PROD_WARPS, PT = PW * 32;  // producer warps / threads
     constexpr int P_EPI_WARPS = EW, P_PROD_WARP0 = EW, P_TMA_WARP = EW + PW, P_MMA_WARP = EW + PW + 1, P_THREADS = (EW + PW + 2) * 32;
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = (uint8_t *)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -1095,28 +975,25 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
     uint64_t *bars = (uint64_t *)(thr_s + a.n_tile);
     uint64_t *full = bars, *empty = bars + STAGES;
     uint64_t *meta_full = bars + 2 * STAGES, *tmem_full = meta_full + 2, *tmem_empty = tmem_full + 2;
-    uint64_t *xchg = tmem_empty + 2;  // CL2: the peer's offset mask of a tile pair has arrived
+    // xchg, peer_kmask and nt_flags are unused: the layout is kept because every change to it, even deleting the nt_flags
+    // store below, alters register allocation and scheduling of all instances (DESIGN 3.5); compacting it needs a B200 A/B.
+    uint64_t *xchg = tmem_empty + 2;  // [2] unused (only initialised)
     uint64_t *meta_empty = xchg + 2;  // every reader of meta[slot] / rows[slot] of the slot's previous tile has taken its copy
     PMeta *meta = (PMeta *)(meta_empty + 2);
     uint32_t *tmem_ptr = (uint32_t *)(meta + 2);
     uint32_t *lean_off = tmem_ptr + 1;  // set once a staged channel block fails the lean-epilogue preconditions
-    uint32_t *peer_kmask = lean_off + 1;  // [2] CL2: written by the peer CTA through DSMEM
-    uint32_t *nt_flags = peer_kmask + 2;  // [16] tie-free flag of every 16-channel chunk of the staged block (stage_nt_chunks)
-    const uint32_t cl_rank = CL2 ? cluster_ctarank() : 0u;
-    // tile sequence of this CTA: p = p0, p0 + p_step, ... < p_end; tile = CL2 ? 2 p + rank : p
-    const int p0 = CL2 ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
-    const int p_step = CL2 ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+    uint32_t *peer_kmask = lean_off + 1;  // [2] unused
+    uint32_t *nt_flags = peer_kmask + 2;  // [16] unused (zeroed only)
+    const int tile0 = (int)blockIdx.x, tile_step = (int)gridDim.x;  // tiles of this CTA: tile0, tile0 + tile_step, ...
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int n_chunks = (a.K + TC_KB - 1) / TC_KB;
     const int total_tiles = tiles_m * tiles_n;
-    const int p_end = CL2 ? (total_tiles + 1) / 2 : total_tiles;
-#define FPCC_TILE_OF(p) (CL2 ? 2 * (p) + (int)cl_rank : (p))
 
     if (warp == P_MMA_WARP && lane == 0) {
         for (int s = 0; s < STAGES; ++s) {
             mbar_init(&full[s], PT + 1);
-            mbar_init(&empty[s], CL2 ? 2 : 1);
+            mbar_init(&empty[s], 1);
         }
         for (int b = 0; b < 2; ++b) {
             mbar_init(&meta_full[b], PT);
@@ -1137,7 +1014,7 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
     const int64_t zp_all = KIND == 0 ? ep.zp[0] : 0;
     int64_t vmax = 0;
     const int sgn_mode = KIND == 0 ? lean_mode(ep, zp_all, (int64_t)a.K * (MODE == 0 ? a.kvol : 1), ep.row_bias_bound, &vmax) : SGN_NONE;
-    if (tid >= 32 && tid < 48) nt_flags[tid - 32] = 0u;
+    if (tid >= 32 && tid < 48) nt_flags[tid - 32] = 0u;  // unused (see the carve-up above)
     if (tid == 0) {
         *lean_off = sgn_mode != SGN_NONE ? 0u : 1u;
         thr_s[0] = (1 << 24) - 1; thr_s[1] = 0;
@@ -1154,22 +1031,17 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
         }
     }
     __syncthreads();
-    // tie-free chunks: int8-output instances on the lean path (the int32 first stages sit at shifts 5..16 where ties are common)
-    const bool nt_on = FPCC_NT_SMEM && KIND == 0 && OUTK == OK_I8 && sgn_mode != SGN_NONE;
-    const int64_t abound = (int64_t)a.K * (MODE == 0 ? a.kvol : 1) * 16384 + (ep.row_bias ? (int64_t)ep.row_bias_bound : 0);  // |acc (+ row bias)|
     if (chan_static)
-        for (int cb = warp * 32; cb < a.n_tile; cb += P_THREADS) {  // warp-uniform trip count (stage_nt_chunks ballots)
+        for (int cb = warp * 32; cb < a.n_tile; cb += P_THREADS) {  // per-warp form kept: `c = tid; c += P_THREADS` changes the SASS
             const int c = cb + lane;
             const bool valid = c < a.n_tile;
             if (KIND == 0) {
                 const int32_t b = c < a.N && ep.bias ? ep.bias[c] : 0;
                 const uint32_t mu = c < a.N ? ep.mul[ep.mul_is_scalar ? 0 : c] : 0u;
-                bool ok = true;
                 if (valid) {
-                    ok = stage_channel(b, mu, zp_all, ep.shift, ep.out_type, vmax, &chan4_s[c]);
+                    const bool ok = stage_channel(b, mu, zp_all, ep.shift, ep.out_type, vmax, &chan4_s[c]);
                     if (!ok && sgn_mode != SGN_NONE) atomicOr(lean_off, 1u);
                 }
-                stage_nt_chunks(nt_on, valid, ok, c, b, mu, zp_all, ep.shift, abound, nt_flags);
             } else if (valid) {
                 chan_s[c] = make_int2(c < a.N && fe.bias ? __float_as_int(fe.bias[c]) : 0, 0);
             }
@@ -1177,7 +1049,6 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    if (CL2) cluster_sync_all();  // the peer's barriers are initialised before any remote arrive / multicast write
     const uint32_t tmem_base = *tmem_ptr;
 
     if (warp >= P_PROD_WARP0 && warp < P_PROD_WARP0 + PW) {
@@ -1196,9 +1067,8 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
 #pragma unroll
             for (int u = 0; u < PRE; ++u) nv[u] = (ok && u < a.kvol) ? __ldg(&a.nbr[(int64_t)u * a.ld + m]) : 0;
         };
-        if (pre) fetch(FPCC_TILE_OF(p0));
-        for (int p = p0; p < p_end; p += p_step, ++j) {
-            const int tile = FPCC_TILE_OF(p);
+        if (pre) fetch(tile0);
+        for (int tile = tile0; tile < total_tiles; tile += tile_step, ++j) {
             const int slot = j & 1;
             const int tile_m = tile / tiles_n;
             int32_t *rows = rows_s + slot * rows_k * TC_M;
@@ -1221,7 +1091,7 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
                             rows[u * TC_M + r] = nv[u] - 1;
                             mine |= (uint32_t)(nv[u] != 0) << u;
                         }
-                    fetch(FPCC_TILE_OF(p + p_step));
+                    fetch(tile + tile_step);
                 } else {
                     for (int k = 0; k < a.kvol; ++k) {
                         int32_t v = m < a.n_out ? __ldg(&a.nbr[(int64_t)k * a.ld + m]) : 0;
@@ -1234,33 +1104,11 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
             } else {
                 if (r == 0) { pairs_tile_lookup(a, tile_m, &meta[slot]); }
                 asm volatile("bar.sync 1, %0;" ::"n"(PT) : "memory");
-#if FPCC_PAIRS_PRODUCER_WARPS == 4  // the default build keeps the measured code verbatim (ptxas scheduling is sensitive here)
                 const int p = meta[slot].begin + r;
                 const bool ok = meta[slot].begin >= 0 && p < meta[slot].end;
                 rows[r] = ok ? (a.in_idx ? __ldg(&a.in_idx[p]) : p) : -1;
                 rows[TC_M + r] = ok ? (a.out_idx ? __ldg(&a.out_idx[p]) : p) : -1;
-#else
-#pragma unroll
-                for (int rr = r; rr < TC_M; rr += PT) {
-                    const int p = meta[slot].begin + rr;
-                    const bool ok = meta[slot].begin >= 0 && p < meta[slot].end;
-                    rows[rr] = ok ? (a.in_idx ? __ldg(&a.in_idx[p]) : p) : -1;
-                    rows[TC_M + rr] = ok ? (a.out_idx ? __ldg(&a.out_idx[p]) : p) : -1;
-                }
-#endif
                 if (r == 0) meta[slot].kmask = meta[slot].begin >= 0 && meta[slot].begin < meta[slot].end ? 1u : 0u;
-            }
-            if (CL2) {
-                // union of the pair's offset masks: own mask -> peer (DSMEM store + remote arrive), wait for the peer's
-                asm volatile("bar.sync 1, %0;" ::"n"(PT) : "memory");  // every warp's atomicOr has landed
-                if (r == 0) {
-                    const uint32_t own = *(volatile uint32_t *)&meta[slot].kmask;
-                    const uint32_t peer = cl_rank ^ 1u;
-                    asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(mapa_u32(smem_u32(&peer_kmask[slot]), peer)), "r"(own) : "memory");
-                    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(mapa_u32(smem_u32(&xchg[slot]), peer)) : "memory");
-                    mbar_wait_cluster(&xchg[slot], (j >> 1) & 1);
-                    meta[slot].kmask = own | *(volatile uint32_t *)&peer_kmask[slot];
-                }
             }
             __threadfence_block();
             mbar_arrive(&meta_full[slot]);
@@ -1276,7 +1124,6 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
                 // 8 consecutive lanes fetch the 8 16-byte pieces of ONE row (a full 128-byte line), 4 rows per
                 // instruction: 4 L1 wavefronts per LDGSTS instead of 32 with one row per lane.
                 // This lane serves rows base..base+7 (two 16-byte shared loads fetch their source rows).
-#if FPCC_PAIRS_PRODUCER_WARPS == 4
                 const int base = (r & ~31) + (lane >> 3) * 8;
                 const uint32_t rk = smem_u32(rows + (MODE == 0 ? k : 0) * TC_M + base);
                 const int4 s0 = lds128(rk), s1 = lds128(rk + 16);
@@ -1284,38 +1131,14 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
                 const int piece = lane & 7;
                 const bool k_ok = kc * TC_KB + piece * 16 < a.K;
                 const uint32_t dst0 = smem_u32(sA + stage * a_bytes);
-                {
 #pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const int32_t src = srcs[i];
-                        const int row = base + i;
-                        const bool ok = src >= 0 && k_ok;
-                        const int8_t *gsrc = a.A + (ok ? (int64_t)src * a.K + kc * TC_KB + piece * 16 : 0);
-                        cp_async16(dst0 + row * TC_KB + ((piece ^ (row & 7)) << 4), gsrc, ok ? 16u : 0u);
-                    }
+                for (int i = 0; i < 8; ++i) {
+                    const int32_t src = srcs[i];
+                    const int row = base + i;
+                    const bool ok = src >= 0 && k_ok;
+                    const int8_t *gsrc = a.A + (ok ? (int64_t)src * a.K + kc * TC_KB + piece * 16 : 0);
+                    cp_async16(dst0 + row * TC_KB + ((piece ^ (row & 7)) << 4), gsrc, ok ? 16u : 0u);
                 }
-#else
-                const int piece = lane & 7;
-                const bool k_ok = kc * TC_KB + piece * 16 < a.K;
-                const uint32_t dst0 = smem_u32(sA + stage * a_bytes);
-#pragma unroll
-                for (int h = 0; h < TC_M / PT; ++h) {  // two passes with half as many producer threads as rows
-                    const int base = (r & ~31) + (lane >> 3) * 8 + h * PT;
-                    const uint32_t rk = smem_u32(rows + (MODE == 0 ? k : 0) * TC_M + base);
-                    const int4 s0 = lds128(rk), s1 = lds128(rk + 16);
-                    const int32_t srcs[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
-                    {
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            const int32_t src = srcs[i];
-                            const int row = base + i;
-                            const bool ok = src >= 0 && k_ok;
-                            const int8_t *gsrc = a.A + (ok ? (int64_t)src * a.K + kc * TC_KB + piece * 16 : 0);
-                            cp_async16(dst0 + row * TC_KB + ((piece ^ (row & 7)) << 4), gsrc, ok ? 16u : 0u);
-                        }
-                    }
-                }
-#endif
                 // The stage's full barrier is signalled by the copy engine itself once this thread's copies have
                 // landed (no commit/wait lag in the producer): all STAGES stages can be in flight or queued.
                 asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(&full[stage])) : "memory");
@@ -1325,8 +1148,7 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
         // ================= weight producer (TMA) =================
         if (lane == 0) {
             int it = 0, j = 0;
-            for (int p = p0; p < p_end; p += p_step, ++j) {
-                const int tile = FPCC_TILE_OF(p);
+            for (int tile = tile0; tile < total_tiles; tile += tile_step, ++j) {
                 const int slot = j & 1;
                 const int n0 = (tile % tiles_n) * a.n_tile;
                 mbar_wait(&meta_full[slot], (j >> 1) & 1);
@@ -1341,13 +1163,7 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
                     mbar_wait(&empty[stage], ((it / STAGES) & 1) ^ 1);
                     mbar_expect_tx(&full[stage], (uint32_t)b_bytes);
                     const int wrow = (MODE == 0 ? k : group) * a.N + n0;
-                    if (CL2) {  // this CTA's half of the weight tile, into both CTAs (the peer sends the other half)
-                        const int half = a.n_tile >> 1;
-                        tma_load_2d_mc(smem_u32(sB + (size_t)stage * b_bytes + (size_t)cl_rank * half * TC_KB), &tmap_w, &full[stage],
-                                       kc * TC_KB, wrow + (int)cl_rank * half, (uint16_t)3);
-                    } else {
-                        tma_load_2d(smem_u32(sB + (size_t)stage * b_bytes), &tmap_w, &full[stage], kc * TC_KB, wrow);
-                    }
+                    tma_load_2d(smem_u32(sB + (size_t)stage * b_bytes), &tmap_w, &full[stage], kc * TC_KB, wrow);
                 }
             }
         }
@@ -1356,7 +1172,7 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
         if (lane == 0) {
             const uint32_t idesc = KIND == 0 ? umma_idesc_i8(a.n_tile) : umma_idesc_f16(a.n_tile, KIND == 2);
             int it = 0, j = 0;
-            for (int p = p0; p < p_end; p += p_step, ++j) {
+            for (int tile = tile0; tile < total_tiles; tile += tile_step, ++j) {
                 const int slot = j & 1;
                 mbar_wait(&meta_full[slot], (j >> 1) & 1);
                 const int total = __popc(meta[slot].kmask) * n_chunks;
@@ -1372,15 +1188,12 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
                     tc_fence_after();
                     const uint64_t ad = umma_desc_sw128(smem_u32(sA + stage * a_bytes));
                     const uint64_t bd = umma_desc_sw128(smem_u32(sB + (size_t)stage * b_bytes));
-                    {
 #pragma unroll
-                        for (int q = 0; q < TC_KB / 32; ++q) {  // 32 bytes of K per instruction for both kinds
-                            if (KIND == 0) umma_i8(tacc, ad + 2 * q, bd + 2 * q, idesc, (uint32_t)(i > 0 || q > 0));
-                            else umma_f16(tacc, ad + 2 * q, bd + 2 * q, idesc, (uint32_t)(i > 0 || q > 0));
-                        }
+                    for (int q = 0; q < TC_KB / 32; ++q) {  // 32 bytes of K per instruction for both kinds
+                        if (KIND == 0) umma_i8(tacc, ad + 2 * q, bd + 2 * q, idesc, (uint32_t)(i > 0 || q > 0));
+                        else umma_f16(tacc, ad + 2 * q, bd + 2 * q, idesc, (uint32_t)(i > 0 || q > 0));
                     }
-                    if (CL2) umma_commit_mc(&empty[stage], (uint16_t)3);  // the stage is free once BOTH CTAs consumed it
-                    else umma_commit(&empty[stage]);
+                    umma_commit(&empty[stage]);
                 }
                 TRACE(j, 4);
                 if (total > 0) umma_commit(&tmem_full[slot]);
@@ -1407,16 +1220,15 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
             lu.ovf_lim = shift <= 31 ? (1u << shift) - 1u : 0xffffffffu;
         }
         lu.post2_addr = smem_u32(thr_s + 4);
-        lu.nt_addr = smem_u32(nt_flags);
         const bool post2_on = KIND == 0 && OUTK == OK_POST2;
         // Output rows of grouped convs (row_perm): fetched ONE TILE AHEAD -- the dependent global load sat on the tile
         // boundary of every epilogue warp (~1 us per tile in the FPCC_TC_TRACE timeline).
         const bool use_perm = MODE == 0 && a.row_perm != nullptr;
         constexpr bool QUAD = KIND == 0 && OUTK == OK_I32;
         int32_t pm_next = 0, qpm_next[4] = {0, 0, 0, 0};
-        auto perm_fetch = [&](int pp) {
-            if (pp >= p_end) return;
-            const int64_t base = (int64_t)(FPCC_TILE_OF(pp) / tiles_n) * TC_M;
+        auto perm_fetch = [&](int t) {
+            if (t >= total_tiles) return;
+            const int64_t base = (int64_t)(t / tiles_n) * TC_M;
             if (base + r < a.n_out) pm_next = __ldg(&a.row_perm[base + r]);
             if (QUAD) {
 #pragma unroll
@@ -1426,49 +1238,37 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
                 }
             }
         };
-        if (use_perm) perm_fetch(p0);
-        int64_t staged_key = -1;  // (bias block, channel block) whose constants are staged
+        if (use_perm) perm_fetch(tile0);
         int j = 0;
-        for (int p = p0; p < p_end; p += p_step, ++j) {
-            const int tile = FPCC_TILE_OF(p);
+        for (int tile = tile0; tile < total_tiles; tile += tile_step, ++j) {
             const int slot = j & 1;
             const int tile_m = tile / tiles_n, n0 = (tile % tiles_n) * a.n_tile;
             const int32_t pm = pm_next;
             int32_t qpm[4];
 #pragma unroll
             for (int i = 0; i < 4; ++i) qpm[i] = qpm_next[i];
-            if (use_perm) perm_fetch(p + p_step);
-            mbar_wait_epi(&meta_full[slot], (j >> 1) & 1);
+            if (use_perm) perm_fetch(tile + tile_step);
+            mbar_wait(&meta_full[slot], (j >> 1) & 1);
             const bool have_acc = meta[slot].kmask != 0;
             const int pbase = (MODE == 1 && a.bias_per_group) ? meta[slot].group * a.N : 0;
-            // grouped weights / several channel blocks: restage (bias, mul) of this tile's block.  Restaging only when the
-            // block changes (the tiles of a weight group are consecutive: 8 restages per CTA for a C -> 8C selection linear)
-            // measured SLOWER on B200 -- selection linear with the fused second stage 0.203 -> 0.310 ms: without the two
-            // CTA-wide barriers per tile the 16 epilogue warps reach the accumulator wait early and their mbarrier polls take
-            // issue slots from the four gather-producer warps these kernels are bound by (profiles/r02_sel_linear_variants.txt).
-            // FPCC_RESTAGE_SKIP keeps the experiment.
-            const int64_t stage_key = ((int64_t)pbase << 20) | (int64_t)n0;
-#ifdef FPCC_RESTAGE_SKIP
-            const bool restage = !chan_static && stage_key != staged_key;
-#else
-            const bool restage = !chan_static;
-#endif
-            staged_key = stage_key;
-            if (restage) {
+            // grouped weights / several channel blocks: restage (bias, mul) of this tile's block, on every tile.  Restaging
+            // only when the block changes measured SLOWER on B200 -- selection linear with the fused second stage 0.203 ->
+            // 0.310 ms: without the two CTA-wide barriers per tile the 16 epilogue warps reach the accumulator wait early and
+            // their mbarrier polls take issue slots from the four gather-producer warps these kernels are bound by
+            // (profiles/r02_sel_linear_variants.txt).
+            if (!chan_static) {
                 asm volatile("bar.sync 2, %0;" ::"n"(P_EPI_WARPS * 32) : "memory");  // every epilogue warp is done with the previous tile's values
                 const int t = warp * 32 + lane;
-                if (warp * 32 < a.n_tile) {  // warp-uniform (stage_nt_chunks ballots); n_tile <= 256 <= 32 * epilogue warps
+                if (warp * 32 < a.n_tile) {  // n_tile <= 256 <= 32 * epilogue warps
                     const bool valid = t < a.n_tile;
                     const int pc = pbase + min(n0 + t, a.N - 1);
                     if (KIND == 0) {
                         const int32_t b = ep.bias ? __ldg(&ep.bias[pc]) : 0;
                         const uint32_t mu = __ldg(&ep.mul[ep.mul_is_scalar ? 0 : pc]);
-                        bool ok = true;
                         if (valid) {
-                            ok = stage_channel(b, mu, zp_all, ep.shift, ep.out_type, vmax, &chan4_s[t]);
+                            const bool ok = stage_channel(b, mu, zp_all, ep.shift, ep.out_type, vmax, &chan4_s[t]);
                             if (!ok && sgn_mode != SGN_NONE) atomicOr(lean_off, 1u);
                         }
-                        stage_nt_chunks(nt_on, valid, ok, t, b, mu, zp_all, ep.shift, abound, nt_flags);
                     } else if (valid) {
                         chan_s[t] = make_int2(fe.bias ? __float_as_int(__ldg(&fe.bias[pc])) : 0, 0);
                     }
@@ -1508,7 +1308,7 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
             // this warp holds its copies of meta[slot] / rows[slot]: the producers may build tile j+2 in the slot
             __syncwarp();
             if (lane == 0) mbar_arrive(&meta_empty[slot]);
-            mbar_wait_epi(&tmem_full[slot], (j >> 1) & 1);
+            mbar_wait(&tmem_full[slot], (j >> 1) & 1);
             tc_fence_after();
             if (tid == 0) TRACE(j, 5);
             const uint32_t tacc = tmem_base + (uint32_t)(slot * a.tmem_cols) + ((uint32_t)(quarter * 32) << 16);
@@ -1583,11 +1383,9 @@ __global__ void __launch_bounds__((EW + prod_warps<MODE>() + 2) * 32, 1) igemm_t
     }
     tc_fence_before();
     __syncthreads();
-    if (CL2) cluster_sync_all();  // no CTA leaves while its peer may still multicast into it or arrive on its barriers
     if (warp == P_MMA_WARP) {
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(2 * a.tmem_cols)) : "memory");
     }
-#undef FPCC_TILE_OF
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1699,48 +1497,16 @@ static int pick_tile(int N, int *n_tile, int *tmem_cols) {
 constexpr size_t TC_SMEM_MAX = 227 * 1024;
 template <int MODE, int STAGES, int KIND, int OUTK>
 static int launch_outk(const TcArgs &a, const CUtensorMap &tmap, const EpiParams &ep, const FEpi &fe, void *out, int tiles_m,
-                       int n_blocks_n, int grid, size_t smem, bool cl2, cudaStream_t s) {
+                       int n_blocks_n, int grid, size_t smem, cudaStream_t s) {
     // Epilogue warps per kernel instance.  The register file splits over four sub-partitions: 12 + 6 warps get 96 registers
     // per thread, 16 + 6 warps 80, 8 + 6 warps 128.  The int32-output instances (quad layout, residual prefetch) spill at 96 / 80
     // and run faster on FEWER warps with more registers (ResBlock conv2: 0.354 -> 0.307 ms with 8, 0.371 ms with 16;
     // profiles/r02_epilogue_warps.txt).
-#ifndef FPCC_CONV2_EW
-#define FPCC_CONV2_EW 8
-#endif
-#ifndef FPCC_LIN32_EW
-#define FPCC_LIN32_EW 8
-#endif
-#ifndef FPCC_LINP2_EW
-#define FPCC_LINP2_EW 8
-#endif
-#ifndef FPCC_CONV1_EW
-#define FPCC_CONV1_EW EPI_WARPS_CONV
-#endif
-#ifndef FPCC_LIN8_EW
-#define FPCC_LIN8_EW EPI_WARPS_PAIRS
-#endif
-    constexpr int EW = KIND != 0 ? (MODE == 0 ? EPI_WARPS_CONV : EPI_WARPS_PAIRS)
-                       : MODE == 0 ? ((OUTK == OK_I32 || OUTK == OK_POST2) ? FPCC_CONV2_EW : FPCC_CONV1_EW)
-                                   : (OUTK == OK_I32 ? FPCC_LIN32_EW : (OUTK == OK_POST2 ? FPCC_LINP2_EW : FPCC_LIN8_EW));
+    constexpr bool I32_OUT = KIND == 0 && (OUTK == OK_I32 || OUTK == OK_POST2);
+    constexpr int EW = I32_OUT ? 8 : (MODE == 0 ? EPI_WARPS_CONV : EPI_WARPS_PAIRS);
     constexpr int OK = KIND == 0 ? OUTK : OK_I8;
-    constexpr int THREADS = (EW + prod_warps<MODE>() + 2) * 32;
-    if (MODE == 0 && KIND == 0 && cl2) {  // 2-CTA clusters sharing every weight tile (see CL2 at the kernel)
-        auto kern = igemm_tc_persistent<MODE, STAGES, KIND, EW, OK, (MODE == 0 && KIND == 0)>;
-        static bool configured = false;
-        if (!configured) {
-            FPCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_MAX));
-            configured = true;
-        }
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        FPCC_CUDA(cudaLaunchKernelEx(&cfg, kern, a, tmap, ep, fe, out, tiles_m, n_blocks_n));
-        return FPCC_OK;
-    }
-    auto kern = igemm_tc_persistent<MODE, STAGES, KIND, EW, OK, false>;
+    constexpr int THREADS = (EW + PROD_WARPS + 2) * 32;
+    auto kern = igemm_tc_persistent<MODE, STAGES, KIND, EW, OK>;
     static bool configured = false;
     if (!configured) {
         FPCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_MAX));
@@ -1753,26 +1519,14 @@ static int launch_outk(const TcArgs &a, const CUtensorMap &tmap, const EpiParams
 
 template <int MODE, int STAGES, int KIND>
 static int launch_stages(const TcArgs &a, const CUtensorMap &tmap, const EpiParams &ep, const FEpi &fe, void *out, int tiles_m,
-                         int n_blocks_n, int grid, int rows_k, bool cl2, cudaStream_t s) {
+                         int n_blocks_n, int grid, int rows_k, cudaStream_t s) {
     size_t smem = PSmem<STAGES>::bytes(a.n_tile, rows_k);
     FPCC_REQUIRE(smem <= TC_SMEM_MAX, "igemm_tc: %zu bytes of shared memory exceed the 227 KB limit", smem);
-    if (KIND != 0) return launch_outk<MODE, STAGES, KIND, OK_I8>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, smem, cl2, s);
-    if (ep.post_mul && !ep.aux_out) return launch_outk<MODE, STAGES, KIND, OK_POST2>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, smem, cl2, s);
-    if (ep.out_type == FPCC_OUT_I8) return launch_outk<MODE, STAGES, KIND, OK_I8>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, smem, cl2, s);
-    if (ep.out_type == FPCC_OUT_I32) return launch_outk<MODE, STAGES, KIND, OK_I32>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, smem, cl2, s);
-    return launch_outk<MODE, STAGES, KIND, OK_I16>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, smem, cl2, s);
-}
-
-// Measured on B200 (391 k rows, C = 256, grouped 3x3x3): 0.222 ms with the clusters against 0.199 ms without -- the
-// lock-step of the pair costs more than the halved weight reads save (the conv is not L2->SM bandwidth bound after all).
-// Kept as an experiment: FPCC_CL2=1 selects it, the default is off.
-static int g_cl2_mode = -1;  // -1: read FPCC_CL2 from the environment on first use
-static bool cl2_enabled() {
-    if (g_cl2_mode < 0) {
-        const char *e = getenv("FPCC_CL2");
-        g_cl2_mode = (e && e[0] == '1') ? 1 : 0;
-    }
-    return g_cl2_mode == 1;
+    if (KIND != 0) return launch_outk<MODE, STAGES, KIND, OK_I8>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, smem, s);
+    if (ep.post_mul && !ep.aux_out) return launch_outk<MODE, STAGES, KIND, OK_POST2>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, smem, s);
+    if (ep.out_type == FPCC_OUT_I8) return launch_outk<MODE, STAGES, KIND, OK_I8>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, smem, s);
+    if (ep.out_type == FPCC_OUT_I32) return launch_outk<MODE, STAGES, KIND, OK_I32>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, smem, s);
+    return launch_outk<MODE, STAGES, KIND, OK_I16>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, smem, s);
 }
 
 template <int MODE, int KIND>
@@ -1782,22 +1536,14 @@ static int launch_tc(TcArgs &a, const void *W, int64_t w_rows, int tiles_m, cons
     const int rows_k = MODE == 0 ? a.kvol : 2;
     int total = tiles_m * n_blocks_n;
     int sms = g_sm_budget > 0 && g_sm_budget < sm_count() ? g_sm_budget : sm_count();
-    // int8 sparse conv with one channel block and enough tiles: 2-CTA clusters, each CTA loads half of a weight tile
-    const bool cl2 = MODE == 0 && KIND == 0 && n_blocks_n == 1 && (a.n_tile % 16) == 0 && total >= 4 && sms >= 2 && cl2_enabled();
     CUtensorMap tmap;
-    int rc = weight_tensor_map((const int8_t *)W, w_rows, a.K, cl2 ? a.n_tile / 2 : a.n_tile, &tmap);
+    int rc = weight_tensor_map((const int8_t *)W, w_rows, a.K, a.n_tile, &tmap);
     if (rc) return rc;
     int grid = total < sms ? total : sms;
-    if (cl2) {
-        const int pairs = (total + 1) / 2, clusters = sms / 2;
-        grid = 2 * (pairs < clusters ? pairs : clusters);
-    }
-    // FPCC_STAGES=3 (environment, experiments): three operand stages leave ~48 KB of shared memory per SM, enough for the
-    // serial range-coder blocks of other streams to share an SM with a persistent GEMM CTA
-    static const bool force3 = [] { const char *e = getenv("FPCC_STAGES"); return e && e[0] == '3'; }();
-    if (!force3 && PSmem<4>::bytes(a.n_tile, rows_k) <= TC_SMEM_MAX)
-        return launch_stages<MODE, 4, KIND>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, rows_k, cl2, s);
-    return launch_stages<MODE, 3, KIND>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, rows_k, cl2, s);
+    // four operand stages where they fit in shared memory, three otherwise (wide tiles with many kernel offsets)
+    if (PSmem<4>::bytes(a.n_tile, rows_k) <= TC_SMEM_MAX)
+        return launch_stages<MODE, 4, KIND>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, rows_k, s);
+    return launch_stages<MODE, 3, KIND>(a, tmap, ep, fe, out, tiles_m, n_blocks_n, grid, rows_k, s);
 }
 
 int launch_conv_tc(const int8_t *feats, int n_in, int c_in, const int8_t *weight, int kvol, int c_out, const int32_t *nbr,

@@ -1,7 +1,6 @@
 #!/bin/bash
-# SM budget / operand stage sweep of the bench step (pipelined schedule, 3 groups). usage: bash tools/sweep_budget.sh
-for cfg in "0 4" "100 4" "116 4" "132 4" "148 4" "116 3" "132 3" "148 3"; do
-  set -- $cfg
-  line=$(FPCC_SM_BUDGET=$1 FPCC_STAGES=$2 python bench.py --steps 3 --warmup 2 --no-cpu-baseline --groups 3 2>&1 >/dev/null | grep "step_device\|Error\|error" | tr '\n' ' ')
-  echo "budget=$1 stages=$2: $line"
+# SM budget sweep of the bench step (pipelined schedule, 3 groups). usage: bash tools/sweep_budget.sh
+for budget in 0 100 116 132 148; do
+  line=$(FPCC_SM_BUDGET=$budget python bench.py --steps 3 --warmup 2 --no-cpu-baseline --groups 3 2>&1 >/dev/null | grep "step_device\|Error\|error" | tr '\n' ' ')
+  echo "budget=$budget: $line"
 done
