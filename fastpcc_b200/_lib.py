@@ -66,6 +66,9 @@ SIGNATURES = {
     'fpcc_linear_i8': (_i, [_vp, _i, _i, _vp, _i, _vp, _vp, _vp, _i, _i, _EP, _vp, _vp]),
     'fpcc_spconv_f16': (_i, [_vp, _i, _i, _i, _vp, _i, _i, _vp, _i64, _i, _vp, _vp, _i, C.c_float, _vp, _i, C.c_float, _vp, _i, _vp]),
     'fpcc_spconv_wgrad_f16': (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _i, _vp, _i, _i, _vp]),
+    'fpcc_kmap_transpose': (_i, [_vp, _i, _i, _i64, _i, _vp, _i64, _vp]),
+    'fpcc_act_grad_workspace': (_sz, [_i64, _i]),
+    'fpcc_act_grad_f16': (_i, [_vp, _i, _i64, _vp, _i, _i64, _i64, _i, _i, C.c_float, _vp, _i, _i, _vp, _vp, _sz, _vp]),
     'fpcc_linear_f16': (_i, [_vp, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _i, _i, _vp, _i, C.c_float, _vp, _i, C.c_float, _vp, _i, _vp]),
     'fpcc_set_tc_mode': (_i, [_i]),
     'fpcc_set_sm_budget': (_i, [_i]),

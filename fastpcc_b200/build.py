@@ -8,7 +8,7 @@ HERE = osp.dirname(osp.abspath(__file__))
 CSRC = osp.join(HERE, 'csrc')
 OUT_DIR = osp.join(HERE, '_C')
 SO = osp.join(OUT_DIR, 'libfastpcc_b200.so')
-SOURCES = ['common.cu', 'coords.cu', 'igemm_simt.cu', 'igemm_tc.cu', 'ops_api.cu', 'entropy.cu', 'rans.cu', 'frontend.cu', 'container.cu', 'metrics.cu']
+SOURCES = ['common.cu', 'coords.cu', 'igemm_simt.cu', 'igemm_tc.cu', 'ops_api.cu', 'entropy.cu', 'rans.cu', 'frontend.cu', 'container.cu', 'metrics.cu', 'train.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr']
 

@@ -12,7 +12,14 @@ Differences that matter to a caller:
     the state dict, features travel in the compute dtype (`set_compute_dtype`);
   * coordinate sets are kept in Morton order (x least significant, ME's convention relied on at
     lossy_coord_v2/model.py:122-124), so generated / strided coordinates have a defined, reproducible row order;
-  * a following activation can ride in the conv epilogue (`fused_act`), which is how ConvBlock uses it.
+  * a following activation can ride in the conv epilogue (`fused_act`), which is how ConvBlock uses it;
+  * training: when grad is enabled and a parameter or the input features require it, every conv / linear layer runs
+    through `autograd.MELayerFunction` -- the same forward kernels in the same order (the output bits do not depend on
+    the grad mode), dgrad / wgrad on the tcgen05 kernels, the fused ReLU / LeakyReLU (slope >= 0) backward in one pass
+    (`fpcc_act_grad_f16`).  On that path a PReLU or a negative LeakyReLU slope is applied after the layer as a torch op,
+    so a PReLU slope trains.  Feature gradients travel in the compute dtype, parameter gradients are fp32.  Pruning,
+    cat, +, batch norm and max (un)pooling are torch ops and differentiate as such: max pooling shares the gradient
+    among tied maxima (torch's `scatter_reduce` amax rule), where ME routes it to one argmax.
 """
 from enum import Enum
 from typing import Dict, Optional, Tuple, Union
@@ -334,6 +341,11 @@ def cat(*tensors):
 _ACT = {'none': (ops.ACT_NONE, 0.0), 'relu': (ops.ACT_RELU, 0.0)}
 
 
+def _fusable_act(act) -> bool:
+    """an activation module (or None) that the conv / linear epilogue can apply"""
+    return act is None or isinstance(act, (MinkowskiReLU, MinkowskiLeakyReLU)) or (isinstance(act, MinkowskiPReLU) and act.weight.numel() == 1)
+
+
 def _act_code(act) -> Tuple[int, float]:
     """(code, slope) of a fusable activation module / None"""
     if act is None:
@@ -345,6 +357,28 @@ def _act_code(act) -> Tuple[int, float]:
     if isinstance(act, MinkowskiPReLU) and act.weight.numel() == 1:
         return ops.ACT_LEAKY, float(act.weight.item())
     return -1, 0.0
+
+
+def _needs_grad(f: torch.Tensor, *params) -> bool:
+    return torch.is_grad_enabled() and (f.requires_grad or any(p is not None and p.requires_grad for p in params))
+
+
+def _epilogue_act(act, grad: bool):
+    """-> (code, slope, module applied after the layer | None).  Inference fuses every fusable activation.  With grad the
+    epilogue keeps only activations whose derivative follows from the output (ReLU, LeakyReLU with slope >= 0); a PReLU
+    (its slope may train; no host read of it) and a negative LeakyReLU slope run after the layer as torch ops."""
+    if grad and (isinstance(act, MinkowskiPReLU) or (isinstance(act, MinkowskiLeakyReLU) and act.negative_slope < 0)):
+        return ops.ACT_NONE, 0.0, act
+    code, slope = _act_code(act)
+    return code, slope, None
+
+
+def _differentiable(x, kernel, bias, c_in, c_out, code, slope, run, after, out_key, kind, **spec):
+    """the output SparseTensor of a conv / linear layer on the training path: `run()` is the layer's inference call"""
+    from . import autograd  # imported here: oracle/me_cpu.py executes this file's source outside the package
+    sp = autograd.MESpec(kind, c_in, c_out, code, slope, _COMPUTE, **spec)
+    out = SparseTensor(autograd.me_layer(x.F, kernel, bias, sp, run), coordinate_map_key=out_key, coordinate_manager=x.coordinate_manager)
+    return after(out) if after is not None else out
 
 
 def _as_compute(f: torch.Tensor) -> torch.Tensor:
@@ -410,7 +444,8 @@ class _ConvBase(nn.Module):
 class MinkowskiConvolution(_ConvBase):
     def forward(self, x: SparseTensor, coordinates: Optional[CoordinateMapKey] = None, fused_act=None) -> SparseTensor:
         cm, kg = x.coordinate_manager, self.kernel_generator
-        code, slope = _act_code(fused_act)
+        grad = _needs_grad(x.F, self.kernel, self.bias)
+        code, slope, after = _epilogue_act(fused_act, grad)
         assert code >= 0, 'activation cannot be fused'
         if kg.kernel_stride == (1, 1, 1):
             out_key = x.coordinate_map_key if coordinates is None else coordinates
@@ -423,6 +458,12 @@ class MinkowskiConvolution(_ConvBase):
                 table, perm = cm.grouped_kernel_table(*args)
             else:
                 table = cm.kernel_table(*args)
+        if grad:
+            kv = kg.kernel_volume
+            return _differentiable(x, self.kernel, self.bias, self.in_channels, self.out_channels, code, slope,
+                                   lambda: self._run(x.F, table, code, slope, row_perm=perm), after, out_key,
+                                   'conv' if kv > 1 else 'linear', layout='kio' if kv > 1 else 'io',
+                                   table=cm.kernel_table(*args) if kv > 1 else None, group=x.F.shape[0] >= GROUP_ROWS_MIN)
         f = self._run(x.F, table, code, slope, row_perm=perm)
         return SparseTensor(f, coordinate_map_key=out_key, coordinate_manager=cm)
 
@@ -434,7 +475,8 @@ class MinkowskiConvolutionTranspose(_ConvBase):
     def forward(self, x: SparseTensor, coordinates: CoordinateMapKey, fused_act=None) -> SparseTensor:
         cm, kg = x.coordinate_manager, self.kernel_generator
         assert kg.kernel_size == (2, 2, 2) and kg.kernel_stride == (2, 2, 2), 'only k=2, s=2 transposed convs are used'
-        code, slope = _act_code(fused_act)
+        grad = _needs_grad(x.F, self.kernel, self.bias)
+        code, slope, after = _epilogue_act(fused_act, grad)
         ts = x.coordinate_map_key.tensor_stride[0]
         half = ts // 2
         oc = cm.get_coordinates(coordinates)
@@ -448,16 +490,26 @@ class MinkowskiConvolutionTranspose(_ConvBase):
             slot = (d[:, 0] + 2 * d[:, 1] + 4 * d[:, 2]).to(torch.uint8)  # x fastest
             slot = torch.where(par >= 0, slot, torch.full_like(slot, 255))  # orphans join no group -> bias only
             cm._kmaps[tag] = ops.slot_pairs(par.clamp(min=0).contiguous(), slot.contiguous())
+            cm._kmaps[('tconv_slots',) + tag[1:]] = (par.clamp(min=0).contiguous(), slot.contiguous())
         sel = cm._kmaps[tag]
-        w, b, cin_p, cout_p = self._weights()
-        f = _pad_cols(_as_compute(x.F), cin_p).contiguous()
-        # rows without a parent belong to no group: they keep act(bias)
-        fill = torch.zeros(cout_p, dtype=torch.float32, device=f.device) if b is None else b
-        fill = torch.relu(fill) if code == ops.ACT_RELU else (torch.where(fill < 0, fill * slope, fill) if code == ops.ACT_LEAKY else fill)
-        out = fill.to(_COMPUTE)[None].repeat(oc.shape[0], 1)
-        res = ops.linear_f16(f, w.reshape(8 * cout_p, cin_p), bias=b, act=code, slope=slope, sel=sel, n_out_rows=oc.shape[0], out=out)
-        res = res[:, :self.out_channels] if cout_p != self.out_channels else res
-        return SparseTensor(res, coordinate_map_key=coordinates, coordinate_manager=cm)
+
+        def run():
+            w, b, cin_p, cout_p = self._weights()
+            f = _pad_cols(_as_compute(x.F), cin_p).contiguous()
+            # rows without a parent belong to no group: they keep act(bias)
+            fill = torch.zeros(cout_p, dtype=torch.float32, device=f.device) if b is None else b
+            fill = torch.relu(fill) if code == ops.ACT_RELU else (torch.where(fill < 0, fill * slope, fill) if code == ops.ACT_LEAKY else fill)
+            out = fill.to(_COMPUTE)[None].repeat(oc.shape[0], 1)
+            res = ops.linear_f16(f, w.reshape(8 * cout_p, cin_p), bias=b, act=code, slope=slope, sel=sel, n_out_rows=oc.shape[0], out=out)
+            return res[:, :self.out_channels] if cout_p != self.out_channels else res
+
+        if grad:
+            ttag = ('tconv_table',) + tag[1:]
+            if ttag not in cm._kmaps:  # k-major [8, n_child]: parent row + 1 in the child's slot row (the conv form of sel)
+                cm._kmaps[ttag] = ops.slot_table(*cm._kmaps[('tconv_slots',) + tag[1:]])
+            return _differentiable(x, self.kernel, self.bias, self.in_channels, self.out_channels, code, slope, run, after,
+                                   coordinates, 'tconv', table=cm._kmaps[ttag], group=x.F.shape[0] >= GROUP_ROWS_MIN)
+        return SparseTensor(run(), coordinate_map_key=coordinates, coordinate_manager=cm)
 
 
 class MinkowskiGenerativeConvolutionTranspose(_ConvBase):
@@ -467,7 +519,8 @@ class MinkowskiGenerativeConvolutionTranspose(_ConvBase):
     def forward(self, x: SparseTensor, coordinates=None, fused_act=None) -> SparseTensor:
         cm, kg = x.coordinate_manager, self.kernel_generator
         assert kg.kernel_size == (2, 2, 2) and kg.kernel_stride == (2, 2, 2), 'only k=2, s=2 generative convs are used'
-        code, slope = _act_code(fused_act)
+        grad = _needs_grad(x.F, self.kernel, self.bias)
+        code, slope, after = _epilogue_act(fused_act, grad)
         ts = x.coordinate_map_key.tensor_stride[0]
         half = ts // 2
         tag = ('gen', x.coordinate_map_key)
@@ -476,13 +529,19 @@ class MinkowskiGenerativeConvolutionTranspose(_ConvBase):
             offs = torch.tensor([[0, k & 1, (k >> 1) & 1, (k >> 2) & 1] for k in range(8)], dtype=torch.int32, device=c.device) * half
             cm._kmaps[tag] = cm._new_key((half,) * 3, (c[:, None] + offs[None]).reshape(-1, 4))
         out_key = cm._kmaps[tag]
-        w, b, cin_p, cout_p = self._weights()
-        f = _pad_cols(_as_compute(x.F), cin_p).contiguous()
-        b8 = None if b is None else b.repeat(8)
-        res = ops.linear_f16(f, w.reshape(8 * cout_p, cin_p), bias=b8, act=code, slope=slope)
-        res = res.reshape(-1, cout_p)
-        res = res[:, :self.out_channels] if cout_p != self.out_channels else res
-        return SparseTensor(res, coordinate_map_key=out_key, coordinate_manager=cm)
+
+        def run():
+            w, b, cin_p, cout_p = self._weights()
+            f = _pad_cols(_as_compute(x.F), cin_p).contiguous()
+            b8 = None if b is None else b.repeat(8)
+            res = ops.linear_f16(f, w.reshape(8 * cout_p, cin_p), bias=b8, act=code, slope=slope)
+            res = res.reshape(-1, cout_p)
+            return res[:, :self.out_channels] if cout_p != self.out_channels else res
+
+        if grad:
+            return _differentiable(x, self.kernel, self.bias, self.in_channels, self.out_channels, code, slope, run, after,
+                                   out_key, 'gen')
+        return SparseTensor(run(), coordinate_map_key=out_key, coordinate_manager=cm)
 
 
 class MinkowskiLinear(nn.Module):
@@ -492,8 +551,9 @@ class MinkowskiLinear(nn.Module):
         self._cache = None
 
     def forward(self, x: SparseTensor, fused_act=None) -> SparseTensor:
-        code, slope = _act_code(fused_act)
         lin = self.linear
+        grad = _needs_grad(x.F, lin.weight, lin.bias)
+        code, slope, after = _epilogue_act(fused_act, grad)
         key = (lin.weight._version, lin.weight.data_ptr(), _COMPUTE, None if lin.bias is None else lin.bias._version)
         if self._cache is None or self._cache[0] != key:
             cin_p, cout_p = max(16, (lin.in_features + 7) // 8 * 8), max(16, lin.out_features)
@@ -506,10 +566,17 @@ class MinkowskiLinear(nn.Module):
             _publish(w)
             self._cache = (key, w, b, cin_p, cout_p)
         _, w, b, cin_p, cout_p = self._cache
-        f = _pad_cols(_as_compute(x.F), cin_p).contiguous()
-        od = torch.float32 if lin.out_features == 1 else None  # single-channel heads keep fp32 (see _ConvBase._run)
-        out = ops.linear_f16(f, w, bias=b, act=code, slope=slope, out_dtype=od)
-        return x._like(out[:, :lin.out_features] if cout_p != lin.out_features else out)
+
+        def run():
+            f = _pad_cols(_as_compute(x.F), cin_p).contiguous()
+            od = torch.float32 if lin.out_features == 1 else None  # single-channel heads keep fp32 (see _ConvBase._run)
+            out = ops.linear_f16(f, w, bias=b, act=code, slope=slope, out_dtype=od)
+            return out[:, :lin.out_features] if cout_p != lin.out_features else out
+
+        if grad:
+            return _differentiable(x, lin.weight, lin.bias, lin.in_features, lin.out_features, code, slope, run, after,
+                                   x.coordinate_map_key, 'linear', layout='oi')
+        return x._like(run())
 
 
 class _Pointwise(nn.Module):

@@ -30,7 +30,7 @@ def get_act_module(act: Union[str, nn.Module, None]) -> Optional[nn.Module]:
 
 
 def _fusable(act_module) -> bool:
-    return act_module is None or ME._act_code(act_module)[0] >= 0
+    return ME._fusable_act(act_module)
 
 
 class MEMLPBlock(nn.Module):

@@ -274,12 +274,28 @@ def occ_to_bits(occ):
     return out
 
 
-def slot_pairs(child_parent, child_slot):
-    """Pair lists grouped by child slot for the selection linear: (sel_row, sel_out, offsets[9])."""
+def slot_table(child_parent, child_slot):
+    """k-major child-slot table [8, n_child]: parent row + 1 in the row of the child's slot, 0 elsewhere."""
     n = child_parent.shape[0]
     table = torch.empty((8, n), dtype=torch.int32, device=child_parent.device)
     _call('fpcc_slot_table', _p(child_parent), _p(child_slot), n, _p(table), n, _s())
-    return kmap_compact(table)
+    return table
+
+
+def slot_pairs(child_parent, child_slot):
+    """Pair lists grouped by child slot for the selection linear: (sel_row, sel_out, offsets[9])."""
+    return kmap_compact(slot_table(child_parent, child_slot))
+
+
+def kmap_transpose(table, n_in):
+    """Transposed k-major neighbour table [kvol, n_in]: tt[k, j] = m + 1 where table[k, m] == j + 1, 0 elsewhere (the
+    map of the dgrad).  Every (offset, input row) pair must have at most one output row (fpcc_kmap_transpose)."""
+    _need(table, torch.int32, 'table', 2)
+    kv, n_out = table.shape
+    tt = torch.empty((kv, n_in), dtype=torch.int32, device=table.device)
+    _call('fpcc_kmap_transpose', _p(table), kv, n_out, n_out, int(n_in), _p(tt), int(n_in), _s(),
+          work={'bytes': 4.0 * kv * n_out + 4.0 * kv * n_in + 4.0 * int(torch.count_nonzero(table).item()) if _prof is not None else 0.0})
+    return tt
 
 
 def gather_patches(feats, table, kp):
@@ -674,6 +690,33 @@ def spconv_wgrad_f16(x, dy, in_map, out_map, offsets_host, c_in, c_out):
         _call('fpcc_spconv_wgrad_f16', _p(xp), _p(gp), _F_DT[x.dtype], c_in_p, c_out_p, _p(in_map), _p(out_map), _p(tl), tl.shape[0],
               _p(dw), c_in, c_out, _s(), tag='spconv_wgrad_tc', work={'ops': 2.0 * n_pairs * c_in * c_out})
     return dw
+
+
+def act_grad_f16(dy, y, act, slope, c_pad, out_dtype=None, want_bias=True):
+    """Backward of an activation fused into the conv / linear epilogue (fpcc_act_grad_f16), one pass:
+    -> (dz [n, c_pad] in out_dtype (default: y's dtype, fp16 / bf16) with zero pad columns, dbias fp32 [c] | None).
+    dy, y: [n, c] fp16 / bf16 / fp32 with unit column stride (y = the forward output; unused for ACT_NONE)."""
+    n, c = dy.shape
+    out_dtype = (y.dtype if y is not None and y.dtype != torch.float32 else torch.float16) if out_dtype is None else out_dtype
+    if out_dtype not in _F_DT:
+        raise RuntimeError(f'act_grad_f16: dz must be fp16 or bf16, got {out_dtype}')
+    for t, name in ((dy, 'dy'), (y, 'y')):
+        if t is None:
+            continue
+        if t.dtype not in _F_OUT or not t.is_cuda or t.dim() != 2 or tuple(t.shape) != (n, c):
+            raise RuntimeError(f'act_grad_f16: {name} must be a 2-D fp16 / bf16 / fp32 CUDA tensor of shape {(n, c)}')
+    rows = lambda t: t if t.stride(1) == 1 and t.stride(0) >= c else t.contiguous()  # noqa: E731  (any row pitch >= c)
+    dy = rows(dy)
+    y = rows(y) if y is not None else None
+    dz = torch.empty((n, c_pad), dtype=out_dtype, device=dy.device)
+    db = torch.empty(c, dtype=torch.float32, device=dy.device) if want_bias else None
+    ws = workspace(_lib.load().fpcc_act_grad_workspace(n, c), dy.device) if want_bias else None
+    ld_y = y.stride(0) if y is not None else c
+    nbytes = float(n) * c * (dy.element_size() + (y.element_size() if (y is not None and act != ACT_NONE) else 0)) + float(n) * c_pad * dz.element_size()
+    _call('fpcc_act_grad_f16', _p(dy), _F_OUT[dy.dtype], dy.stride(0), _p(y), _F_OUT[y.dtype] if y is not None else 0,
+          ld_y, n, c, int(act), float(slope), _p(dz), _F_DT[out_dtype], int(c_pad), _p(db), _p(ws), 0 if ws is None else ws.numel(), _s(),
+          work={'bytes': nbytes})
+    return dz, db
 
 
 def linear_f16(a, weight, bias=None, act=ACT_NONE, slope=0.0, residual=None, post_act=ACT_NONE, post_slope=0.0,

@@ -365,6 +365,27 @@ int fpcc_spconv_f16(const void *feats, int dtype, int n_in, int c_in, const void
 int fpcc_spconv_wgrad_f16(const void *x, const void *dy, int dtype, int c_in_p, int c_out_p, const int32_t *in_idx,
                           const int32_t *out_idx, const int32_t *tiles, int n_tiles, float *dw, int c_in, int c_out,
                           void *stream);
+/* Transposed neighbour table for the dgrad of fpcc_spconv_f16 (MinkowskiEngine's backward runs the same gather-GEMM-
+ * scatter on the transposed kernel map; the training step of lossy_coord_v2 / lossy_coord_lossy_color, train.py:359-404,
+ * reaches it through loss.backward()).  table: k-major [kvol, ld] with table[k, m] = input row + 1 of output row m (0 =
+ * none), n_out columns used.  tt: k-major [kvol, ld_t], n_in columns written: tt[k, j] = m + 1 where table[k, m] == j + 1,
+ * 0 elsewhere.  Precondition: every (k, input row) pair has at most one output row -- true for stride-1 and strided
+ * HYPER_CUBE maps, maps onto an explicit target key, and the child-slot table of fpcc_slot_table -- so the result is
+ * deterministic without atomics.  Entries outside 1..n_in are ignored. */
+int fpcc_kmap_transpose(const int32_t *table, int kvol, int n_out, int64_t ld, int n_in, int32_t *tt, int64_t ld_t,
+                        void *stream);
+/* Backward of an activation fused into the fpcc_spconv_f16 / fpcc_linear_f16 epilogue, one pass over [n, c]:
+ *   dz[r, j] = dy[r, j] * act'(y[r, j])  rounded once to dz_type (0 fp16, 1 bf16), rows of c_pad columns with zeros
+ *              in c <= j < c_pad (the operand width of the dgrad / wgrad kernels);
+ *   dbias[j] = sum_r of the unrounded products (fp32 result; NULL = not wanted).
+ * dy / y: element types 0 fp16, 1 bf16, 2 fp32, row pitches ld_dy / ld_y; y is the forward OUTPUT.  act: 0 none (y may be
+ * NULL), 1 ReLU, 2 LeakyReLU with slope >= 0 -- for these act'(y) is read from y alone (y > 0 ? 1 : slope).  dbias is
+ * reduced from fp64 per-CTA partials in a fixed order (no float atomics), so it is reproducible bit for bit.
+ * workspace: fpcc_act_grad_workspace(n, c) bytes when dbias is wanted. */
+size_t fpcc_act_grad_workspace(int64_t n, int c);
+int fpcc_act_grad_f16(const void *dy, int dy_type, int64_t ld_dy, const void *y, int y_type, int64_t ld_y, int64_t n, int c,
+                      int act, float slope, void *dz, int dz_type, int c_pad, float *dbias, void *workspace,
+                      size_t workspace_bytes, void *stream);
 int fpcc_linear_f16(const void *A, int dtype, int m, int k, const void *W, int n, const int32_t *sel_row,
                     const int32_t *sel_out, const int32_t *sel_offsets, int n_groups, int n_sel, const float *bias,
                     int act, float slope, const void *residual, int post_act, float post_slope, void *out,
