@@ -88,6 +88,10 @@ SIGNATURES = {
     'fpcc_indexed_ranges': (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     'fpcc_indexed_decode': (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _i64, _i, _vp, _vp, _vp]),
     'fpcc_pmf_to_quantized_cdf': (_i, [_vp, _i, _i, _vp, _i, _vp, _vp, _vp]),
+    'fpcc_factorized_bits': (_i, [_vp, _i64, _i64, _i, _vp, C.c_float, _vp, _vp]),
+    'fpcc_factorized_grad_workspace': (_sz, [_i64, _i]),
+    'fpcc_factorized_grad': (_i, [_vp, _i64, _vp, _i64, _i64, _i, _vp, C.c_float, _vp, _vp, _vp, _sz, _vp]),
+    'fpcc_factorized_pmf': (_i, [_vp, _i, _i, _i, _vp, _vp]),
 }
 
 _LIB = None

@@ -4,7 +4,7 @@ Colour: the all-ties nearest-neighbour search fpcc_nn_tie_attr and the recolouri
 Lossy geometry decodes to points that are not in the original cloud; `recolor` gives each of them a colour taken
 from the original, the step before colours can be coded or scored (and how the training targets of
 models/convolutional/lossy_coord_lossy_color are built, layers.py:269-333).  `metrics.pc_error` uses the same search
-for its colour figures.
+for its colour figures, and `rgb_to_yuv` for its colour space (as does the colour loss of `train.LossyColorNet`).
 
 The rule of `recolor` is this project's own definition, a forward / backward transfer in the spirit of MPEG's
 recolouring; the reference's layers.py:269-333 was not available when this module was written, and parity with it
@@ -44,6 +44,14 @@ def _rows(query: torch.Tensor, ref: torch.Tensor, n_batch: Optional[int]):
         tops = [int(t[:, 0].max().item()) for t in (query, ref) if t.shape[0]]
         n_batch = max([0] + tops) + 1
     return query.contiguous(), ref.contiguous(), n_batch, 1, 0
+
+
+def rgb_to_yuv(rgb: torch.Tensor) -> torch.Tensor:
+    """[n, 3] RGB in 0..255 (any dtype) -> BT.709 YUV normalised to [0, 1], double (pc_error's colour space)"""
+    r, g, b = rgb.double().unbind(1)
+    return torch.stack([(0.2126 * r + 0.7152 * g + 0.0722 * b) / 255,
+                        (-0.1146 * r - 0.3854 * g + 0.5 * b) / 255 + 0.5,
+                        (0.5 * r - 0.4542 * g - 0.0458 * b) / 255 + 0.5], 1)
 
 
 def nearest_tie_attr(query: torch.Tensor, ref: torch.Tensor, ref_rgb: torch.Tensor, n_batch: Optional[int] = None):

@@ -13,6 +13,9 @@ kernels, shared by the torchsparse-shaped layers (`torchsparse_nn.py`) and the M
                                                                     rows), split-K tiles meeting in fp32 atomics; a
                                                                     per-offset library GEMM only above 256 channels
 
+The deep-factorized entropy model (`FactorizedBitsFunction`) is one fused kernel each way: bits of the latents forward,
+dy and the packed parameter gradient backward (`fpcc_factorized_bits` / `fpcc_factorized_grad`).
+
 MinkowskiEngine computes the same three products per kernel offset (ME backward = transposed gather-GEMM-scatter).
 The ME layer kinds map onto these products as follows (`MELayerFunction`):
 
@@ -219,3 +222,26 @@ class MELayerFunction(torch.autograd.Function):
 def me_layer(feats, kernel, bias, spec, run):
     """differentiable ME-shim layer: `run()` computes the forward output from `feats` with the layer's inference kernels"""
     return MELayerFunction.apply(feats, kernel, bias, spec, run)
+
+
+class FactorizedBitsFunction(torch.autograd.Function):
+    """bits = -log2(max(L(y), bound)) of the deep-factorized prior (fpcc_factorized_bits): y fp32 [n, C], params fp32
+    [C, 43] (the packed rows of `entropy_models.NoisyDeepFactorizedEntropyModel`).  The backward recomputes the
+    forward in the kernel and returns the gradient of the raw params, reduced in a fixed order."""
+
+    @staticmethod
+    def forward(ctx, y, params, bound):
+        ctx.save_for_backward(y, params)
+        ctx.bound = bound
+        return ops.factorized_bits(y, params, bound)
+
+    @staticmethod
+    def backward(ctx, dbits):
+        y, params = ctx.saved_tensors
+        dy, dp = ops.factorized_grad(y, params, dbits.float(), ctx.bound)
+        return (dy if ctx.needs_input_grad[0] else None), (dp if ctx.needs_input_grad[1] else None), None
+
+
+def factorized_bits(y, params, bound=1e-9):
+    """differentiable bits of the deep-factorized prior; y is cast to fp32 (latents arrive in the compute dtype)"""
+    return FactorizedBitsFunction.apply(y.float(), params, float(bound))

@@ -56,12 +56,7 @@ def _psnr(mse: float, peak: float) -> float:
     return float('inf') if mse == 0 else 10.0 * math.log10(3.0 * peak * peak / mse)
 
 
-def _yuv(rgb: torch.Tensor) -> torch.Tensor:
-    """[n, 3] RGB in 0..255 (double) -> BT.709 YUV normalised to [0, 1]"""
-    r, g, b = rgb.double().unbind(1)
-    return torch.stack([(0.2126 * r + 0.7152 * g + 0.0722 * b) / 255,
-                        (-0.1146 * r - 0.3854 * g + 0.5 * b) / 255 + 0.5,
-                        (0.5 * r - 0.4542 * g - 0.0458 * b) / 255 + 0.5], 1)
+_yuv = attributes.rgb_to_yuv
 
 
 def _color_mse(a: torch.Tensor, a_rgb: torch.Tensor, b: torch.Tensor, b_rgb: torch.Tensor):

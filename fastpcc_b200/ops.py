@@ -744,3 +744,53 @@ def linear_f16(a, weight, bias=None, act=ACT_NONE, slope=0.0, residual=None, pos
               n_out_rows, pb, act, float(slope), pr, post_act, float(post_slope), _p(out), _F_OUT[out_dtype], _s(),
               tag='linear_sel_f16_tc', work={'ops': 2.0 * n_out_rows * k * n})
     return out
+
+
+# ---------------------------------------------------------------------------------------------
+# deep-factorized entropy model (csrc/entropy_model.cu)
+# ---------------------------------------------------------------------------------------------
+def _em_rows(t, c, name):
+    if t.dtype != torch.float32 or not t.is_cuda or t.dim() != 2 or t.shape[1] != c:
+        raise RuntimeError(f'factorized entropy model: {name} must be a 2-D fp32 CUDA tensor with {c} columns')
+    return t if t.stride(1) == 1 and t.stride(0) >= c else t.contiguous()  # any row pitch >= c
+
+
+def _em_params(params):
+    if params.dtype != torch.float32 or not params.is_cuda or params.dim() != 2 or params.shape[1] != 43:
+        raise RuntimeError('factorized entropy model: params must be an fp32 CUDA tensor [C, 43]')
+    return params.contiguous()
+
+
+def factorized_bits(y, params, bound=1e-9):
+    """-log2(max(L_c(y), bound)) per element: y fp32 [n, C], params fp32 [C, 43] -> bits fp32 [n, C]"""
+    params = _em_params(params)
+    n, c = y.shape[0], params.shape[0]
+    y = _em_rows(y, c, 'y')
+    bits = torch.empty((n, c), dtype=torch.float32, device=y.device)
+    _call('fpcc_factorized_bits', _p(y), y.stride(0), n, c, _p(params), float(bound), _p(bits), _s(),
+          work={'bytes': 8.0 * n * c + 172.0 * c})
+    return bits
+
+
+def factorized_grad(y, params, dbits, bound=1e-9):
+    """-> (dy fp32 [n, C], dparams fp32 [C, 43]) of sum(dbits * factorized_bits(y, params)); dparams with respect to the
+    raw params, reproducible bit for bit"""
+    params = _em_params(params)
+    n, c = y.shape[0], params.shape[0]
+    y, dbits = _em_rows(y, c, 'y'), _em_rows(dbits, c, 'dbits')
+    if dbits.shape[0] != n:
+        raise RuntimeError('factorized entropy model: dbits must have the rows of y')
+    dy = torch.empty((n, c), dtype=torch.float32, device=y.device)
+    dp = torch.empty((c, 43), dtype=torch.float32, device=y.device)
+    ws = workspace(_lib.load().fpcc_factorized_grad_workspace(n, c), y.device)
+    _call('fpcc_factorized_grad', _p(y), y.stride(0), _p(dbits), dbits.stride(0), n, c, _p(params), float(bound), _p(dy), _p(dp),
+          _p(ws), ws.numel(), _s(), work={'bytes': 12.0 * n * c + 344.0 * c})
+    return dy, dp
+
+
+def factorized_pmf(params, lo=-64, n_sym=129):
+    """pmf fp64 [C, n_sym]: pmf[c, k] = L_c(lo + k), by the device function of factorized_bits"""
+    params = _em_params(params)
+    pmf = torch.empty((params.shape[0], n_sym), dtype=torch.float64, device=params.device)
+    _call('fpcc_factorized_pmf', _p(params), params.shape[0], int(lo), int(n_sym), _p(pmf), _s())
+    return pmf

@@ -120,6 +120,44 @@ def batched_pmf_to_quantized_cdf(pmf_array: np.ndarray, offset_array: np.ndarray
     return [cdf_h[t, :lens_h[t]].tolist() for t in range(T)]
 
 
+def _table_args(tables, overflow):
+    flat, off, lens, offsets = tables
+    return _p(flat), _p(off), _p(lens), lens.numel(), _p(offsets), int(bool(overflow))
+
+
+def indexed_encode(tables, overflow, sym, idx, n, n_streams):
+    """IndexedRansCoder's encoder on device tensors: tables = (cdf_flat int32, cdf_off int64, cdf_len int32, offsets
+    int32), sym int32 [n_streams * n] (idx: int32 table ids, or None for table = position mod n_tables)
+    -> one bytes object per stream"""
+    cnt = torch.empty(n_streams * n, dtype=torch.int32, device=sym.device)
+    _lib.call('fpcc_indexed_count', *_table_args(tables, overflow), _p(sym), _p(idx), n, n_streams, _p(cnt), _s())
+    incl = torch.cumsum(cnt.to(torch.int64), 0)
+    pos = (incl - cnt).contiguous()
+    total = int(incl[-1].item())
+    ranges = torch.empty(total, dtype=torch.int32, device=sym.device)
+    bits = torch.empty(total, dtype=torch.uint8, device=sym.device)
+    _lib.call('fpcc_indexed_ranges', *_table_args(tables, overflow), _p(sym), _p(idx), n, n_streams, _p(pos), _p(ranges), _p(bits), _s())
+    rng_off = torch.cat([pos[::n], incl[-1:]]).contiguous()
+    per = (rng_off[1:] - rng_off[:-1])
+    cap = int(per.max().item()) * 2 + 64
+    out, out_len = ops.rans_encode(ranges, rng_off, cap, bits=bits)
+    out, out_len = out.cpu().numpy(), out_len.cpu().numpy()
+    assert (out_len > 0).all()
+    return [out[b, cap - out_len[b]:].tobytes() for b in range(n_streams)]
+
+
+def indexed_decode(tables, overflow, blob, byte_off, byte_len, idx, n, n_streams):
+    """IndexedRansCoder's decoder on device tensors (streams at blob[byte_off[b]:][:byte_len[b]]) -> int32 [n_streams, n]
+    on the device; raises when a stream ends early"""
+    out = torch.empty((n_streams, n), dtype=torch.int32, device=blob.device)
+    err = torch.zeros(1, dtype=torch.int32, device=blob.device)
+    _lib.call('fpcc_indexed_decode', *_table_args(tables, overflow), _p(blob), _p(byte_off), _p(byte_len), _p(idx), n, n_streams,
+              _p(out), _p(err), _s())
+    if int(err.item()):
+        raise RuntimeError('IndexedRansCoder: read past the end of a stream')
+    return out
+
+
 class IndexedRansCoder:
     def __init__(self, overflow_coding: bool, batch_size: int, enc_buf_size: int = 8 * 1024 * 1024):
         assert batch_size > 0
@@ -145,31 +183,13 @@ class IndexedRansCoder:
     def get_offset_array(self):
         return self.offset_array
 
-    def _targs(self):
-        flat, off, lens, offsets = self._t
-        return _p(flat), _p(off), _p(lens), len(self.cdfs), _p(offsets), int(self.overflow_coding)
-
     def _encode(self, symbol_array, index_array):
         sym = np.ascontiguousarray(symbol_array, dtype=np.int32)
         assert sym.ndim == 2 and sym.shape[0] == self.batch_size
         B, n = sym.shape
         d_sym = _dev(sym)
         d_idx = _dev(np.ascontiguousarray(index_array, dtype=np.int32)) if index_array is not None else None
-        cnt = torch.empty(B * n, dtype=torch.int32, device='cuda')
-        _lib.call('fpcc_indexed_count', *self._targs(), _p(d_sym), _p(d_idx), n, B, _p(cnt), _s())
-        incl = torch.cumsum(cnt.to(torch.int64), 0)
-        pos = (incl - cnt).contiguous()
-        total = int(incl[-1].item())
-        ranges = torch.empty(total, dtype=torch.int32, device='cuda')
-        bits = torch.empty(total, dtype=torch.uint8, device='cuda')
-        _lib.call('fpcc_indexed_ranges', *self._targs(), _p(d_sym), _p(d_idx), n, B, _p(pos), _p(ranges), _p(bits), _s())
-        rng_off = torch.cat([pos[::n], incl[-1:]]).contiguous()
-        per = (rng_off[1:] - rng_off[:-1])
-        cap = int(per.max().item()) * 2 + 64
-        out, out_len = ops.rans_encode(ranges, rng_off, cap, bits=bits)
-        out, out_len = out.cpu().numpy(), out_len.cpu().numpy()
-        assert (out_len > 0).all()
-        return [out[b, cap - out_len[b]:].tobytes() for b in range(B)]
+        return indexed_encode(self._t, self.overflow_coding, d_sym, d_idx, n, B)
 
     def encode(self, symbol_array):
         return self._encode(symbol_array, None)
@@ -183,13 +203,8 @@ class IndexedRansCoder:
         blob = np.frombuffer(b''.join(bytes(e) for e in encoded_list), dtype=np.uint8)
         lens = np.array([len(e) for e in encoded_list], dtype=np.int32)
         d_idx = _dev(np.ascontiguousarray(index_array, dtype=np.int32)) if index_array is not None else None
-        out = torch.empty((B, n), dtype=torch.int32, device='cuda')
-        err = torch.zeros(1, dtype=torch.int32, device='cuda')
         d_blob, d_off, d_len = _dev(blob), _dev(np.concatenate([[0], np.cumsum(lens[:-1])]).astype(np.int64)), _dev(lens)
-        _lib.call('fpcc_indexed_decode', *self._targs(), _p(d_blob), _p(d_off), _p(d_len), _p(d_idx), n, B, _p(out), _p(err), _s())
-        symbol_array[...] = out.cpu().numpy()
-        if int(err.item()):
-            raise RuntimeError('IndexedRansCoder: read past the end of a stream')
+        symbol_array[...] = indexed_decode(self._t, self.overflow_coding, d_blob, d_off, d_len, d_idx, n, B).cpu().numpy()
         return 0
 
     def decode(self, encoded_list, symbol_array):

@@ -9,7 +9,8 @@ all-reduce).
 forward and dgrad on the fused tcgen05 kernel, wgrad on `fpcc_spconv_wgrad_f16`.
 
 `LossyGeoNet` is the lossy geometry codec (lossy_coord_v2) in miniature on the MinkowskiEngine-shaped layers, trained
-with `train_step_lossy`.
+with `train_step_lossy`.  `LossyColorNet` adds a learned entropy bottleneck and a colour head to it: the joint
+geometry + colour codec (lossy_coord_lossy_color) in miniature, trained rate-distortion with `train_step_color`.
 """
 from typing import List
 
@@ -17,7 +18,8 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from . import lossy_heads, ops, synth
+from . import attributes, lossy_heads, ops, synth
+from .entropy_models import NoisyDeepFactorizedEntropyModel
 from . import me as ME
 from . import minkowski_sparse_conv_layers as L
 from .sparse_tensor import SparseTensor
@@ -85,10 +87,10 @@ class LossyGeoNet(nn.Module):
     tensor on a fresh coordinate manager (as ME training does per batch) and returns the sum of the two binary cross
     entropies against "the generated child is a voxel of the input"."""
 
-    def __init__(self, channels: int = 64):
+    def __init__(self, channels: int = 64, in_channels: int = 1):
         super().__init__()
         c = channels
-        self.enc0 = L.ConvBlock(1, 16, 3, 1)
+        self.enc0 = L.ConvBlock(in_channels, 16, 3, 1)
         self.enc1 = L.ConvBlock(16, c, 2, 2)
         self.res = L.ResBlock(c, 'HYPER_CUBE', False, 'relu')
         self.inception = L.InceptionResBlock(c, 'HYPER_CUBE', False, 'relu')
@@ -102,8 +104,15 @@ class LossyGeoNet(nn.Module):
 
     def forward(self, coords: torch.Tensor) -> torch.Tensor:
         x = ME.SparseTensor(torch.ones((coords.shape[0], 1), device=coords.device), coordinates=coords)
+        return self.decode(x, coords, self.encode(x))[0]
+
+    def encode(self, x):
+        """stride-1 input -> stride-2 features [n2, C]"""
+        return self.inception(self.res(self.enc1(self.enc0(x))))
+
+    def decode(self, x, coords, y):
+        """-> (bce1 + bce2, the refine branch's features on the kept key (stride 1))"""
         cm = x.coordinate_manager
-        y = self.inception(self.res(self.enc1(self.enc0(x))))
         g = self.gen(self.dec0(y))
         logits = self.head(self.mlp(g)).F.reshape(-1)
         # ground truth: the candidate voxel exists in the input (a 1x1x1 kernel map = one hash probe per candidate)
@@ -113,8 +122,9 @@ class LossyGeoNet(nn.Module):
         n_per_sample = torch.bincount(coords[:, 0].long()).tolist()
         keep = lossy_heads.get_keep(logits.detach(), g.C, 1, 2, target_points_num=n_per_sample) | gt
         kept = self.prune(g, keep)
-        logits2 = self.head2(self.tconv(y, kept.coordinate_map_key)).F.reshape(-1)
-        return loss + bce(logits2.float(), gt[keep].float())
+        r = self.tconv(y, kept.coordinate_map_key)
+        logits2 = self.head2(r).F.reshape(-1)
+        return loss + bce(logits2.float(), gt[keep].float()), r
 
 
 def make_lossy_batch(clouds: List[np.ndarray], device) -> torch.Tensor:
@@ -138,3 +148,70 @@ def train_step_lossy(model: nn.Module, opt: torch.optim.Optimizer, batch: torch.
         scaler.step(opt)
         scaler.update()
     return loss.detach()
+
+
+class LossyColorNet(LossyGeoNet):
+    """Joint geometry + colour codec (config 5, lossy_coord_lossy_color) in miniature: `LossyGeoNet`'s geometry path
+    plus a learned entropy bottleneck on the stride-2 latent and a colour branch, trained rate-distortion.
+
+      input     [1, Y, U, V] per voxel (BT.709 in [0, 1], attributes.rgb_to_yuv)
+      encoder   LossyGeoNet's, on 4 input channels                                                      stride 2
+      latent    MEMLPBlock(C -> L, no act) -> NoisyDeepFactorizedEntropyModel(L) -> MEMLPBlock(L -> C)
+      decoder   LossyGeoNet's occupancy decoder and refine branch, from the decoded latent
+      colour    MEMLPBlock(16 -> 3, no act) on the refine branch's features at the kept key = predicted YUV
+
+    loss = bce1 + bce2 + lambda_d * MSE_YUV(pred, yuv(recolor(org, org_rgb, kept))) + lambda_r * sum(bits) / n_points,
+    the colour target built under no_grad by `attributes.recolor` (two-way) from the input cloud.  Defaults:
+    latent L = 8, lambda_d = 10 (a YUV MSE of 1e-2 weighs like 0.1 of BCE), lambda_r = 0.01 (a bit per point weighs
+    like 0.01 of BCE).  forward(coords, rgb) -> (loss, {'bce', 'mse', 'bpp'} detached).
+
+    It stands in for the reference topology of SURVEY 3.4 (lossy_coord_lossy_color/model.py:167-214, layers.py:135-164
+    and 269-333, channels 32 / 64 / 128 of baseline_r1.yaml).  The reference source was not available when this was
+    written: the layer sizes are in miniature and parity with the reference's colour model is NOT claimed."""
+
+    def __init__(self, channels: int = 64, latent: int = 8, lambda_d: float = 10.0, lambda_r: float = 0.01):
+        super().__init__(channels, in_channels=4)
+        self.lambda_d, self.lambda_r = float(lambda_d), float(lambda_r)
+        self.to_latent = L.MEMLPBlock(channels, latent, act=None)
+        self.entropy_model = NoisyDeepFactorizedEntropyModel(latent)
+        self.from_latent = L.MEMLPBlock(latent, channels)
+        self.color_head = L.MEMLPBlock(16, 3, act=None)
+
+    def forward(self, coords: torch.Tensor, rgb: torch.Tensor):
+        yuv = attributes.rgb_to_yuv(rgb).float()
+        feats = torch.cat([torch.ones((coords.shape[0], 1), device=coords.device), yuv], 1)
+        x = ME.SparseTensor(feats, coordinates=coords)
+        z = self.to_latent(self.encode(x))
+        z_q, bits = self.entropy_model(z.F)
+        geo, r = self.decode(x, coords, self.from_latent(z._like(z_q)))
+        pred = self.color_head(r).F.float()
+        with torch.no_grad():
+            target = attributes.rgb_to_yuv(attributes.recolor(coords, rgb, r.C.contiguous())).float()
+        mse = torch.nn.functional.mse_loss(pred, target)
+        bpp = bits.sum() / coords.shape[0]
+        loss = geo + self.lambda_d * mse + self.lambda_r * bpp
+        return loss, {'bce': geo.detach(), 'mse': mse.detach(), 'bpp': bpp.detach()}
+
+
+def make_color_batch(clouds: List[np.ndarray], rgbs: List[np.ndarray], device):
+    """voxel clouds [n_b, 3] with uint8 colours [n_b, 3] (synth.colored_surface; unique rows) -> (int32 (batch, x, y, z)
+    rows in the shim's Morton order, uint8 [n, 3] colours in the same order)"""
+    c = torch.from_numpy(np.concatenate([synth.with_batch(xyz, b) for b, xyz in enumerate(clouds)])).to(device).to(torch.int32)
+    rgb = torch.from_numpy(np.concatenate(rgbs)).to(device)
+    order = ME.morton_order(c)
+    return c[order].contiguous(), rgb[order].contiguous()
+
+
+def train_step_color(model: nn.Module, opt: torch.optim.Optimizer, batch, scaler=None):
+    """One rate-distortion step of `LossyColorNet` (or a DistributedDataParallel around it), as `train_step_lossy`:
+    -> (loss, {'bce', 'mse', 'bpp'}), detached.  fp16 wants a GradScaler."""
+    opt.zero_grad(set_to_none=True)
+    loss, terms = model(*batch)
+    if scaler is None:
+        loss.backward()
+        opt.step()
+    else:
+        scaler.scale(loss).backward()
+        scaler.step(opt)
+        scaler.update()
+    return loss.detach(), terms

@@ -19,6 +19,7 @@
  *   lib/entropy_models/rans_coder/rans_wrapper.cpp:430-451  IndexedRansCoder / BinaryRansCoder / batched_pmf_to_quantized_cdf
  *   models/convolutional/lossl_coord_int/model.py:261-295, 344-353, 81-91   get_bin / batch_quantize_pmf_torch / child generation
  *   lib/knn3d/src/knn3d.cu:25,75                        KNearestNeighborKernelV0/V2 (fpcc_knn_search)
+ *   lib/entropy_models/distributions/deep_factorized.py   NoisyDeepFactorized likelihood (fpcc_factorized_*; not a verified drop-in)
  */
 #ifndef FASTPCC_B200_H_
 #define FASTPCC_B200_H_
@@ -493,6 +494,30 @@ int fpcc_indexed_decode(const uint32_t *cdf_flat, const int64_t *cdf_off, const 
  * of table t, or -1 when no frequency could be stolen. */
 int fpcc_pmf_to_quantized_cdf(double *pmf, int n_tables, int pmf_size, int32_t *offsets, int overflow,
                               uint32_t *cdf_out, int32_t *cdf_len, void *stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Deep-factorized entropy model (csrc/entropy_model.cu; DESIGN 3.10).  params fp32 [C, 43], one row per channel:
+ *   H0[3x1] b0[3] a0[3] | H1[3x3] b1[3] a1[3] | H2[3x3] b2[3] a2[3] | H3[1x3] b3[1]    (H row-major [out][in])
+ * f_c(x): v = x; per layer v <- softplus(H_i) v + b_i, and for i < 3 v <- v + tanh(a_i) * tanh(v) (monotone in x).
+ * L_c(y) = |sigmoid(s u) - sigmoid(s l)|, u = f_c(y + 1/2), l = f_c(y - 1/2), s = -1 if u + l > 0 else +1.
+ * bits = -log2(max(L, bound)), 0 < bound < 1.  The gradient at the bound follows compressai's LowerBound: it passes
+ * where L >= bound or where it would raise L.  The parity of this definition with the reference is unpinned.
+ * ---------------------------------------------------------------------------------------------- */
+
+/* bits fp32 [n, C] (dense) of y fp32 [n, C] with row pitch ld_y >= C */
+int fpcc_factorized_bits(const float *y, int64_t ld_y, int64_t n, int C, const float *params, float bound, float *bits,
+                         void *stream);
+/* dy fp32 [n, C] (dense) and dparams fp32 [C, 43] (with respect to the RAW params, through softplus / tanh) from the
+ * upstream dbits [n, C] (row pitch ld_db).  The forward is recomputed; dparams is reduced from fp64 per-CTA partials
+ * in a fixed order (no float atomics), so it is reproducible bit for bit.  workspace: fpcc_factorized_grad_workspace
+ * bytes. */
+size_t fpcc_factorized_grad_workspace(int64_t n, int C);
+int fpcc_factorized_grad(const float *y, int64_t ld_y, const float *dbits, int64_t ld_db, int64_t n, int C,
+                         const float *params, float bound, float *dy, float *dparams, void *workspace,
+                         size_t workspace_bytes, void *stream);
+/* pmf fp64 [C, n_sym]: pmf[c, k] = L_c(lo + k), unbounded, by the device function of fpcc_factorized_bits (the input
+ * of fpcc_pmf_to_quantized_cdf) */
+int fpcc_factorized_pmf(const float *params, int C, int lo, int n_sym, double *pmf, void *stream);
 
 #ifdef __cplusplus
 }
