@@ -92,6 +92,11 @@ SIGNATURES = {
     'fpcc_factorized_grad_workspace': (_sz, [_i64, _i]),
     'fpcc_factorized_grad': (_i, [_vp, _i64, _vp, _i64, _i64, _i, _vp, C.c_float, _vp, _vp, _vp, _sz, _vp]),
     'fpcc_factorized_pmf': (_i, [_vp, _i, _i, _i, _vp, _vp]),
+    'fpcc_gaussian_bits': (_i, [_vp, _i64, _vp, _i64, _vp, _i64, _i64, _i, C.c_float, C.c_float, _vp, _vp]),
+    'fpcc_gaussian_grad': (_i, [_vp, _i64, _vp, _i64, _vp, _i64, _vp, _i64, _i64, _i, C.c_float, C.c_float, _vp, _vp, _vp, _vp]),
+    'fpcc_gaussian_tail_multiplier': (C.c_double, [C.c_double]),
+    'fpcc_gaussian_pmf': (_i, [_vp, _i, C.c_double, _i, _vp, _vp, _vp]),
+    'fpcc_gaussian_indexes': (_i, [_vp, _i64, _vp, _i64, _vp, _i64, _i64, _i, C.c_float, _vp, _i, _vp, _vp, _vp]),
 }
 
 _LIB = None

@@ -15,6 +15,8 @@ kernels, shared by the torchsparse-shaped layers (`torchsparse_nn.py`) and the M
 
 The deep-factorized entropy model (`FactorizedBitsFunction`) is one fused kernel each way: bits of the latents forward,
 dy and the packed parameter gradient backward (`fpcc_factorized_bits` / `fpcc_factorized_grad`).
+The Gaussian conditional model of the hyperprior (`GaussianBitsFunction`) likewise: bits forward, dy, dmu and dsigma
+backward (`fpcc_gaussian_bits` / `fpcc_gaussian_grad`).
 
 MinkowskiEngine computes the same three products per kernel offset (ME backward = transposed gather-GEMM-scatter).
 The ME layer kinds map onto these products as follows (`MELayerFunction`):
@@ -245,3 +247,29 @@ class FactorizedBitsFunction(torch.autograd.Function):
 def factorized_bits(y, params, bound=1e-9):
     """differentiable bits of the deep-factorized prior; y is cast to fp32 (latents arrive in the compute dtype)"""
     return FactorizedBitsFunction.apply(y.float(), params, float(bound))
+
+
+class GaussianBitsFunction(torch.autograd.Function):
+    """bits = -log2(max(L, bound)) of the Gaussian conditional model (fpcc_gaussian_bits): y, scales, means fp32 [n, C]
+    (means None: mean 0; means and scales may be column slices of one tensor).  The backward recomputes the forward in
+    the kernel and returns dy, dscales and dmeans."""
+
+    @staticmethod
+    def forward(ctx, y, scales, means, scale_bound, bound):
+        ctx.save_for_backward(y, scales, means)
+        ctx.scale_bound, ctx.bound = scale_bound, bound
+        return ops.gaussian_bits(y, scales, means, scale_bound, bound)
+
+    @staticmethod
+    def backward(ctx, dbits):
+        y, scales, means = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        dy, dm, ds = ops.gaussian_grad(y, scales, dbits.float(), means, ctx.scale_bound, ctx.bound, need_dmu=need[2])
+        return (dy if need[0] else None), (ds if need[1] else None), (dm if need[2] else None), None, None
+
+
+def gaussian_bits(y, scales, means=None, scale_bound=0.11, likelihood_bound=1e-9):
+    """differentiable bits of the Gaussian conditional model; y, scales and means are cast to fp32 (they arrive in the
+    shim's compute dtype)"""
+    return GaussianBitsFunction.apply(y.float(), scales.float(), None if means is None else means.float(),
+                                      float(scale_bound), float(likelihood_bound))

@@ -317,3 +317,230 @@ extern "C" int fpcc_factorized_pmf(const float *params, int C, int lo, int n_sym
     FPCC_LAUNCH_CHECK();
     return FPCC_OK;
 }
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Gaussian conditional (the mean-scale hyperprior's conditional model; DESIGN 3.11).  After compressai's
+// GaussianConditional; parity with the reference's indexed models is unpinned.
+//   v = |y - mu| (mu = 0 when absent), s = max(sigma, scale_bound), u = (1/2 - v) / s, l = (-1/2 - v) / s
+//   L = Phi(u) - Phi(l), Phi(x) = erfc(-x / sqrt 2) / 2 (erfcf: both terms keep their relative precision in the lower
+//   tail), bits = -log2(max(L, bound)).  Both lower bounds pass gradients as compressai's LowerBound does.
+// Elementwise: thread t of a 256-thread CTA -> channel t % cb of a slice of at most SLICE channels, row lane t / cb, 8
+// elements per thread (the factorized kernels' mapping, without the staged parameters).  No reduction anywhere.
+// ---------------------------------------------------------------------------------------------------------------------
+namespace fpcc {
+
+constexpr float GC_RSQRT2 = 0.70710678118654752f;
+constexpr float GC_RSQRT2PI = 0.39894228040143268f;
+constexpr float GC_LN2 = 0.69314718055994531f;
+
+__device__ __forceinline__ float gc_cdf(float x) { return 0.5f * erfcf(-x * GC_RSQRT2); }
+__device__ __forceinline__ float gc_density(float x) { return GC_RSQRT2PI * expf(-0.5f * x * x); }
+
+// L at distance v >= 0 from the mean, scale s > 0 (already bounded); *u_out, *l_out = the standardised interval ends
+__device__ __forceinline__ float gc_likelihood(float v, float s, float *u_out, float *l_out) {
+    const float u = (0.5f - v) / s, l = (-0.5f - v) / s;
+    *u_out = u; *l_out = l;
+    return gc_cdf(u) - gc_cdf(l);
+}
+
+__global__ void __launch_bounds__(EM_THREADS) gaussian_bits_kernel(const float *__restrict__ y, int64_t ld_y,
+                                                                   const float *__restrict__ mu, int64_t ld_mu,
+                                                                   const float *__restrict__ sigma, int64_t ld_s, int64_t n,
+                                                                   int C, float scale_bound, float bound, int rows_per_cta,
+                                                                   float *__restrict__ bits) {
+    const int c0 = blockIdx.y * SLICE;
+    const int cb = min(SLICE, C - c0), rl_n = EM_THREADS / cb;
+    const int cl = threadIdx.x % cb, rl = threadIdx.x / cb;
+    if (rl >= rl_n) return;
+    const int c = c0 + cl;
+    const int64_t r0 = (int64_t)blockIdx.x * rows_per_cta;
+    const int64_t r1 = min(r0 + rows_per_cta, n);
+    for (int64_t r = r0 + rl; r < r1; r += rl_n) {
+        const float m = mu ? __ldg(&mu[r * ld_mu + c]) : 0.f;
+        const float v = fabsf(__ldg(&y[r * ld_y + c]) - m);
+        const float s = fmaxf(__ldg(&sigma[r * ld_s + c]), scale_bound);
+        float u, l;
+        const float L = gc_likelihood(v, s, &u, &l);
+        bits[r * C + c] = -log2f(fmaxf(L, bound));
+    }
+}
+
+__global__ void __launch_bounds__(EM_THREADS) gaussian_grad_kernel(const float *__restrict__ y, int64_t ld_y,
+                                                                   const float *__restrict__ mu, int64_t ld_mu,
+                                                                   const float *__restrict__ sigma, int64_t ld_s,
+                                                                   const float *__restrict__ dbits, int64_t ld_db, int64_t n,
+                                                                   int C, float scale_bound, float bound, int rows_per_cta,
+                                                                   float *__restrict__ dy, float *__restrict__ dmu,
+                                                                   float *__restrict__ dsigma) {
+    const int c0 = blockIdx.y * SLICE;
+    const int cb = min(SLICE, C - c0), rl_n = EM_THREADS / cb;
+    const int cl = threadIdx.x % cb, rl = threadIdx.x / cb;
+    if (rl >= rl_n) return;
+    const int c = c0 + cl;
+    const int64_t r0 = (int64_t)blockIdx.x * rows_per_cta;
+    const int64_t r1 = min(r0 + rows_per_cta, n);
+    for (int64_t r = r0 + rl; r < r1; r += rl_n) {
+        const float m = mu ? __ldg(&mu[r * ld_mu + c]) : 0.f;
+        const float d = __ldg(&y[r * ld_y + c]) - m;
+        const float v = fabsf(d);
+        const float sr = __ldg(&sigma[r * ld_s + c]);
+        const float s = fmaxf(sr, scale_bound);
+        float u, l;
+        const float L = gc_likelihood(v, s, &u, &l);
+        const float Lb = fmaxf(L, bound);
+        // d bits / d Lb = -1 / (Lb ln 2); LowerBound: passes where L >= bound or where it is negative (raises L)
+        float gL = -__ldg(&dbits[r * ld_db + c]) / (Lb * GC_LN2);
+        if (!(L >= bound || gL < 0.f)) gL = 0.f;
+        const float pu = gc_density(u), pl = gc_density(l);
+        const float dLdv = (pl - pu) / s;
+        const float dLds = (l * pl - u * pu) / s;
+        const float sg = d > 0.f ? 1.f : (d < 0.f ? -1.f : 0.f);  // torch's abs' (0 at 0)
+        const float gy = gL * dLdv * sg;
+        float gs = gL * dLds;
+        if (!(sr >= scale_bound || gs < 0.f)) gs = 0.f;          // the scale's LowerBound
+        const int64_t o = r * C + c;
+        dy[o] = gy;
+        if (dmu) dmu[o] = -gy;
+        dsigma[o] = gs;
+    }
+}
+
+// one CTA per table t: pmf[t, k] = L(|k - center_t|, scale_table[t]) for k <= 2 center_t (cut at S), 0 beyond
+__global__ void __launch_bounds__(256) gaussian_pmf_kernel(const float *__restrict__ scale_table, double m, int S,
+                                                           double *__restrict__ pmf, int32_t *__restrict__ offsets) {
+    const int t = blockIdx.x;
+    const float s = __ldg(&scale_table[t]);
+    const int center = (int)ceil((double)s * m);
+    if (threadIdx.x == 0) offsets[t] = -center;
+    for (int k = threadIdx.x; k < S; k += blockDim.x) {
+        double p = 0.0;
+        if (k <= 2 * center) {
+            float u, l;
+            p = (double)gc_likelihood(fabsf((float)(k - center)), s, &u, &l);
+        }
+        pmf[(int64_t)t * S + k] = p;
+    }
+}
+
+// idx = first t with scale_table[t] >= max(sigma, scale_bound), capped at T - 1; with y also sym = rint(y - mu)
+__global__ void __launch_bounds__(EM_THREADS) gaussian_indexes_kernel(const float *__restrict__ y, int64_t ld_y,
+                                                                      const float *__restrict__ mu, int64_t ld_mu,
+                                                                      const float *__restrict__ sigma, int64_t ld_s,
+                                                                      int64_t n, int C, float scale_bound,
+                                                                      const float *__restrict__ scale_table, int T,
+                                                                      int rows_per_cta, int32_t *__restrict__ sym,
+                                                                      int32_t *__restrict__ idx) {
+    const int c0 = blockIdx.y * SLICE;
+    const int cb = min(SLICE, C - c0), rl_n = EM_THREADS / cb;
+    const int cl = threadIdx.x % cb, rl = threadIdx.x / cb;
+    if (rl >= rl_n) return;
+    const int c = c0 + cl;
+    const int64_t r0 = (int64_t)blockIdx.x * rows_per_cta;
+    const int64_t r1 = min(r0 + rows_per_cta, n);
+    for (int64_t r = r0 + rl; r < r1; r += rl_n) {
+        const float s = fmaxf(__ldg(&sigma[r * ld_s + c]), scale_bound);
+        int a = 0, b = T - 1;  // lower bound over scale_table[0 .. T - 1), T - 1 when none is >= s
+        while (a < b) {
+            const int mid = (a + b) >> 1;
+            if (__ldg(&scale_table[mid]) >= s) b = mid; else a = mid + 1;
+        }
+        const int64_t o = r * C + c;
+        idx[o] = a;
+        if (y) {
+            const float m = mu ? __ldg(&mu[r * ld_mu + c]) : 0.f;
+            sym[o] = (int32_t)rintf(__ldg(&y[r * ld_y + c]) - m);
+        }
+    }
+}
+
+// host: Phi^-1(p) for 0 < p < 1/2 by bisection on erfc in double (monotone; 200 halvings reach the last bit)
+static double normal_quantile_lower(double p) {
+    double lo = -40.0, hi = 0.0;
+    for (int i = 0; i < 200; ++i) {
+        const double mid = 0.5 * (lo + hi);
+        if (mid == lo || mid == hi) break;
+        if (0.5 * erfc(-mid * 0.70710678118654752440) < p) lo = mid; else hi = mid;
+    }
+    return hi;
+}
+
+// launch geometry of the elementwise kernels: (CTAs along the rows, rows per CTA)
+static int gc_rows_per_cta(int C) { return (EM_THREADS / (C < SLICE ? C : SLICE)) * 8; }  // 8 elements per thread
+
+}  // namespace fpcc
+
+static bool scale_bound_ok(float b) { return b > 0.f && b <= 3.0e38f; }  // false for NaN and inf
+
+extern "C" double fpcc_gaussian_tail_multiplier(double tail_mass) {
+    if (!(tail_mass > 0.0 && tail_mass < 1.0)) return NAN;
+    return -normal_quantile_lower(0.5 * tail_mass);
+}
+
+extern "C" int fpcc_gaussian_bits(const float *y, int64_t ld_y, const float *mu, int64_t ld_mu, const float *sigma, int64_t ld_s,
+                                  int64_t n, int C, float scale_bound, float bound, float *bits, void *stream) {
+    FPCC_REQUIRE(y && sigma && bits, "gaussian_bits: NULL pointer");
+    FPCC_REQUIRE(C > 0 && C <= (1 << 22), "gaussian_bits: C %d must be in 1..2^22", C);
+    FPCC_REQUIRE(n >= 0 && n <= ((int64_t)1 << 40), "gaussian_bits: bad row count");
+    FPCC_REQUIRE(ld_y >= C && ld_s >= C && (!mu || ld_mu >= C), "gaussian_bits: row pitch below the channel count");
+    FPCC_REQUIRE(scale_bound_ok(scale_bound), "gaussian_bits: scale bound must be positive and finite");
+    FPCC_REQUIRE(bound_ok(bound), "gaussian_bits: likelihood bound must be in (0, 1)");
+    if (n == 0) return FPCC_OK;
+    const int rows = gc_rows_per_cta(C);
+    const int64_t ctas = (n + rows - 1) / rows;
+    FPCC_REQUIRE(ctas <= INT32_MAX, "gaussian_bits: too many rows");
+    gaussian_bits_kernel<<<dim3((unsigned)ctas, ceil_div(C, SLICE)), EM_THREADS, 0, (cudaStream_t)stream>>>(
+        y, ld_y, mu, ld_mu, sigma, ld_s, n, C, scale_bound, bound, rows, bits);
+    FPCC_LAUNCH_CHECK();
+    return FPCC_OK;
+}
+
+extern "C" int fpcc_gaussian_grad(const float *y, int64_t ld_y, const float *mu, int64_t ld_mu, const float *sigma, int64_t ld_s,
+                                  const float *dbits, int64_t ld_db, int64_t n, int C, float scale_bound, float bound, float *dy,
+                                  float *dmu, float *dsigma, void *stream) {
+    FPCC_REQUIRE(y && sigma && dbits && dy && dsigma, "gaussian_grad: NULL pointer");
+    FPCC_REQUIRE(mu || !dmu, "gaussian_grad: dmu needs mu");
+    FPCC_REQUIRE(C > 0 && C <= (1 << 22), "gaussian_grad: C %d must be in 1..2^22", C);
+    FPCC_REQUIRE(n >= 0 && n <= ((int64_t)1 << 40), "gaussian_grad: bad row count");
+    FPCC_REQUIRE(ld_y >= C && ld_s >= C && ld_db >= C && (!mu || ld_mu >= C), "gaussian_grad: row pitch below the channel count");
+    FPCC_REQUIRE(scale_bound_ok(scale_bound), "gaussian_grad: scale bound must be positive and finite");
+    FPCC_REQUIRE(bound_ok(bound), "gaussian_grad: likelihood bound must be in (0, 1)");
+    if (n == 0) return FPCC_OK;
+    const int rows = gc_rows_per_cta(C);
+    const int64_t ctas = (n + rows - 1) / rows;
+    FPCC_REQUIRE(ctas <= INT32_MAX, "gaussian_grad: too many rows");
+    gaussian_grad_kernel<<<dim3((unsigned)ctas, ceil_div(C, SLICE)), EM_THREADS, 0, (cudaStream_t)stream>>>(
+        y, ld_y, mu, ld_mu, sigma, ld_s, dbits, ld_db, n, C, scale_bound, bound, rows, dy, dmu, dsigma);
+    FPCC_LAUNCH_CHECK();
+    return FPCC_OK;
+}
+
+extern "C" int fpcc_gaussian_pmf(const float *scale_table, int T, double tail_mass, int S, double *pmf, int32_t *offsets,
+                                 void *stream) {
+    FPCC_REQUIRE(scale_table && pmf && offsets, "gaussian_pmf: NULL pointer");
+    FPCC_REQUIRE(T > 0 && T <= (1 << 16), "gaussian_pmf: T %d must be in 1..65536", T);
+    FPCC_REQUIRE(tail_mass > 0.0 && tail_mass < 1.0, "gaussian_pmf: tail mass must be in (0, 1)");
+    FPCC_REQUIRE(S > 0 && S <= (1 << 20), "gaussian_pmf: S %d must be in 1..2^20", S);
+    gaussian_pmf_kernel<<<T, 256, 0, (cudaStream_t)stream>>>(scale_table, fpcc_gaussian_tail_multiplier(tail_mass), S, pmf, offsets);
+    FPCC_LAUNCH_CHECK();
+    return FPCC_OK;
+}
+
+extern "C" int fpcc_gaussian_indexes(const float *y, int64_t ld_y, const float *mu, int64_t ld_mu, const float *sigma, int64_t ld_s,
+                                     int64_t n, int C, float scale_bound, const float *scale_table, int T, int32_t *sym,
+                                     int32_t *idx, void *stream) {
+    FPCC_REQUIRE(sigma && scale_table && idx, "gaussian_indexes: NULL pointer");
+    FPCC_REQUIRE(!y == !sym, "gaussian_indexes: y and sym go together (both or neither)");
+    FPCC_REQUIRE(C > 0 && C <= (1 << 22), "gaussian_indexes: C %d must be in 1..2^22", C);
+    FPCC_REQUIRE(n >= 0 && n <= ((int64_t)1 << 40), "gaussian_indexes: bad row count");
+    FPCC_REQUIRE(ld_s >= C && (!y || ld_y >= C) && (!mu || ld_mu >= C), "gaussian_indexes: row pitch below the channel count");
+    FPCC_REQUIRE(scale_bound_ok(scale_bound), "gaussian_indexes: scale bound must be positive and finite");
+    FPCC_REQUIRE(T > 0 && T <= (1 << 16), "gaussian_indexes: T %d must be in 1..65536", T);
+    if (n == 0) return FPCC_OK;
+    const int rows = gc_rows_per_cta(C);
+    const int64_t ctas = (n + rows - 1) / rows;
+    FPCC_REQUIRE(ctas <= INT32_MAX, "gaussian_indexes: too many rows");
+    gaussian_indexes_kernel<<<dim3((unsigned)ctas, ceil_div(C, SLICE)), EM_THREADS, 0, (cudaStream_t)stream>>>(
+        y, ld_y, mu, ld_mu, sigma, ld_s, n, C, scale_bound, scale_table, T, rows, sym, idx);
+    FPCC_LAUNCH_CHECK();
+    return FPCC_OK;
+}

@@ -794,3 +794,111 @@ def factorized_pmf(params, lo=-64, n_sym=129):
     pmf = torch.empty((params.shape[0], n_sym), dtype=torch.float64, device=params.device)
     _call('fpcc_factorized_pmf', _p(params), params.shape[0], int(lo), int(n_sym), _p(pmf), _s())
     return pmf
+
+
+# ---------------------------------------------------------------------------------------------
+# Gaussian conditional entropy model (csrc/entropy_model.cu)
+# ---------------------------------------------------------------------------------------------
+def _gc_rows(t, n, c, name):
+    if t.dtype != torch.float32 or not t.is_cuda or t.dim() != 2 or t.shape[1] != c or t.shape[0] != n:
+        raise RuntimeError(f'gaussian conditional: {name} must be a 2-D fp32 CUDA tensor [{n}, {c}]')
+    return t if t.stride(1) == 1 and t.stride(0) >= c else t.contiguous()  # any row pitch >= c: column slices pass as they are
+
+
+def _gc_scales(scales):
+    if scales.dtype != torch.float32 or scales.dim() != 2 or scales.shape[1] < 1:
+        raise RuntimeError('gaussian conditional: scales must be a 2-D fp32 tensor [n, C]')
+    return scales.shape[0], scales.shape[1]
+
+
+def _gc_table(scale_table):
+    """strictly increasing, positive fp32 scale table [T] (read on the host once per call)"""
+    if scale_table.dtype != torch.float32 or scale_table.dim() != 1 or scale_table.numel() < 1:
+        raise RuntimeError('gaussian conditional: scale_table must be a non-empty 1-D fp32 tensor')
+    h = scale_table.detach().cpu()
+    if not bool((h > 0).all()) or not bool(torch.isfinite(h).all()):
+        raise RuntimeError('gaussian conditional: scale_table must be positive and finite')
+    if h.numel() > 1 and not bool((h[1:] > h[:-1]).all()):
+        raise RuntimeError('gaussian conditional: scale_table must be strictly increasing')
+    if not scale_table.is_cuda:
+        raise RuntimeError('gaussian conditional: scale_table must be a CUDA tensor')
+    return scale_table.contiguous(), h
+
+
+def _gc_bounds(scale_bound, bound=0.5):
+    if not (0.0 < scale_bound < float('inf')):
+        raise RuntimeError('gaussian conditional: scale_bound must be positive and finite')
+    if not (0.0 < bound < 1.0):
+        raise RuntimeError('gaussian conditional: likelihood bound must be in (0, 1)')
+
+
+def gaussian_bits(y, scales, means=None, scale_bound=0.11, bound=1e-9):
+    """-log2(max(L, bound)) per element (DESIGN 3.11): y, scales, means fp32 [n, C], any row pitch >= C (means None:
+    mean 0) -> bits fp32 [n, C]"""
+    _gc_bounds(scale_bound, bound)
+    n, c = _gc_scales(scales)
+    s, y = _gc_rows(scales, n, c, 'scales'), _gc_rows(y, n, c, 'y')
+    m = None if means is None else _gc_rows(means, n, c, 'means')
+    bits = torch.empty((n, c), dtype=torch.float32, device=y.device)
+    _call('fpcc_gaussian_bits', _p(y), y.stride(0), _p(m), 0 if m is None else m.stride(0), _p(s), s.stride(0), n, c,
+          float(scale_bound), float(bound), _p(bits), _s(), work={'bytes': 4.0 * n * c * (4 if m is not None else 3)})
+    return bits
+
+
+def gaussian_grad(y, scales, dbits, means=None, scale_bound=0.11, bound=1e-9, need_dmu=True):
+    """-> (dy, dmu | None, dscales), fp32 [n, C] each, of sum(dbits * gaussian_bits(y, scales, means)); dmu = -dy, only
+    with means and need_dmu"""
+    _gc_bounds(scale_bound, bound)
+    n, c = _gc_scales(scales)
+    s, y, dbits = _gc_rows(scales, n, c, 'scales'), _gc_rows(y, n, c, 'y'), _gc_rows(dbits, n, c, 'dbits')
+    m = None if means is None else _gc_rows(means, n, c, 'means')
+    dy = torch.empty((n, c), dtype=torch.float32, device=y.device)
+    ds = torch.empty_like(dy)
+    dm = torch.empty_like(dy) if (m is not None and need_dmu) else None
+    _call('fpcc_gaussian_grad', _p(y), y.stride(0), _p(m), 0 if m is None else m.stride(0), _p(s), s.stride(0), _p(dbits),
+          dbits.stride(0), n, c, float(scale_bound), float(bound), _p(dy), _p(dm), _p(ds), _s(),
+          work={'bytes': 4.0 * n * c * (4 + (m is not None) + 2 + (dm is not None))})
+    return dy, dm, ds
+
+
+def gaussian_tail_multiplier(tail_mass=1e-9):
+    """m = -Phi^-1(tail_mass / 2): the table of scale s spans ceil(s m) symbols either side of the mean"""
+    if not (0.0 < tail_mass < 1.0):
+        raise RuntimeError('gaussian conditional: tail_mass must be in (0, 1)')
+    return float(_lib.load().fpcc_gaussian_tail_multiplier(float(tail_mass)))
+
+
+def gaussian_centers(scale_table, tail_mass=1e-9):
+    """center_t = ceil(scale_table[t] * m) in double, as fpcc_gaussian_pmf computes them -> int64 [T] on the host"""
+    _, h = _gc_table(scale_table)
+    return torch.ceil(h.double() * gaussian_tail_multiplier(tail_mass)).to(torch.int64)
+
+
+def gaussian_pmf(scale_table, tail_mass=1e-9):
+    """-> (pmf fp64 [T, S], offsets int32 [T]) on the device: row t = L(k) at sigma = scale_table[t] for
+    k = -center_t .. center_t, zero-padded to S = 2 max(center) + 1; offsets = -center"""
+    table, h = _gc_table(scale_table)
+    centers = torch.ceil(h.double() * gaussian_tail_multiplier(tail_mass))
+    T, S = table.numel(), 2 * int(centers.max()) + 1
+    if S > (1 << 20):
+        raise RuntimeError(f'gaussian conditional: a table of {S} symbols is over 2^20 (lower the largest scale or raise tail_mass)')
+    pmf = torch.empty((T, S), dtype=torch.float64, device=table.device)
+    offsets = torch.empty(T, dtype=torch.int32, device=table.device)
+    _call('fpcc_gaussian_pmf', _p(table), T, float(tail_mass), S, _p(pmf), _p(offsets), _s())
+    return pmf, offsets
+
+
+def gaussian_indexes(scale_table, scales, means=None, y=None, scale_bound=0.11):
+    """idx int32 [n, C]: the first table t with scale_table[t] >= max(scales, scale_bound), capped at T - 1.  With y,
+    -> (sym, idx), sym int32 [n, C] = rint(y - means) (half to even) from the same pass."""
+    table, _ = _gc_table(scale_table)
+    _gc_bounds(scale_bound)
+    n, c = _gc_scales(scales)
+    s = _gc_rows(scales, n, c, 'scales')
+    m = None if means is None else _gc_rows(means, n, c, 'means')
+    yy = None if y is None else _gc_rows(y, n, c, 'y')
+    idx = torch.empty((n, c), dtype=torch.int32, device=s.device)
+    sym = None if y is None else torch.empty_like(idx)
+    _call('fpcc_gaussian_indexes', _p(yy), 0 if yy is None else yy.stride(0), _p(m), 0 if m is None else m.stride(0), _p(s),
+          s.stride(0), n, c, float(scale_bound), _p(table), table.numel(), _p(sym), _p(idx), _s())
+    return idx if y is None else (sym, idx)

@@ -19,7 +19,7 @@ import torch
 import torch.nn as nn
 
 from . import attributes, lossy_heads, ops, synth
-from .entropy_models import NoisyDeepFactorizedEntropyModel
+from .entropy_models import HyperpriorEntropyModel, NoisyDeepFactorizedEntropyModel
 from . import me as ME
 from . import minkowski_sparse_conv_layers as L
 from .sparse_tensor import SparseTensor
@@ -165,15 +165,24 @@ class LossyColorNet(LossyGeoNet):
     latent L = 8, lambda_d = 10 (a YUV MSE of 1e-2 weighs like 0.1 of BCE), lambda_r = 0.01 (a bit per point weighs
     like 0.01 of BCE).  forward(coords, rgb) -> (loss, {'bce', 'mse', 'bpp'} detached).
 
+    prior='hyperprior' replaces the deep-factorized latent prior with `HyperpriorEntropyModel(L, L, C)` (a mean-scale
+    hyperprior at stride 4); sum(bits) is then the latent's plus the hyper-latent's, and bpp their sum per point.
+
     It stands in for the reference topology of SURVEY 3.4 (lossy_coord_lossy_color/model.py:167-214, layers.py:135-164
     and 269-333, channels 32 / 64 / 128 of baseline_r1.yaml).  The reference source was not available when this was
     written: the layer sizes are in miniature and parity with the reference's colour model is NOT claimed."""
 
-    def __init__(self, channels: int = 64, latent: int = 8, lambda_d: float = 10.0, lambda_r: float = 0.01):
+    def __init__(self, channels: int = 64, latent: int = 8, lambda_d: float = 10.0, lambda_r: float = 0.01,
+                 prior: str = 'factorized'):
         super().__init__(channels, in_channels=4)
-        self.lambda_d, self.lambda_r = float(lambda_d), float(lambda_r)
+        if prior not in ('factorized', 'hyperprior'):
+            raise ValueError(f"LossyColorNet: prior must be 'factorized' or 'hyperprior', not {prior!r}")
+        self.lambda_d, self.lambda_r, self.prior = float(lambda_d), float(lambda_r), prior
         self.to_latent = L.MEMLPBlock(channels, latent, act=None)
-        self.entropy_model = NoisyDeepFactorizedEntropyModel(latent)
+        if prior == 'factorized':
+            self.entropy_model = NoisyDeepFactorizedEntropyModel(latent)
+        else:
+            self.entropy_model = HyperpriorEntropyModel(latent, latent, channels)
         self.from_latent = L.MEMLPBlock(latent, channels)
         self.color_head = L.MEMLPBlock(16, 3, act=None)
 
@@ -182,13 +191,18 @@ class LossyColorNet(LossyGeoNet):
         feats = torch.cat([torch.ones((coords.shape[0], 1), device=coords.device), yuv], 1)
         x = ME.SparseTensor(feats, coordinates=coords)
         z = self.to_latent(self.encode(x))
-        z_q, bits = self.entropy_model(z.F)
-        geo, r = self.decode(x, coords, self.from_latent(z._like(z_q)))
+        if self.prior == 'factorized':
+            z_q, bits = self.entropy_model(z.F)
+            z_q, rate = z._like(z_q), bits.sum()
+        else:
+            z_q, bits_y, bits_z = self.entropy_model(z)
+            rate = bits_y.sum() + bits_z.sum()
+        geo, r = self.decode(x, coords, self.from_latent(z_q))
         pred = self.color_head(r).F.float()
         with torch.no_grad():
             target = attributes.rgb_to_yuv(attributes.recolor(coords, rgb, r.C.contiguous())).float()
         mse = torch.nn.functional.mse_loss(pred, target)
-        bpp = bits.sum() / coords.shape[0]
+        bpp = rate / coords.shape[0]
         loss = geo + self.lambda_d * mse + self.lambda_r * bpp
         return loss, {'bce': geo.detach(), 'mse': mse.detach(), 'bpp': bpp.detach()}
 

@@ -20,6 +20,8 @@
  *   models/convolutional/lossl_coord_int/model.py:261-295, 344-353, 81-91   get_bin / batch_quantize_pmf_torch / child generation
  *   lib/knn3d/src/knn3d.cu:25,75                        KNearestNeighborKernelV0/V2 (fpcc_knn_search)
  *   lib/entropy_models/distributions/deep_factorized.py   NoisyDeepFactorized likelihood (fpcc_factorized_*; not a verified drop-in)
+ *   lib/entropy_models/distributions/ (noisy normal), continuous_indexed.py   Gaussian conditional likelihood and indexed
+ *                                                       tables (fpcc_gaussian_*; not a verified drop-in)
  */
 #ifndef FASTPCC_B200_H_
 #define FASTPCC_B200_H_
@@ -518,6 +520,38 @@ int fpcc_factorized_grad(const float *y, int64_t ld_y, const float *dbits, int64
 /* pmf fp64 [C, n_sym]: pmf[c, k] = L_c(lo + k), unbounded, by the device function of fpcc_factorized_bits (the input
  * of fpcc_pmf_to_quantized_cdf) */
 int fpcc_factorized_pmf(const float *params, int C, int lo, int n_sym, double *pmf, void *stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Gaussian conditional entropy model (csrc/entropy_model.cu; DESIGN 3.11), after compressai's GaussianConditional.
+ * All float inputs are fp32 rows [n, C] with a row pitch ld_* >= C (mu and sigma may be the two column halves of
+ * one [n, 2C] tensor); mu may be NULL (mean 0).  Per element:
+ *   v = |y - mu|, s = max(sigma, scale_bound), u = (1/2 - v) / s, l = (-1/2 - v) / s,
+ *   L = Phi(u) - Phi(l), Phi(x) = erfc(-x / sqrt 2) / 2 (erfcf), bits = -log2(max(L, bound)), 0 < bound < 1.
+ * Both lower bounds pass gradients as compressai's LowerBound: where the value is at or above the bound, or where the
+ * step would raise it.  n == 0 is a no-op.  The parity of this definition with the reference is unpinned.
+ * ---------------------------------------------------------------------------------------------- */
+
+/* bits fp32 [n, C] (dense) */
+int fpcc_gaussian_bits(const float *y, int64_t ld_y, const float *mu, int64_t ld_mu, const float *sigma, int64_t ld_s,
+                       int64_t n, int C, float scale_bound, float bound, float *bits, void *stream);
+/* dy, dmu (NULL: not written; needs mu) and dsigma fp32 [n, C] (dense) from the upstream dbits [n, C] (row pitch
+ * ld_db); the forward is recomputed in registers.  Elementwise, no reduction: deterministic. */
+int fpcc_gaussian_grad(const float *y, int64_t ld_y, const float *mu, int64_t ld_mu, const float *sigma, int64_t ld_s,
+                       const float *dbits, int64_t ld_db, int64_t n, int C, float scale_bound, float bound, float *dy,
+                       float *dmu, float *dsigma, void *stream);
+/* m = -Phi^-1(tail_mass / 2) in double (NaN unless 0 < tail_mass < 1): the half-width factor of the tables */
+double fpcc_gaussian_tail_multiplier(double tail_mass);
+/* Tables of a strictly increasing, positive scale_table fp32 [T] (compressai's rule): center_t = ceil(scale_table[t] * m)
+ * in double, pmf fp64 [T, S] row t = L(k) at mean 0, sigma = scale_table[t] for k = -center_t .. center_t, zero-padded;
+ * offsets[t] = -center_t.  S = 2 max(center) + 1 holds every row (a longer row is cut at S).  The input of
+ * fpcc_pmf_to_quantized_cdf with overflow coding. */
+int fpcc_gaussian_pmf(const float *scale_table, int T, double tail_mass, int S, double *pmf, int32_t *offsets, void *stream);
+/* idx int32 [n, C] (dense): the first t with scale_table[t] >= max(sigma, scale_bound), capped at T - 1 (compressai's
+ * build_indexes: never a narrower table than the model).  With y (and sym), also sym int32 [n, C] = rint(y - mu)
+ * (half to even; |y - mu| < 2^31 is the caller's to ensure).  The decoder passes y = sym = NULL and gets the same idx. */
+int fpcc_gaussian_indexes(const float *y, int64_t ld_y, const float *mu, int64_t ld_mu, const float *sigma, int64_t ld_s,
+                          int64_t n, int C, float scale_bound, const float *scale_table, int T, int32_t *sym,
+                          int32_t *idx, void *stream);
 
 #ifdef __cplusplus
 }
