@@ -1713,6 +1713,9 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_tc_kernel(WgArgs a) {
         for (int t = blockIdx.x; t < a.n_tiles; t += gridDim.x) {
             const int4 tl = __ldg(&a.tiles[t]);
             const int n_st = (tl.z - tl.y + WG_PAIRS - 1) / WG_PAIRS;
+            // a tile of no pairs consumes none of the indices fetched for it: fetch the next tile's here, or that tile's
+            // first stage would gather nothing
+            if (n_st <= 0) fetch_idx(t + gridDim.x, 0);
             for (int s = 0; s < n_st; ++s, ++it) {
                 int32_t cin_[4], cout_[4];
 #pragma unroll

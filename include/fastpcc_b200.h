@@ -362,7 +362,7 @@ int fpcc_spconv_f16(const void *feats, int dtype, int n_in, int c_in, const void
  * torchsparse's backward: per kernel offset dW[k] = X[in_k]^T * dY[out_k], reference call sites train.py:359-404 via
  * loss.backward()).  x [*, c_in_p], dy [*, c_out_p] fp16 (dtype 0) / bf16 (1) rows padded to c_in_p in {128, 256} and
  * c_out_p a multiple of 64 (<= 256); in_idx / out_idx are the compacted pair lists of fpcc_kmap_compact; tiles holds
- * n_tiles int32 quadruples (offset k, first pair, end pair, 0), each at most 2048 pairs of ONE offset; dw is the fp32
+ * n_tiles int32 quadruples (offset k, first pair, end pair, 0), each at most 2048 pairs (none allowed) of ONE offset; dw is the fp32
  * [kvol, c_in, c_out] gradient, ACCUMULATED into (zero it first).  Contraction over the gathered rows: tcgen05.mma with
  * both operands MN-major; partial sums of the tiles of an offset meet in dw through fp32 atomics. */
 int fpcc_spconv_wgrad_f16(const void *x, const void *dy, int dtype, int c_in_p, int c_out_p, const int32_t *in_idx,
