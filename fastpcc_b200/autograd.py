@@ -1,5 +1,6 @@
 """Training support for the float sparse convolution (SURVEY §8a row 19): torch.autograd.Functions around the tcgen05
-kernels, shared by the torchsparse-shaped layers (`torchsparse_nn.py`) and the MinkowskiEngine shim (`me.py`).
+kernels.  Every float conv / linear layer, of the torchsparse-shaped layers (`torchsparse_nn.py`) and of the
+MinkowskiEngine shim (`me.py`) alike, trains through `MELayerFunction`: its forward is the layer's own inference call.
 
   forward   out[m]  = act(sum_k  A[nbr_k(m)] @ W[k] + bias)          fused tcgen05 kernel, fp32 accumulation
   act'      dZ      = dOut * act'(out), dbias = sum_m dZ[m]          `fpcc_act_grad_f16`: one pass, read from the
@@ -19,9 +20,10 @@ The Gaussian conditional model of the hyperprior (`GaussianBitsFunction`) likewi
 backward (`fpcc_gaussian_bits` / `fpcc_gaussian_grad`).
 
 MinkowskiEngine computes the same three products per kernel offset (ME backward = transposed gather-GEMM-scatter).
-The ME layer kinds map onto these products as follows (`MELayerFunction`):
+The layer kinds map onto these products as follows (`MELayerFunction`):
 
   conv   kv > 1 (stride 1, k2s2, explicit target key)   dgrad on kmap_transpose(table), wgrad on kmap_compact(table)
+         (torchsparse: every conv but 1x1 at stride 1)
   linear 1x1 conv, MinkowskiLinear                      dgrad linear_f16(dZ, W^T), wgrad with kv = 1 identity pairs
   tconv  k2s2 onto an existing key (selection linear)   the conv rules on the child-slot table [8, n_child]
   gen    generative k2s2 (dense C_in -> 8 C_out)        dgrad linear_f16(dZ.view(N, 8 C_out'), W8^T), wgrad with
@@ -32,12 +34,6 @@ import torch
 from . import ops
 
 WGRAD_TC = True  # False: per-offset library GEMMs (A/B switch for the tests)
-
-
-def transpose_table(table: torch.Tensor, n_in: int) -> torch.Tensor:
-    """k-major map of the transposed convolution: tt[k, j] = m + 1 where table[k, m] == j + 1 (0 = none).  Each
-    (offset, input row) pairs with at most one output row, so the scatter has no collisions (fpcc_kmap_transpose)."""
-    return ops.kmap_transpose(table, n_in)
 
 
 # Tensors derived from a kernel map (transposed map for dgrad, compacted pair lists + tile offsets for wgrad) are the same
@@ -61,7 +57,7 @@ def _derived(table: torch.Tensor, n_in: int) -> dict:
 def _transposed(table, n_in):
     ent = _derived(table, n_in)
     if 'tt' not in ent:
-        ent['tt'] = transpose_table(table, n_in)
+        ent['tt'] = ops.kmap_transpose(table, n_in)
     return ent['tt']
 
 
@@ -96,56 +92,12 @@ def _wgrad(x, dz, in_map, out_map, off, c_in, c_out):
     return dw
 
 
-class SparseConvFunction(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, feats, weight, bias, table, compute_dtype):
-        kv, c_in, c_out = weight.shape
-        cin_p, cout_p = max(16, (c_in + 7) // 8 * 8), max(16, c_out)
-        f = torch.nn.functional.pad(feats.to(compute_dtype), (0, cin_p - c_in)).contiguous()
-        w_t = torch.zeros((kv, cout_p, cin_p), dtype=compute_dtype, device=weight.device)
-        w_t[:, :c_out, :c_in] = weight.detach().permute(0, 2, 1).to(compute_dtype)
-        b = None
-        if bias is not None:
-            b = torch.zeros(cout_p, dtype=torch.float32, device=weight.device)
-            b[:c_out] = bias.detach().float().reshape(-1)
-        out = ops.spconv_f16(f, w_t, table, bias=b, out_dtype=torch.float32)[:, :c_out]
-        ctx.save_for_backward(feats, weight, table)
-        ctx.has_bias, ctx.compute_dtype = bias is not None, compute_dtype
-        return out.to(feats.dtype if feats.dtype.is_floating_point else torch.float32)
-
-    @staticmethod
-    def backward(ctx, grad_out):
-        feats, weight, table = ctx.saved_tensors
-        kv, c_in, c_out = weight.shape
-        dt = ctx.compute_dtype
-        g = grad_out.contiguous()
-        d_feats = d_weight = d_bias = None
-        if ctx.needs_input_grad[0]:
-            cin_p, cout_p = max(16, c_in), max(16, (c_out + 7) // 8 * 8)
-            gp = torch.nn.functional.pad(g.to(dt), (0, cout_p - c_out)).contiguous()
-            w = torch.zeros((kv, cin_p, cout_p), dtype=dt, device=weight.device)   # [K, "C_out" = c_in, "C_in" = c_out]
-            w[:, :c_in, :c_out] = weight.detach().to(dt)
-            tt = _transposed(table, feats.shape[0])
-            d_feats = ops.spconv_f16(gp, w, tt, out_dtype=torch.float32)[:, :c_in].to(feats.dtype)
-        if ctx.needs_input_grad[1]:
-            in_map, out_map, off = _compacted(table, feats.shape[0])
-            d_weight = _wgrad(feats.to(dt), g.to(dt), in_map, out_map, off, c_in, c_out).to(weight.dtype)
-        if ctx.has_bias and ctx.needs_input_grad[2]:
-            d_bias = g.float().sum(0)
-        return d_feats, d_weight, d_bias, None, None
-
-
-def sparse_conv(feats, weight, bias, table, compute_dtype=torch.float16):
-    """differentiable sparse convolution: feats [n_in, C_in], weight [K, C_in, C_out], k-major table [K, n_out]"""
-    return SparseConvFunction.apply(feats, weight, bias, table, compute_dtype)
-
-
 class MESpec:
-    """What the backward of one MinkowskiEngine-shim layer needs (built by `me.py`, which owns the forward):
+    """What the backward of one layer needs (built by `me.py` or `torchsparse_nn.py`, which own the forward):
     kind 'conv' | 'linear' | 'tconv' | 'gen'; table: the UNGROUPED k-major map (conv) or the child-slot table (tconv);
     group: regroup the transposed table (the forward's GROUP_ROWS_MIN rule on the dgrad's output rows); layout of the
     kernel parameter: 'kio' [K, C_in, C_out], 'io' [C_in, C_out] (1x1 conv), 'oi' [C_out, C_in] (nn.Linear); dtype: the
-    compute dtype of the forward, in which the feature gradients travel."""
+    compute dtype of the forward, in which the feature gradients travel (fp32 for fp32 input features)."""
 
     def __init__(self, kind, c_in, c_out, act, slope, dtype, layout='kio', table=None, group=False):
         self.kind, self.c_in, self.c_out, self.act, self.slope, self.dtype = kind, c_in, c_out, act, slope, dtype
@@ -158,7 +110,7 @@ def _kio(kernel, layout):
 
 
 class MELayerFunction(torch.autograd.Function):
-    """One conv / linear layer of the ME shim with its fused epilogue (bias, ReLU / LeakyReLU slope >= 0).  The forward
+    """One float conv / linear layer with its fused epilogue (bias, ReLU / LeakyReLU slope >= 0).  The forward
     is the layer's own inference call (`run`), so the output bits do not depend on the grad mode."""
 
     @staticmethod
@@ -177,30 +129,25 @@ class MELayerFunction(torch.autograd.Function):
         need_b = ctx.bias_shape is not None and ctx.needs_input_grad[2]
         dt = sp.dtype
         c_in, c_out = sp.c_in, sp.c_out
-        c_pad = max(16, (c_out + 7) // 8 * 8)  # operand width of the dgrad / wgrad kernels
+        c_pad = ops.f16_widths(c_out, c_in)[0]  # dgrad / wgrad reduce over the layer's outputs: the forward's roles swapped
         dz, db = ops.act_grad_f16(dy, y, sp.act, sp.slope, c_pad, out_dtype=dt, want_bias=need_b)
         w = _kio(kernel, sp.layout)  # fp32 [K, C_in, C_out]
-        kv = w.shape[0]
         d_feats = d_kernel = d_bias = None
         n_in = feats.shape[0]
         if need_x:
-            cin_o = max(16, c_in)
+            wd = ops.f16_weight(w.transpose(1, 2), dt)  # [K, "C_out" = c_in, "C_in" = c_out], padded
+            dx_dt = torch.float32 if feats.dtype == torch.float32 else dt  # fp32 features get fp32 gradients
             if sp.kind in ('conv', 'tconv'):
-                wd = torch.zeros((kv, cin_o, c_pad), dtype=dt, device=w.device)  # [K, "C_out" = c_in, "C_in" = c_out]
-                wd[:, :c_in, :c_out] = w.to(dt)
                 if sp.group:
                     tt, perm = _transposed_grouped(sp.table, n_in)
                 else:
                     tt, perm = _transposed(sp.table, n_in), None
-                d_feats = ops.spconv_f16(dz, wd, tt, out_dtype=dt, row_perm=perm)
+                d_feats = ops.spconv_f16(dz, wd, tt, out_dtype=dx_dt, row_perm=perm)
             elif sp.kind == 'linear':
-                wl = torch.zeros((cin_o, c_pad), dtype=dt, device=w.device)
-                wl[:c_in, :c_out] = w[0].to(dt)
-                d_feats = ops.linear_f16(dz, wl, out_dtype=dt)
+                d_feats = ops.linear_f16(dz, wd[0], out_dtype=dx_dt)
             else:  # gen: the 8 children of row n are rows 8n..8n+7 of dZ, i.e. one row of dZ.view(N, 8 c_pad)
-                wg = torch.zeros((cin_o, 8, c_pad), dtype=dt, device=w.device)
-                wg[:c_in, :, :c_out] = w.permute(1, 0, 2).to(dt)
-                d_feats = ops.linear_f16(dz.view(n_in, 8 * c_pad), wg.reshape(cin_o, 8 * c_pad), out_dtype=dt)
+                wg = wd.permute(1, 0, 2).reshape(wd.shape[1], 8 * c_pad)
+                d_feats = ops.linear_f16(dz.view(n_in, 8 * c_pad), wg, out_dtype=dx_dt)
             d_feats = d_feats[:, :c_in] if d_feats.shape[1] != c_in else d_feats
         if need_w:
             x = feats.to(dt).contiguous()
@@ -222,7 +169,7 @@ class MELayerFunction(torch.autograd.Function):
 
 
 def me_layer(feats, kernel, bias, spec, run):
-    """differentiable ME-shim layer: `run()` computes the forward output from `feats` with the layer's inference kernels"""
+    """differentiable float layer: `run()` computes the forward output from `feats` with the layer's inference kernels"""
     return MELayerFunction.apply(feats, kernel, bias, spec, run)
 
 

@@ -17,9 +17,9 @@ Differences that matter to a caller:
     through `autograd.MELayerFunction` -- the same forward kernels in the same order (the output bits do not depend on
     the grad mode), dgrad / wgrad on the tcgen05 kernels, the fused ReLU / LeakyReLU (slope >= 0) backward in one pass
     (`fpcc_act_grad_f16`).  On that path a PReLU or a negative LeakyReLU slope is applied after the layer as a torch op,
-    so a PReLU slope trains.  Feature gradients travel in the compute dtype, parameter gradients are fp32.  Pruning,
-    cat, +, batch norm and max (un)pooling are torch ops and differentiate as such: max pooling shares the gradient
-    among tied maxima (torch's `scatter_reduce` amax rule), where ME routes it to one argmax.
+    so a PReLU slope trains.  Feature gradients travel in the compute dtype (fp32 for fp32 input features), parameter
+    gradients are fp32.  Pruning, cat, +, batch norm and max (un)pooling are torch ops and differentiate as such: max
+    pooling shares the gradient among tied maxima (torch's `scatter_reduce` amax rule), where ME routes it to one argmax.
 """
 from enum import Enum
 from typing import Dict, Optional, Tuple, Union
@@ -385,10 +385,6 @@ def _as_compute(f: torch.Tensor) -> torch.Tensor:
     return f if f.dtype == _COMPUTE else f.to(_COMPUTE)
 
 
-def _pad_cols(t: torch.Tensor, n: int) -> torch.Tensor:
-    return t if t.shape[1] == n else torch.nn.functional.pad(t, (0, n - t.shape[1]))
-
-
 class _ConvBase(nn.Module):
     def __init__(self, in_channels, out_channels, kernel_size=-1, stride=1, dilation=1, bias=False,
                  kernel_generator: Optional[KernelGenerator] = None, dimension=3, **_):
@@ -411,24 +407,21 @@ class _ConvBase(nn.Module):
         key = (self.kernel._version, self.kernel.data_ptr(), _COMPUTE, None if self.bias is None else self.bias._version)
         if self._cache is None or self._cache[0] != key:
             k = self.kernel.detach()
-            k = k[None] if k.dim() == 2 else k
-            cin_p = max(16, (k.shape[1] + 7) // 8 * 8)
-            cout_p = max(16, k.shape[2])
-            w = torch.zeros((k.shape[0], cout_p, cin_p), dtype=_COMPUTE, device=k.device)
-            w[:, :k.shape[2], :k.shape[1]] = k.permute(0, 2, 1).to(_COMPUTE)
+            w = ops.f16_weight(k[None] if k.dim() == 2 else k, _COMPUTE)
+            cout_p, cin_p = w.shape[1:]
             b = None
             if self.bias is not None:
                 b = torch.zeros(cout_p, dtype=torch.float32, device=k.device)
-                b[:k.shape[2]] = self.bias.detach().reshape(-1).float()
+                b[:k.shape[-1]] = self.bias.detach().reshape(-1).float()
             _publish(w)
             self._cache = (key, w, b, cin_p, cout_p)
         return self._cache[1:]
 
     def _run(self, f, table, act, slope, residual=None, row_perm=None):
         w, b, cin_p, cout_p = self._weights()
-        f = _pad_cols(_as_compute(f), cin_p).contiguous()
+        f = ops.pad_cols(_as_compute(f), cin_p).contiguous()
         if residual is not None:
-            residual = _pad_cols(_as_compute(residual), cout_p).contiguous()
+            residual = ops.pad_cols(_as_compute(residual), cout_p).contiguous()
         kv = w.shape[0]
         # single-channel heads (occupancy logits, top-k scores, the clipped bottom feature) keep the fp32 accumulator:
         # rounded to fp16 they collide into ties that the codecs' `kthvalue` / `>` selections (lossy_coord_v2/layers.py:
@@ -495,7 +488,7 @@ class MinkowskiConvolutionTranspose(_ConvBase):
 
         def run():
             w, b, cin_p, cout_p = self._weights()
-            f = _pad_cols(_as_compute(x.F), cin_p).contiguous()
+            f = ops.pad_cols(_as_compute(x.F), cin_p).contiguous()
             # rows without a parent belong to no group: they keep act(bias)
             fill = torch.zeros(cout_p, dtype=torch.float32, device=f.device) if b is None else b
             fill = torch.relu(fill) if code == ops.ACT_RELU else (torch.where(fill < 0, fill * slope, fill) if code == ops.ACT_LEAKY else fill)
@@ -532,7 +525,7 @@ class MinkowskiGenerativeConvolutionTranspose(_ConvBase):
 
         def run():
             w, b, cin_p, cout_p = self._weights()
-            f = _pad_cols(_as_compute(x.F), cin_p).contiguous()
+            f = ops.pad_cols(_as_compute(x.F), cin_p).contiguous()
             b8 = None if b is None else b.repeat(8)
             res = ops.linear_f16(f, w.reshape(8 * cout_p, cin_p), bias=b8, act=code, slope=slope)
             res = res.reshape(-1, cout_p)
@@ -556,9 +549,8 @@ class MinkowskiLinear(nn.Module):
         code, slope, after = _epilogue_act(fused_act, grad)
         key = (lin.weight._version, lin.weight.data_ptr(), _COMPUTE, None if lin.bias is None else lin.bias._version)
         if self._cache is None or self._cache[0] != key:
-            cin_p, cout_p = max(16, (lin.in_features + 7) // 8 * 8), max(16, lin.out_features)
-            w = torch.zeros((cout_p, cin_p), dtype=_COMPUTE, device=lin.weight.device)
-            w[:lin.out_features, :lin.in_features] = lin.weight.detach().to(_COMPUTE)
+            w = ops.f16_weight(lin.weight.t()[None], _COMPUTE)[0]
+            cout_p, cin_p = w.shape
             b = None
             if lin.bias is not None:
                 b = torch.zeros(cout_p, dtype=torch.float32, device=w.device)
@@ -568,7 +560,7 @@ class MinkowskiLinear(nn.Module):
         _, w, b, cin_p, cout_p = self._cache
 
         def run():
-            f = _pad_cols(_as_compute(x.F), cin_p).contiguous()
+            f = ops.pad_cols(_as_compute(x.F), cin_p).contiguous()
             od = torch.float32 if lin.out_features == 1 else None  # single-channel heads keep fp32 (see _ConvBase._run)
             out = ops.linear_f16(f, w, bias=b, act=code, slope=slope, out_dtype=od)
             return out[:, :lin.out_features] if cout_p != lin.out_features else out

@@ -617,6 +617,30 @@ _F_OUT = {torch.float16: 0, torch.bfloat16: 1, torch.float32: 2}
 ACT_NONE, ACT_RELU, ACT_LEAKY = 0, 1, 2
 
 
+def f16_widths(c_in, c_out):
+    """(c_in, c_out) -> (cin_p, cout_p): the operand widths `spconv_f16` / `linear_f16` take for a layer of c_in -> c_out
+    channels.  The reduced dimension is padded to a multiple of 8 and at least 16, the output dimension to at least 16
+    (fpcc_spconv_f16 / fpcc_linear_f16 require C_in % 8 == 0, C_in >= 16, C_out >= 16).  A dgrad reduces over the
+    layer's outputs: its widths are f16_widths(c_out, c_in)."""
+    return max(16, (c_in + 7) // 8 * 8), max(16, c_out)
+
+
+def f16_weight(kernel, dtype):
+    """kernel [K, C_in, C_out] -> the zero-padded weight operand [K, cout_p, cin_p] in dtype (f16_widths).  Passing
+    kernel.transpose(1, 2) gives the dgrad's operand [K, cin_p', cout_p'] of the same layer."""
+    k = kernel.detach()
+    kv, c_in, c_out = k.shape
+    cin_p, cout_p = f16_widths(c_in, c_out)
+    w = torch.zeros((kv, cout_p, cin_p), dtype=dtype, device=k.device)
+    w[:, :c_out, :c_in] = k.permute(0, 2, 1).to(dtype)
+    return w
+
+
+def pad_cols(t, n):
+    """t [rows, c] zero-padded to n columns (t itself when c == n)"""
+    return t if t.shape[1] == n else torch.nn.functional.pad(t, (0, n - t.shape[1]))
+
+
 def _fargs(bias, residual, out_dtype):
     if bias is not None:
         _need(bias, torch.float32, 'bias', 1)

@@ -9,14 +9,16 @@ torchsparse hash map (lib/int_sparse_conv/src/hashmap/hashmap_cuda.cuh:221-275: 
 even kernels z fastest), a strided conv with kernel == stride writes to coordinates >> log2(stride), and kernel
 maps / hash tables are cached on the tensor's `_caches` exactly like the integer layers do, so both families share
 them.  Every conv is ONE fused kernel (`fpcc_spconv_f16`, rows grouped by neighbour pattern for large inputs);
-activations / residual adds that follow can ride in its epilogue (`fused_act`, `residual`)."""
+activations / residual adds that follow can ride in its epilogue (`fused_act`, `residual`).  Training runs the same
+call inside `autograd.MELayerFunction`, the backward the MinkowskiEngine shim's layers train on; there activations and
+residual adds stay torch ops."""
 import math
 from typing import Optional, Tuple, Union
 
 import torch
 import torch.nn as nn
 
-from . import ops
+from . import autograd, ops
 from .int_sparse_conv.cuda_ops import GROUP_ROWS_MIN, KernelMap, build_kernel_map
 from .sparse_tensor import SparseTensor, _triple
 
@@ -27,10 +29,6 @@ def set_compute_dtype(dtype):
     global _COMPUTE
     assert dtype in (torch.float16, torch.bfloat16)
     _COMPUTE = dtype
-
-
-def _pad_cols(t: torch.Tensor, n: int) -> torch.Tensor:
-    return t if t.shape[1] == n else torch.nn.functional.pad(t, (0, n - t.shape[1]))
 
 
 def _out_coords(x: SparseTensor, stride: Tuple[int, int, int]):
@@ -61,7 +59,10 @@ def conv3d(input: SparseTensor, weight: torch.Tensor, kernel_size=3, bias: Optio
            padding=0, dilation=1, transposed: bool = False, generative: bool = False, config=None, training: bool = False,
            fused_act: int = ops.ACT_NONE, slope: float = 0.0, residual: Optional[torch.Tensor] = None,
            post_act: int = ops.ACT_NONE, post_slope: float = 0.0, out_dtype=None, _weight_t=None) -> SparseTensor:
-    """torchsparse.nn.functional.conv3d (non-transposed): weight [K, C_in, C_out] or [C_in, C_out]."""
+    """torchsparse.nn.functional.conv3d (non-transposed): weight [K, C_in, C_out] or [C_in, C_out].
+    With grad enabled and the weight or the features requiring it, the same call runs inside `autograd.me_layer`, which
+    gives it its backward: the output then leaves in the features' float dtype (fp32 for other features), and fused
+    activations and residuals are refused (they follow as torch ops)."""
     assert not transposed and not generative, 'the codec path uses forward convolutions only'
     assert _triple(dilation) == (1, 1, 1)
     ks, st = _triple(kernel_size), _triple(stride)
@@ -69,45 +70,48 @@ def conv3d(input: SparseTensor, weight: torch.Tensor, kernel_size=3, bias: Optio
     w = weight[None] if weight.dim() == 2 else weight
     assert w.shape[0] == kv, f'weight has {w.shape[0]} offsets, kernel {ks} needs {kv}'
     c_in, c_out = w.shape[1], w.shape[2]
-    cin_p, cout_p = max(16, (c_in + 7) // 8 * 8), max(16, c_out)
+    cin_p, cout_p = ops.f16_widths(c_in, c_out)
     training = torch.is_grad_enabled() and (weight.requires_grad or input.F.requires_grad)
-    if _weight_t is None and not training:
-        _weight_t = torch.zeros((kv, cout_p, cin_p), dtype=_COMPUTE, device=w.device)
-        _weight_t[:, :c_out, :c_in] = w.detach().permute(0, 2, 1).to(_COMPUTE)
+    if training:
+        assert fused_act == ops.ACT_NONE and residual is None and post_act == ops.ACT_NONE, 'fused epilogues are inference only'
+        out_dtype = input.F.dtype if input.F.dtype.is_floating_point else torch.float32
+    if _weight_t is None:
+        _weight_t = ops.f16_weight(w, _COMPUTE)
     b = None
     if bias is not None:
         b = torch.zeros(cout_p, dtype=torch.float32, device=w.device)
         b[:c_out] = bias.detach().reshape(-1).float()
-    f = None if training else _pad_cols(input.F.to(_COMPUTE), cin_p).contiguous()
+    f = ops.pad_cols(input.F.to(_COMPUTE), cin_p).contiguous()
     if residual is not None:
-        residual = _pad_cols(residual.to(out_dtype or _COMPUTE), cout_p).contiguous()
+        residual = ops.pad_cols(residual.to(out_dtype or _COMPUTE), cout_p).contiguous()
     out_stride, out_c = _out_coords(input, st)
-    caches = input._caches
-    if training:
-        # training: differentiable path (fastpcc_b200/autograd.py); activations / residuals stay in torch
-        assert fused_act == ops.ACT_NONE and residual is None and post_act == ops.ACT_NONE, 'fused epilogues are inference only'
-        from . import autograd
-        kmap = _kernel_map(input, out_c, ks, st)
-        out = autograd.sparse_conv(input.F, w, bias, kmap.table, _COMPUTE)
-        caches.cmaps.setdefault(input.stride, (input.C, input.spatial_range))
-        caches.cmaps.setdefault(out_stride, (out_c, None))
-        ret = SparseTensor(out, out_c, out_stride, None)
-        ret._caches = caches
-        return ret
-    if kv == 1 and st == (1, 1, 1):
-        out = ops.linear_f16(f, _weight_t[0], bias=b, act=fused_act, slope=slope, residual=residual, post_act=post_act,
-                             post_slope=post_slope, out_dtype=out_dtype)
-    else:
-        kmap = _kernel_map(input, out_c, ks, st)
-        if kmap.table.shape[1] >= GROUP_ROWS_MIN:
-            table, perm = kmap.grouped()
+    linear = kv == 1 and st == (1, 1, 1)
+    kmap = None if linear else _kernel_map(input, out_c, ks, st)
+
+    def run():
+        if linear:
+            out = ops.linear_f16(f, _weight_t[0], bias=b, act=fused_act, slope=slope, residual=residual, post_act=post_act,
+                                 post_slope=post_slope, out_dtype=out_dtype)
         else:
-            table, perm = kmap.table, None
-        out = ops.spconv_f16(f, _weight_t, table, bias=b, act=fused_act, slope=slope, residual=residual, post_act=post_act,
-                             post_slope=post_slope, out_dtype=out_dtype, row_perm=perm)
+            if kmap.table.shape[1] >= GROUP_ROWS_MIN:
+                table, perm = kmap.grouped()
+            else:
+                table, perm = kmap.table, None
+            out = ops.spconv_f16(f, _weight_t, table, bias=b, act=fused_act, slope=slope, residual=residual,
+                                 post_act=post_act, post_slope=post_slope, out_dtype=out_dtype, row_perm=perm)
+        return out[:, :c_out] if cout_p != c_out else out
+
+    if training:
+        sp = autograd.MESpec('linear' if linear else 'conv', c_in, c_out, ops.ACT_NONE, 0.0, _COMPUTE,
+                             layout='kio' if weight.dim() == 3 else 'io', table=None if linear else kmap.table,
+                             group=input.F.shape[0] >= GROUP_ROWS_MIN)
+        out = autograd.me_layer(input.F, weight, bias, sp, run)
+    else:
+        out = run()
+    caches = input._caches
     caches.cmaps.setdefault(input.stride, (input.C, input.spatial_range))
     caches.cmaps.setdefault(out_stride, (out_c, None))
-    ret = SparseTensor(out[:, :c_out] if cout_p != c_out else out, out_c, out_stride, None)
+    ret = SparseTensor(out, out_c, out_stride, None)
     ret._caches = caches
     return ret
 
@@ -137,10 +141,7 @@ class Conv3d(nn.Module):
         key = (self.kernel._version, self.kernel.data_ptr(), _COMPUTE)
         if self._cache is None or self._cache[0] != key:
             k = self.kernel.detach()
-            k = k[None] if k.dim() == 2 else k
-            cin_p, cout_p = max(16, (k.shape[1] + 7) // 8 * 8), max(16, k.shape[2])
-            w = torch.zeros((k.shape[0], cout_p, cin_p), dtype=_COMPUTE, device=k.device)
-            w[:, :k.shape[2], :k.shape[1]] = k.permute(0, 2, 1).to(_COMPUTE)
+            w = ops.f16_weight(k[None] if k.dim() == 2 else k, _COMPUTE)
             torch.cuda.current_stream().synchronize()  # the cache may be read from another stream next
             self._cache = (key, w)
         return self._cache[1]

@@ -10,6 +10,7 @@ against ME itself, which cannot be installed offline.
 import numpy as np
 import torch
 
+from fastpcc_b200.ops import f16_weight, f16_widths, pad_cols  # noqa: F401  operand padding: bookkeeping, not arithmetic
 from . import float_ops as F
 
 ACT_NONE, ACT_RELU, ACT_LEAKY = 0, 1, 2

@@ -125,17 +125,18 @@ def test_torchsparse_style_layers_match_fp32_reference():
     assert (ret.F.cpu().numpy()[:, 0] == occ).all()                            # exact: small integers in fp16 / fp32
 
 
-def test_sparse_conv_autograd_matches_dense_reference():
-    """Training slice (SURVEY §8a row 19): gradients of the fused sparse conv w.r.t. features, weights and bias against
-    torch autograd through the same sum written with index_select + matmul in fp32; then a Block trains one SGD step."""
-    from fastpcc_b200 import synth, autograd as AG, ops, torchsparse_nn as TS
+def test_conv3d_autograd_matches_dense_reference():
+    """Training slice (SURVEY §8a row 19): gradients of the fused sparse conv (`torchsparse_nn.conv3d` with an explicit
+    weight and bias) w.r.t. features, weights and bias against torch autograd through the same sum written with
+    index_select + matmul in fp32, for the conv and the 1x1 (linear) kinds; then a Block trains one SGD step."""
+    from fastpcc_b200 import synth, ops, torchsparse_nn as TS
     from fastpcc_b200.sparse_tensor import SparseTensor
     rng = np.random.default_rng(8)
     C = synth.with_batch(synth.surface_cloud(6, bits=7, n_target=3000))
     C = torch.from_numpy(C[np.lexsort((C[:, 3], C[:, 2], C[:, 1], C[:, 0]))]).cuda()
     n, cin, cout = C.shape[0], 24, 40
     keys, vals = ops.hash_build(C)
-    for ks, st, out_c in (((3, 3, 3), (1, 1, 1), C),
+    for ks, st, out_c in (((3, 3, 3), (1, 1, 1), C), ((1, 1, 1), (1, 1, 1), C),
                           ((2, 2, 2), (2, 2, 2), torch.unique(torch.cat([C[:, :1], C[:, 1:] >> 1], 1), dim=0))):
         table = ops.kmap_lookup(keys, vals, out_c.contiguous(), ks, st)
         kv = table.shape[0]
@@ -143,7 +144,9 @@ def test_sparse_conv_autograd_matches_dense_reference():
         w = (torch.randn(kv, cin, cout, device='cuda') / (kv * cin) ** 0.5).half().float().requires_grad_()
         b = torch.randn(cout, device='cuda').requires_grad_()
         gout = torch.randn(table.shape[1], cout, device='cuda').half().float()
-        out = AG.sparse_conv(a, w, b, table)
+        ret = TS.conv3d(SparseTensor(a, C, 1), w, ks, bias=b, stride=st)
+        assert torch.equal(ret.C, out_c)                                    # the rows of `table`
+        out = ret.F
         out.backward(gout)
         got = (out.detach(), a.grad.clone(), w.grad.clone(), b.grad.clone())
         a.grad = w.grad = b.grad = None
